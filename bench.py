@@ -3,6 +3,7 @@
 knn_predict on an 811,457 x 512 bank, k=200, t=0.1, 9 classes, in the BIT-EXACT `fp32` mode.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--mode fp32|bf16|...] [--data clustered|gauss|relu|absgauss]
+                  [--dump-outputs DIR]      # the last timed step's class ranking -> DIR/pred_labels.npy
   python bench.py --impl reference ...      # the reference algorithm on the host CPU cores
   python bench.py --config ref              # the reference-shaped call: N=37,348, B=64 per call, k=5
 
@@ -209,6 +210,28 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+DUMP_BYTES = 64 * 10**6 - 1024  # 64 MB less room for two .npy headers
+
+
+def dump_outputs(out_dir, pred_labels):
+    """Writes what knn_predict returned, the (Q, C) class ranking, as float64 (class indices are exact
+    in it) to out_dir/pred_labels.npy.  Above DUMP_BYTES in all it keeps a fixed seeded sample of the
+    rows, sorted, and writes their indices to out_dir/pred_labels_rows.npy."""
+    import numpy as np
+
+    pred = pred_labels.cpu().numpy().astype(np.float64)
+    n_rows, n_cols = pred.shape
+    if pred.nbytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n_rows, DUMP_BYTES // (8 * (n_cols + 1)), replace=False))
+        pred = pred[rows]
+    else:
+        rows = None
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "pred_labels.npy"), pred)
+    if rows is not None:
+        np.save(os.path.join(out_dir, "pred_labels_rows.npy"), rows.astype(np.float64))
+
+
 def elem_bytes(cand_mode):
     return {"bf16": 2, "f16": 2, "bf16x3": 4, "f16x2": 2, "tf32x3": 8, "exact": 4}[cand_mode]
 
@@ -365,7 +388,13 @@ def main():
     ap.add_argument("--dim", type=int, default=DIM, help="vector dimension (default 512; 768 = config c5)")
     ap.add_argument("--k", type=int, default=None)
     ap.add_argument("--classes", type=int, default=N_CLASSES, help="9 = WM-811K priors; 38 = MixedWM38 (config c3)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the class ranking the last timed step returned to DIR/pred_labels.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.config == "ref":  # scripts/WM811k_benchmark.py:49,71; knn.py:38; train_data rows (notebook 1.0:1721)
         N_BANK, KNN_K = 37348, 5
         args.queries = args.queries or 64
@@ -449,9 +478,12 @@ def main():
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item())
 
+    last = {}
+
     def step_resident():
         K.query_cache.clear()  # a new batch every step in real use: re-prepare (cast) the queries
-        return predict(q)
+        last["pred"] = predict(q)
+        return last["pred"]
 
     # e2e: every step uploads its own batch from pinned host memory and reads its predictions
     # back.  The upload of step i+1 is enqueued on a copy stream before step i's compute, so
@@ -508,6 +540,8 @@ def main():
     _lib.launch_counter["kernels"] = 0
     with ClockSampler(local) as clocks:
         total_ms = timed(step_resident, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["pred"])
     n_abi_kernels = _lib.launch_counter["kernels"]
     events = K.profile_events
     K.profile_events = None

@@ -1,5 +1,5 @@
 """A stand-in for the reference's ``KNNBenchmarkModule`` (``src/ssl_wafermap/models/knn.py:28-138``)
-for the GPU box, where /root/reference, pytorch_lightning and torchmetrics do not exist.
+for driving the hooks on the GPU without pytorch_lightning and torchmetrics.
 
 TEST INFRASTRUCTURE, like the oracle: it restates the three validation hooks' data flow (what the
 hooks read and write on the module: ``backbone``, ``dataloader_kNN``, ``num_classes``, ``knn_k``,
@@ -8,7 +8,8 @@ hooks read and write on the module: ``backbone``, ``dataloader_kNN``, ``num_clas
 hook_classes=(StandInKNNModule,))`` can be driven end to end and compared with the un-hooked flow.
 The un-hooked hooks look the module-global ``knn_predict`` up at call time, exactly like the
 reference does after ``from lightly.utils.benchmarking import knn_predict`` (``knn.py:16``).
-tests/test_hooks_cpu.py runs the same comparison against the REAL reference file on CPU.
+tests/test_hooks_cpu.py runs the same comparison on CPU against the reference's module file as
+restated in tests/reference_knn.py, imported with its third-party dependencies stubbed.
 """
 import numpy as np
 import torch

@@ -1,12 +1,12 @@
-"""CPU: b200knn.install(hooks=True) against the REAL reference module file
-(/root/reference/src/ssl_wafermap/models/knn.py, imported with its absent third-party
-dependencies — lightly, pytorch_lightning, timm, torchmetrics, wandb, matplotlib, seaborn —
-stubbed out).  Checks that the reference's own classes get their three validation hooks replaced
-(KNNBenchmarkModule) / two (WandBKNNBenchmarkModule, whose epoch-end also draws a W&B figure),
-that the module global `knn_predict` is rebound, and — with the CUDA-only compute steps served by
-the oracle — that one validation epoch through the hooks gives the un-hooked flow's predictions
-and metrics.  Skipped where /root/reference does not exist (the GPU box; there
-tests/test_gpu_round2.py::test_hooks_equal_unhooked_flow drives the hooks on the device)."""
+"""CPU: b200knn.install(hooks=True) against the reference's kNN module file
+(src/ssl_wafermap/models/knn.py, restated in tests/reference_knn.py and imported under the
+reference's module name with its absent third-party dependencies — lightly, pytorch_lightning,
+timm, torchmetrics, wandb, matplotlib, seaborn — stubbed out).  Checks that the reference's classes
+get their three validation hooks replaced (KNNBenchmarkModule) / two (WandBKNNBenchmarkModule,
+whose epoch-end also draws a W&B figure), that the module global `knn_predict` is rebound, and —
+with the CUDA-only compute steps served by the oracle — that one validation epoch through the hooks
+gives the un-hooked flow's predictions and metrics
+(tests/test_gpu_round2.py::test_hooks_equal_unhooked_flow drives the hooks on the device)."""
 import importlib.util
 import os
 import sys
@@ -20,8 +20,7 @@ import torch.nn as nn
 import datagen
 from oracle import knn_oracle as O
 
-REF_FILE = "/root/reference/src/ssl_wafermap/models/knn.py"
-pytestmark = pytest.mark.skipif(not os.path.exists(REF_FILE), reason="reference tree not present")
+REF_FILE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "reference_knn.py")
 
 
 class _Anything:

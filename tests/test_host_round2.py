@@ -117,3 +117,23 @@ def test_bench_library_bar_is_the_reference_op_sequence():
     f, bank, lab = (torch.from_numpy(c[n]) for n in ("feature", "bank", "labels"))
     got = bench.library_knn_predict(f, bank, lab, c["C"], c["k"], c["t"])
     assert torch.equal(got, O.knn_predict_r32(f, bank, lab, c["C"], c["k"], c["t"]))
+
+
+def test_bench_dump_outputs_full_and_sampled(tmp_path, monkeypatch):
+    """--dump-outputs: the whole (Q, C) ranking as float64 while it fits the budget, else the same
+    seeded sample of rows on every run, with their indices."""
+    import bench
+
+    pred = torch.stack([torch.randperm(9, generator=torch.Generator().manual_seed(r)) for r in range(500)])
+    bench.dump_outputs(str(tmp_path / "full"), pred)
+    got = np.load(tmp_path / "full" / "pred_labels.npy")
+    assert got.dtype == np.float64 and np.array_equal(got, pred.numpy())
+    assert not (tmp_path / "full" / "pred_labels_rows.npy").exists()
+    monkeypatch.setattr(bench, "DUMP_BYTES", 8 * 10 * 100)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), pred)
+    rows = np.load(tmp_path / "a" / "pred_labels_rows.npy")
+    assert rows.dtype == np.float64 and len(rows) == 100 and np.all(np.diff(rows) > 0)
+    assert np.array_equal(np.load(tmp_path / "a" / "pred_labels.npy"), pred.numpy()[rows.astype(np.int64)])
+    for name in ("pred_labels.npy", "pred_labels_rows.npy"):
+        assert np.array_equal(np.load(tmp_path / "a" / name), np.load(tmp_path / "b" / name))

@@ -3,7 +3,6 @@ metrics, embedding-table reader)."""
 import os
 
 import numpy as np
-import pytest
 import torch
 
 import datagen
@@ -70,27 +69,20 @@ def test_metrics_from_counts_on_cpu_tensors():
 
 
 def test_load_embedding_table_roundtrip(tmp_path):
+    """The layout of the reference's tables (notebooks/3.0-Embeddings-inference.ipynb:493-507):
+    integer columns 0..511 hold the fp16 embedding, then waferMap, failureType, failureCode."""
     import pandas as pd
 
     from b200knn.retrieval import load_embedding_table
 
     rng = np.random.default_rng(7)
-    emb = rng.standard_normal((30, 16)).astype(np.float16)
-    df = pd.DataFrame(emb, columns=list(range(16)))
+    emb = rng.standard_normal((30, 512)).astype(np.float16)
+    df = pd.DataFrame(emb, columns=list(range(512)))
+    df["waferMap"] = [rng.integers(0, 3, (26, 26), dtype=np.uint8) for _ in range(30)]
     df["failureType"] = ["none"] * 30
     df["failureCode"] = rng.integers(0, 9, 30)
     path = os.path.join(tmp_path, "Demo_preds_subset.pkl.xz")
     df.to_pickle(path)
     got, meta = load_embedding_table(path)
-    assert got.dtype == np.float16 and np.array_equal(got, emb)
-    assert list(meta.columns) == ["failureType", "failureCode"]
-
-
-@pytest.mark.skipif(not os.path.exists("/root/reference/data/interim/model_preds/FastSiam_preds_subset.pkl.xz"),
-                    reason="reference tree not mounted")
-def test_load_reference_table():
-    from b200knn.retrieval import load_embedding_table
-
-    emb, meta = load_embedding_table("/root/reference/data/interim/model_preds/FastSiam_preds_subset.pkl.xz")
-    assert emb.shape == (12449, 512) and emb.dtype == np.float16
-    assert "failureCode" in meta.columns
+    assert got.shape == (30, 512) and got.dtype == np.float16 and np.array_equal(got, emb)
+    assert list(meta.columns) == ["waferMap", "failureType", "failureCode"]
