@@ -220,6 +220,19 @@ int b200knn_vote_ex(const uint64_t* keys, const int64_t* labels, int64_t B, int 
                     int64_t* pred, int64_t pred_ld, int status_col, double* scores,
                     int32_t* err_flag, void* stream);
 
+/*
+ * b200knn_vote_ex for a grid of settings from one neighbour list per row: keys (B, k_max) and
+ * ks[0] < ks[1] < ... < ks[n_k-1] == k_max (1 <= n_k <= 16), ts[0..n_t) non-zero (1 <= n_t <= 8).
+ * pred has row stride pred_ld >= n_k*n_t*C; columns [(i*n_t + j)*C, (i*n_t + j + 1)*C) of a row
+ * hold exactly what b200knn_vote writes for that row's first ks[i] keys at t = ts[j].
+ * status_col: -1, or a column >= n_k*n_t*C for b200knn_vote_ex's status word (bit 0: the
+ * k_max-th slot is empty).
+ */
+int b200knn_vote_multi(const uint64_t* keys, const int64_t* labels, int64_t B, int k_max,
+                       int64_t n_labels, int64_t label_offset, int C, const int* ks, int n_k,
+                       const double* ts, int n_t, int64_t* pred, int64_t pred_ld, int status_col,
+                       int32_t* err_flag, void* stream);
+
 /* out[b] = similarity of keys[b, j] (-inf for an empty slot): the threshold a (B,r) sample
  * hands to b200knn_topk_ex (j = r-1). */
 int b200knn_key_sim_column(const uint64_t* keys, int64_t B, int k, int j, float* out,

@@ -106,5 +106,14 @@ class FeatureBank:
             raise RuntimeError("this FeatureBank was built without labels")
         return K.knn_predict(self._queries(feature, normalize), self.bank, self.labels, num_classes, knn_k, knn_t)
 
+    def knn_predict_multi(self, feature: torch.Tensor, num_classes: int, knn_ks=(200,), knn_ts=(0.1,),
+                          normalize: bool = False) -> torch.Tensor:
+        """``knn_predict`` over a (knn_ks, knn_ts) grid from one neighbour search (``K.knn_predict_multi``):
+        (len(knn_ks), len(knn_ts), B, C); normalize=True fuses the query ``F.normalize``."""
+        if self.labels is None:
+            raise RuntimeError("this FeatureBank was built without labels")
+        return K.knn_predict_multi(self._queries(feature, normalize), self.bank, self.labels, num_classes,
+                                   knn_ks, knn_ts)
+
     def knn_topk(self, feature: torch.Tensor, k: int, normalize: bool = False, mode: Optional[str] = None):
         return K.knn_topk(self._queries(feature, normalize), self.bank, k, mode)

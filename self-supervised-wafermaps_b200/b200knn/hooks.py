@@ -17,6 +17,11 @@ and uploads a W&B figure (``knn.py:241-272``), which is not this path and stays 
 The hooks keep the module's observable state: ``feature_bank`` ((D,N), a zero-copy view),
 ``targets_bank``, ``all_preds`` / ``all_targets``, ``max_accuracy`` / ``max_f1``, the
 ``knn_accuracy`` / ``knn_f1`` log keys and the ``confusion_matrix`` list of numpy arrays.
+
+Opt-in kNN grid: a module with ``b200knn_knn_grid = (ks, ts)`` is scored in ``validation_step`` by one
+``FeatureBank.knn_predict_multi`` over ks x ts extended by its own (knn_k, knn_t); its state above
+stays that of its own setting, and ``on_validation_epoch_end`` also logs ``knn_accuracy_k{k}_t{t}`` and
+``knn_f1_k{k}_t{t}`` for every setting of the extended grid.
 """
 from __future__ import annotations
 
@@ -53,15 +58,40 @@ def on_validation_epoch_start(self):
 
     fb = _bank.FeatureBank.from_batches(batches(), normalize=True, total_rows=_total_rows(self.dataloader_kNN))
     self._b200knn_bank = fb
+    self.__dict__.pop("_b200knn_grid_preds", None)  # an epoch whose end hook is not ours (W&B twin)
     self.feature_bank = fb.bank        # (D, N): what the reference's own knn_predict call would read
     self.targets_bank = fb.labels
+
+
+def _grid(self):
+    """The module's opt-in ``b200knn_knn_grid = (ks, ts)`` extended by its own (knn_k, knn_t), or None."""
+    grid = getattr(self, "b200knn_knn_grid", None)
+    if grid is None:
+        return None
+    ks, ts = [int(k) for k in grid[0]], [float(t) for t in grid[1]]
+    if int(self.knn_k) not in ks:
+        ks.append(int(self.knn_k))
+    if float(self.knn_t) not in ts:
+        ts.append(float(self.knn_t))
+    return ks, ts
 
 
 def validation_step(self, batch, batch_idx):
     images, targets = batch
     feature = self.backbone(images).squeeze()
-    pred_labels = self._b200knn_bank.knn_predict(feature, self.num_classes, self.knn_k, self.knn_t,
-                                                 normalize=True)
+    grid = _grid(self)
+    if grid is None:
+        pred_labels = self._b200knn_bank.knn_predict(feature, self.num_classes, self.knn_k, self.knn_t,
+                                                     normalize=True)
+    else:
+        # every setting of the grid from one neighbour search; the module's own setting is one of them
+        ks, ts = grid
+        pred = self._b200knn_bank.knn_predict_multi(feature, self.num_classes, ks, ts, normalize=True)
+        pred_labels = pred[ks.index(int(self.knn_k)), ts.index(float(self.knn_t))]
+        preds = self.__dict__.setdefault("_b200knn_grid_preds", {})
+        for i, k in enumerate(ks):
+            for j, t in enumerate(ts):
+                preds.setdefault((k, t), []).append(pred[i, j, :, 0])
     self.all_preds.append(pred_labels[:, 0])
     self.all_targets.append(targets)
 
@@ -78,6 +108,10 @@ def on_validation_epoch_end(self):
     self.log("knn_accuracy", acc, on_epoch=True, prog_bar=True)
     self.log("knn_f1", f1, on_epoch=True, prog_bar=True)
     self.confusion_matrix.append(m["confusion"].detach().cpu().numpy())
+    for (k, t), preds in self.__dict__.pop("_b200knn_grid_preds", {}).items():
+        g = _metrics.knn_metrics(torch.cat(preds, dim=0), all_targets, self.num_classes)
+        self.log(f"knn_accuracy_k{k}_t{t:g}", float(g["accuracy"]), on_epoch=True)
+        self.log(f"knn_f1_k{k}_t{t:g}", float(g["f1"]), on_epoch=True)
     self.all_preds.clear()
     self.all_targets.clear()
 

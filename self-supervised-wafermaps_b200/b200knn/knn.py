@@ -1141,26 +1141,110 @@ def vote(keys: torch.Tensor, feature_labels: torch.Tensor, num_classes: int, knn
                                         label_offset, C, float(knn_t), pred.data_ptr(), _ptr(scores),
                                         flag.data_ptr(), _stream()), "vote")
             if check_labels:
-                f = int(flag.item())
-                if f == 1:
-                    # the reference raises here from zeros(...).scatter(...) (lightly knn_predict)
-                    raise RuntimeError("index out of bounds: a feature_labels entry is outside "
-                                       f"[0, num_classes={C})")
-                if f == 2:
-                    raise RuntimeError("index out of bounds: neighbour index outside feature_labels")
+                _raise_vote_flag(int(flag.item()), C)
     if return_flag:  # device int32[1]: 0 ok, 1 label outside [0,C), 2 neighbour index outside labels
         return pred, (flag if B else torch.zeros((1,), dtype=torch.int32, device=dev))
     return (pred, scores) if return_scores else pred
 
 
+MAX_GRID_KS, MAX_GRID_TS = 16, 8  # kVoteMaxKs / kVoteMaxTs of csrc/kernels.h
+
+
+def _vote_multi_into(keys, feature_labels, num_classes, knn_ks, knn_ts, out, status_col, flag) -> None:
+    """b200knn_vote_multi of keys (B, knn_ks[-1]) into the (>= B, ld) int64 tensor `out`."""
+    B, k = keys.shape
+    labels = feature_labels if feature_labels.dtype == torch.int64 else feature_labels.long()
+    labels = labels.contiguous().view(-1)
+    ks = (ctypes.c_int * len(knn_ks))(*[int(x) for x in knn_ks])
+    ts = (ctypes.c_double * len(knn_ts))(*[float(x) for x in knn_ts])
+    keys = keys.contiguous()
+    with torch.cuda.device(keys.device):
+        _lib.check(_lib.load().b200knn_vote_multi(keys.data_ptr(), labels.data_ptr(), B, k, labels.numel(), 0,
+                                                  int(num_classes), ks, len(knn_ks), ts, len(knn_ts),
+                                                  out.data_ptr(), out.stride(0), status_col, flag.data_ptr(),
+                                                  _stream()), "vote_multi")
+
+
+def vote_multi(keys: torch.Tensor, feature_labels: torch.Tensor, num_classes: int, knn_ks, knn_ts,
+               check_labels: bool = True, flag: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """keys (B, k_max) sorted + labels (N,) -> (B, n_k*n_t*C) int64: block (i, j) of a row is what
+    ``vote`` returns for the row's first knn_ks[i] keys at knn_t = knn_ts[j].  knn_ks strictly
+    increasing with knn_ks[-1] == k_max.  flag: optional device int32[1] for the label status
+    (check_labels=False leaves reading it to the caller)."""
+    _require_cuda("feature_labels", feature_labels)
+    B = keys.shape[0]
+    C = int(num_classes)
+    pred = torch.empty((B, len(knn_ks) * len(knn_ts) * C), dtype=torch.int64, device=keys.device)
+    if B:
+        if flag is None:
+            flag = torch.zeros((1,), dtype=torch.int32, device=keys.device)
+        _vote_multi_into(keys, feature_labels, C, knn_ks, knn_ts, pred, -1, flag)
+        if check_labels:
+            _raise_vote_flag(int(flag.item()), C)
+    return pred
+
+
+def vote_multi_packed(keys: torch.Tensor, feature_labels: torch.Tensor, num_classes: int, knn_ks, knn_ts,
+                      n_rows_out: int) -> torch.Tensor:
+    """vote_packed for a grid: (n_rows_out, W+1) int64, W = n_k*n_t*C, the rankings of vote_multi in
+    columns [0, W) and vote_packed's status word in column W; rows past keys.shape[0] are zero."""
+    B = keys.shape[0]
+    W = len(knn_ks) * len(knn_ts) * int(num_classes)
+    dev = keys.device
+    out = torch.zeros((n_rows_out, W + 1), dtype=torch.int64, device=dev) if n_rows_out > B \
+        else torch.empty((n_rows_out, W + 1), dtype=torch.int64, device=dev)
+    if B:
+        flag = torch.zeros((1,), dtype=torch.int32, device=dev)
+        _vote_multi_into(keys, feature_labels, num_classes, knn_ks, knn_ts, out, W, flag)
+    return out
+
+
+def _raise_vote_flag(f: int, C: int) -> None:
+    if f == 1:
+        # the reference raises here from zeros(...).scatter(...) (lightly knn_predict)
+        raise RuntimeError("index out of bounds: a feature_labels entry is outside "
+                           f"[0, num_classes={C})")
+    if f == 2:
+        raise RuntimeError("index out of bounds: neighbour index outside feature_labels")
+
+
+def check_grid(knn_ks, knn_ts):
+    """Validate a (knn_ks, knn_ts) grid: (ks as ints, ts as floats, ascending order of ks)."""
+    ks, ts = list(knn_ks), list(knn_ts)
+    if not ks or not ts:
+        raise ValueError("knn_ks and knn_ts must not be empty")
+    if len(ks) > MAX_GRID_KS or len(ts) > MAX_GRID_TS:
+        raise ValueError(f"at most {MAX_GRID_KS} values of knn_k and {MAX_GRID_TS} of knn_t per call")
+    if any(int(k) != k for k in ks):
+        raise ValueError(f"knn_ks must be integers, got {ks}")
+    ks, ts = [int(k) for k in ks], [float(t) for t in ts]
+    if min(ks) <= 0:
+        raise ValueError(f"every knn_k must be positive, got {ks}")
+    if any(t == 0.0 for t in ts):
+        raise ValueError("knn_t must be non-zero")
+    if len(set(ks)) != len(ks) or len(set(ts)) != len(ts):
+        raise ValueError(f"duplicate values in knn_ks {ks} or knn_ts {ts}")
+    return ks, ts, sorted(range(len(ks)), key=ks.__getitem__)
+
+
 # ----------------------------------------------------------------------------
 # the reference's public symbols for this path
 # ----------------------------------------------------------------------------
+def _vote_step(keys, feature_labels, num_classes, knn_t, flag):
+    """The vote of a call, label status into the device int32[1] `flag`: knn_t a temperature ->
+    (B, C) rankings (``vote``); knn_t a (ks, ts) grid, ks ascending and ks[-1] == keys.shape[1] ->
+    (B, n_k*n_t*C) rankings (``vote_multi``)."""
+    if isinstance(knn_t, tuple):
+        return vote_multi(keys, feature_labels, num_classes, knn_t[0], knn_t[1], check_labels=False, flag=flag)
+    return vote(keys, feature_labels, num_classes, knn_t, check_labels=False, return_flag=True, flag=flag)[0]
+
+
 def _predict_enqueue(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t, mode, track=True, boost=1):
     """Everything of one tensor-core-mode call, enqueued without a host synchronisation (so it can
     be captured into a CUDA graph): (pred (B,C), status int32[2] = [vote flag, rows to recompute],
     bad_rows (B,) mask/flags, fix).  status[0]: 1 label / 2 neighbour index out of range;
-    status[1]: rows a sampled threshold starved, or rows whose re-scoring could not be certified."""
+    status[1]: rows a sampled threshold starved, or rows whose re-scoring could not be certified.
+    knn_t: a temperature, or a (ks, ts) grid (``_vote_step``; pred is then (B, n_k*n_t*C))."""
     # one zeroed status word per call: [vote flag, rows to recompute] — the kernels write into it
     status = torch.zeros((2,), dtype=torch.int32, device=feature.device)
     if mode in RESCORED_MODES:
@@ -1171,8 +1255,7 @@ def _predict_enqueue(feature, feature_bank, feature_labels, num_classes, knn_k, 
         bad_rows = keys[:, -1] == 0
         status[1:2] = bad_rows.sum().to(torch.int32)
         fix = None
-    pred, _ = vote(keys, feature_labels, num_classes, knn_t, check_labels=False, return_flag=True,
-                   flag=status[0:1])
+    pred = _vote_step(keys, feature_labels, num_classes, knn_t, status[0:1])
     return pred, status, bad_rows, fix
 
 
@@ -1188,21 +1271,17 @@ def _predict_finish(pred, status, bad_rows, fix, feature, feature_bank, feature_
         rows = bad_rows.nonzero(as_tuple=False).view(-1)
         fixed = fix(rows, n_fix) if mode in RESCORED_MODES else \
             recompute_rows(feature, feature_bank, knn_k, mode, rows)
-        pred[rows], flag2 = vote(fixed, feature_labels, num_classes, knn_t, check_labels=False, return_flag=True)
+        flag2 = torch.zeros((1,), dtype=torch.int32, device=pred.device)
+        pred[rows] = _vote_step(fixed, feature_labels, num_classes, knn_t, flag2)
         status[0] = max(int(status[0]), int(flag2.item()))
-    if status[0] == 1:
-        # the reference raises here from zeros(...).scatter(...) (lightly knn_predict)
-        raise RuntimeError("index out of bounds: a feature_labels entry is outside "
-                           f"[0, num_classes={int(num_classes)})")
-    if status[0] == 2:
-        raise RuntimeError("index out of bounds: neighbour index outside feature_labels")
+    _raise_vote_flag(int(status[0]), int(num_classes))
     return pred
 
 
 # ---- the reference-shaped call (B = 64 per validation_step, knn.py:87-99; scripts/WM811k_benchmark.py:71)
 # is launch-latency bound: a dozen small kernels and as many Python -> C transitions per call.  For
 # batches of at most GRAPH_MAX_BATCH rows the enqueued part of a call is captured ONCE per
-# (bank, batch shape, k, C, t, mode) into a CUDA graph and replayed: one copy of the queries into
+# (bank, batch shape, k, C, t or (ks, ts) grid, mode) into a CUDA graph and replayed: one copy of the queries into
 # the graph's static input, one graph launch, one read of the status word.  A non-zero status (rows
 # to recompute, label errors — rare) re-runs the call on the ordinary path, so results and errors
 # are exactly those of the un-captured call.
@@ -1228,7 +1307,8 @@ def _graph_boost(feature_bank, mode) -> int:
 def _graph_key(feature, feature_bank, labels, num_classes, knn_k, knn_t, mode):
     return (_graph_boost(feature_bank, mode), feature_bank.data_ptr(), feature_bank._version, tuple(feature_bank.shape), tuple(feature_bank.stride()),
             feature_bank.dtype, feature_bank.device.index, labels.data_ptr(), labels._version,
-            tuple(feature.shape), feature.dtype, int(num_classes), int(knn_k), float(knn_t), mode)
+            tuple(feature.shape), feature.dtype, int(num_classes), int(knn_k),
+            knn_t if isinstance(knn_t, tuple) else float(knn_t), mode)
 
 
 def _graph_for(feature, feature_bank, labels, num_classes, knn_k, knn_t, mode):
@@ -1284,21 +1364,33 @@ def knn_predict(feature: torch.Tensor, feature_bank: torch.Tensor, feature_label
     column 0.  Neighbour order is (similarity desc, bank index asc); class order is
     (score desc, class id asc).
     """
+    return _predict(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t, _default_mode)
+
+
+def _vote_checked(keys, feature_labels, num_classes, knn_t):
+    """``_vote_step`` raising the label errors itself (one host synchronisation)."""
+    if isinstance(knn_t, tuple):
+        return vote_multi(keys, feature_labels, num_classes, knn_t[0], knn_t[1])
+    return vote(keys, feature_labels, num_classes, knn_t)
+
+
+def _predict(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t, mode):
+    """knn_predict in `mode`; knn_t a temperature, or a (ks, ts) grid with ks ascending and
+    ks[-1] == knn_k (``_vote_step``)."""
     _require_cuda("feature_labels", feature_labels)
-    mode = _default_mode
     if feature_labels.numel() != feature_bank.shape[1]:
         _check_feature_bank(feature, feature_bank)
         raise RuntimeError(
             f"feature_labels has {feature_labels.numel()} entries for a bank of {feature_bank.shape[1]}")
     if mode == "exact" or int(knn_k) > MAX_K:
-        return vote(topk_keys(feature, feature_bank, knn_k, mode), feature_labels, num_classes, knn_t)
+        return _vote_checked(topk_keys(feature, feature_bank, knn_k, mode), feature_labels, num_classes, knn_t)
     _check_feature_bank(feature, feature_bank)
     knn_k = int(knn_k)
     if knn_k <= 0 or knn_k > feature_bank.shape[1]:
         raise RuntimeError("selected index k out of range")
     if feature.shape[0] == 0:
-        return vote(torch.empty((0, knn_k), dtype=torch.int64, device=feature.device), feature_labels,
-                    num_classes, knn_t)
+        return _vote_checked(torch.empty((0, knn_k), dtype=torch.int64, device=feature.device), feature_labels,
+                             num_classes, knn_t)
     # Tensor-core modes: everything is enqueued first and ONE host synchronisation reads the
     # status word (vote flag; rows to recompute: rows a sampled threshold starved, or rows whose
     # exact re-scoring could not be certified).
@@ -1326,6 +1418,40 @@ def knn_predict(feature: torch.Tensor, feature_bank: torch.Tensor, feature_label
                                                    knn_t, mode)
     return _predict_finish(pred, status.tolist(), bad_rows, fix, feature, feature_bank, feature_labels,
                            num_classes, knn_k, knn_t, mode)
+
+
+def knn_predict_multi(feature: torch.Tensor, feature_bank: torch.Tensor, feature_labels: torch.Tensor,
+                      num_classes: int, knn_ks=(200,), knn_ts=(0.1,)) -> torch.Tensor:
+    """``knn_predict`` for every (knn_k, knn_t) of a grid from ONE neighbour search at
+    k_max = max(knn_ks) and one vote kernel: (len(knn_ks), len(knn_ts), B, num_classes) int64, where
+    [i, j] is bitwise ``knn_predict(..., knn_ks[i], knn_ts[j])`` in the default mode.  The top-k list
+    is the first k entries of the top-k_max list: the (sim desc, index asc) order and the
+    similarities themselves do not depend on k.  At most 16 values of k and 8 of t, no duplicates."""
+    ks, ts, order = check_grid(knn_ks, knn_ts)
+    mode = _default_mode
+    parts = [_predict(feature, feature_bank, feature_labels, num_classes, part[-1], (part, tuple(ts)), mode)
+             for part in grid_parts(tuple(ks[i] for i in order), mode)]
+    return grid_view(torch.cat(parts, dim=1) if len(parts) > 1 else parts[0], order, len(ts), num_classes)
+
+
+def grid_parts(ks_ascending: tuple, mode: str) -> list:
+    """The searches a grid needs: one at k_max, except in a raw tensor-core mode whose ks straddle
+    MAX_K — lists longer than MAX_K come from the exact kernel, shorter ones from the mode's own
+    similarities, so each side gets its own search."""
+    if mode in TC_MODES and ks_ascending[0] <= MAX_K < ks_ascending[-1]:
+        n_lo = sum(k <= MAX_K for k in ks_ascending)
+        return [ks_ascending[:n_lo], ks_ascending[n_lo:]]
+    return [ks_ascending]
+
+
+def grid_view(pred: torch.Tensor, order, n_t: int, num_classes: int) -> torch.Tensor:
+    """(B, n_k*n_t*C) rankings over ks sorted by `order` -> (n_k, n_t, B, C) in the caller's order."""
+    B = pred.shape[0]
+    g = pred.view(B, len(order), n_t, int(num_classes)).permute(1, 2, 0, 3)
+    inv = [0] * len(order)
+    for pos, i in enumerate(order):
+        inv[i] = pos
+    return g[torch.tensor(inv, device=pred.device)] if inv != list(range(len(order))) else g.contiguous()
 
 
 def knn_topk(feature: torch.Tensor, feature_bank: torch.Tensor, k: int,

@@ -113,6 +113,12 @@ class _CudaOps:
         return vote_packed(keys, labels, num_classes, knn_t, n_rows_out)
 
     @staticmethod
+    def vote_multi_packed(keys, labels, num_classes, knn_ks, knn_ts, n_rows_out):
+        """vote_packed for a (knn_ks ascending, knn_ts) grid: (n_rows_out, n_k*n_t*C + 1)."""
+        from .knn import vote_multi_packed
+        return vote_multi_packed(keys, labels, num_classes, knn_ks, knn_ts, n_rows_out)
+
+    @staticmethod
     def decode_keys(keys):
         from .knn import decode_keys
         return decode_keys(keys)
@@ -516,16 +522,18 @@ class ShardedBank:
         self._mark("  merge + certify")
         return merged, flags
 
-    def _predict_level_packed(self, feature, C, knn_k, knn_t, level):
-        """One cascade level for all (replicated) query rows: (G*per, C+1) int64, identical on every
-        rank — class rankings in columns [0, C), status word in column C (bit 0 starved row, bits
-        1 / 2 label / index out of range, bit 3 uncertified)."""
+    def _predict_level_packed(self, feature, knn_k, W, vote_packed, level):
+        """One cascade level for all (replicated) query rows: (G*per, W+1) int64, identical on every
+        rank — class rankings (W = C columns, or n_k*n_t*C for a grid) in columns [0, W), status word
+        in column W (bit 0 starved row, bits 1 / 2 label / index out of range, bit 3 uncertified).
+        vote_packed(keys, n_rows_out): the call's vote step (``_CudaOps.vote_packed`` or
+        ``vote_multi_packed`` with the call's settings bound)."""
         n = feature.shape[0]
         per, lo, hi = self._owned(n)
         merged, flags = self._owned_keys_rescored(feature, knn_k, level)
-        packed = self.ops.vote_packed(merged[:hi - lo], self.labels, C, knn_t, per)
-        packed[:hi - lo, C] |= flags.to(torch.int64) << 3
-        gathered = torch.empty((per * self.world_size, C + 1), dtype=torch.int64, device=feature.device)
+        packed = vote_packed(merged[:hi - lo], per)
+        packed[:hi - lo, W] |= flags.to(torch.int64) << 3
+        gathered = torch.empty((per * self.world_size, W + 1), dtype=torch.int64, device=feature.device)
         dist.all_gather_into_tensor(gathered, packed, group=self.group)
         self._mark("vote+gather")
         return gathered
@@ -537,7 +545,7 @@ class ShardedBank:
     _boost = 1
     _calm = 0
 
-    def _knn_predict_rescored(self, feature, C, knn_k, knn_t, levels) -> torch.Tensor:
+    def _knn_predict_rescored(self, feature, C, knn_k, W, vote_packed, levels) -> torch.Tensor:
         """Sharded fp32 mode, ONE host synchronisation per call.
         Level 1 (all rows): `_owned_keys_rescored` at the cascade's first level.  Rows it leaves
         uncertified or starved (status bits 3 / 0 — identical on every rank after the all-gather)
@@ -549,33 +557,33 @@ class ShardedBank:
         uncertified on some shard, or more open rows than the capacity) take the host-driven path."""
         B = feature.shape[0]
         self._mark("start")
-        packed = self._predict_level_packed(feature, C, knn_k, knn_t, levels[0])
+        packed = self._predict_level_packed(feature, knn_k, W, vote_packed, levels[0])
         out = packed[:B]
         n_open = None
         if hasattr(self.ops, "compact_rows"):
             if self._l2_cap is None:
                 self._l2_cap = {}
             cap = self._l2_cap.get(B) or min(B, max(256, -(-B // 64)))  # first call: 1/64 of the batch
-            rows, count = self.ops.compact_rows(out, C, 9, cap)
+            rows, count = self.ops.compact_rows(out, W, 9, cap)
             sub = feature.index_select(0, rows)
             loc = self.ops.local_exact_keys(sub, self.bank_shard, knn_k, self.mode, self.lo,
                                             self.world_size)                                # (cap, k+1)
             allk = self._gather(loc)                                                        # (G, cap, k+1)
             keys2 = self.ops.merge_keys(allk[:, :, :knn_k].contiguous(), knn_k)
-            pk2 = self.ops.vote_packed(keys2, self.labels, C, knn_t, cap)
-            pk2[:, C] |= (allk[:, :, knn_k].amax(0) != 0).to(torch.int64) << 3
+            pk2 = vote_packed(keys2, cap)
+            pk2[:, W] |= (allk[:, :, knn_k].amax(0) != 0).to(torch.int64) << 3
             self.ops.scatter_rows(out, pk2, rows, count)
             n_open = count
             self._mark("level 2 (open rows, per shard)")
         # one host read: OR of the status bits over all rows + the number of rows level 1 left open
         shifts = torch.arange(4, device=out.device)
-        bits = ((out[:, C:C + 1] >> shifts) & 1).amax(0)
+        bits = ((out[:, W:W + 1] >> shifts) & 1).amax(0)
         if n_open is None:
             host = bits.tolist() + [0]
         else:
             host = torch.cat([bits, n_open.view(1).to(bits.dtype)]).tolist()
-        status = out[:, C]
-        pred = out[:, :C].contiguous()
+        status = out[:, W]
+        pred = out[:, :W].contiguous()
         self.last_uncertified = int(host[4]) if n_open is not None else int(((status & 9) != 0).sum().item())
         if n_open is not None:
             # the second level costs every shard the same whatever G is: size it to ~1.5x the rows
@@ -590,16 +598,12 @@ class ShardedBank:
             rows = ((status & 9) != 0).nonzero(as_tuple=False).view(-1)
             sub = feature[rows].contiguous()
             keys = self.ops.merge_keys(self._gather(self.local_keys(sub, knn_k, None)), knn_k)
-            pk = self.ops.vote_packed(keys, self.labels, C, knn_t, rows.numel())
-            pred[rows] = pk[:, :C]
-            worst = int(pk[:, C].max().item()) if rows.numel() else 0
+            pk = vote_packed(keys, rows.numel())
+            pred[rows] = pk[:, :W]
+            worst = int(pk[:, W].max().item()) if rows.numel() else 0
             host[1] = host[1] or (worst & 2)
             host[2] = host[2] or (worst & 4)
-        if host[1]:
-            raise RuntimeError("index out of bounds: a feature_labels entry is outside "
-                               f"[0, num_classes={C})")
-        if host[2]:
-            raise RuntimeError("index out of bounds: neighbour index outside feature_labels")
+        _raise_label_bits((2 if host[1] else 0) | (4 if host[2] else 0), C)
         return pred
 
     def knn_predict(self, feature: torch.Tensor, num_classes: int, knn_k: int = 200,
@@ -607,6 +611,36 @@ class ShardedBank:
         """Same contract as ``knn_predict`` with the bank sharded; identical on every rank."""
         if exchange == "allgather" or self.world_size == 1 or not hasattr(self.ops, "vote_packed"):
             return self.ops.vote(self.topk_keys(feature, knn_k), self.labels, num_classes, knn_t)
+        C = int(num_classes)
+        return self._predict(feature, C, knn_k, C,
+                             lambda keys, n: self.ops.vote_packed(keys, self.labels, C, knn_t, n), exchange)
+
+    def knn_predict_multi(self, feature: torch.Tensor, num_classes: int, knn_ks=(200,), knn_ts=(0.1,),
+                          exchange: str = "alltoall") -> torch.Tensor:
+        """Same contract as ``knn_predict_multi`` with the bank sharded: (n_k, n_t, B, C), identical on
+        every rank and bitwise the 1-GPU result.  One sharded search at k_max (two when k_max is
+        beyond a raw tensor-core mode's lists and some k is not, as on one GPU)."""
+        from .knn import check_grid, get_default_mode, grid_parts, grid_view
+        ks, ts, order = check_grid(knn_ks, knn_ts)
+        C = int(num_classes)
+        preds = []
+        for part in grid_parts(tuple(ks[i] for i in order), self.mode or get_default_mode()):
+            W = len(part) * len(ts) * C
+
+            def vote_packed(keys, n, part=part):
+                return self.ops.vote_multi_packed(keys, self.labels, C, part, tuple(ts), n)
+
+            if exchange == "allgather" or self.world_size == 1:
+                packed = vote_packed(self.topk_keys(feature, part[-1]), feature.shape[0])
+                _raise_label_bits(int(packed[:, W].max().item()) if feature.shape[0] else 0, C)
+                preds.append(packed[:, :W])
+            else:
+                preds.append(self._predict(feature, C, part[-1], W, vote_packed, exchange))
+        return grid_view(torch.cat(preds, dim=1), order, len(ts), C)
+
+    def _predict(self, feature, C, knn_k, W, vote_packed, exchange) -> torch.Tensor:
+        """The all-to-all path of knn_predict / knn_predict_multi: (B, W) rankings; vote_packed(keys,
+        n_rows_out) -> (n_rows_out, W+1) is the call's vote step (see ``_predict_level_packed``)."""
         if exchange != "alltoall":
             raise ValueError(f"unknown exchange {exchange!r}")
         if knn_k > self.n_rows:
@@ -614,8 +648,8 @@ class ShardedBank:
         levels = self.ops.cascade_levels(self.bank_shard, self.mode, self._boost) \
             if hasattr(self.ops, "cascade_levels") else None
         if levels and self.rescore_at_row_owner and feature.shape[0] > 0:
-            return self._knn_predict_rescored(feature, int(num_classes), knn_k, knn_t, levels)
-        B, C = feature.shape[0], int(num_classes)
+            return self._knn_predict_rescored(feature, C, knn_k, W, vote_packed, levels)
+        B = feature.shape[0]
         per, lo, hi = self._owned(B)
         mark = self._mark
         mark("start")
@@ -623,24 +657,31 @@ class ShardedBank:
         mark("threshold")  # sample + all-gather of (B,16) + merge
         merged = self.owned_keys(feature, knn_k, tau0)
         mark("topk+exchange+merge")
-        # (per, C+1): class ranking + a status column, for the owned rows only (pad rows stay 0)
-        packed = self.ops.vote_packed(merged[:hi - lo], self.labels, C, knn_t, per)
-        gathered = torch.empty((per * self.world_size, C + 1), dtype=torch.int64, device=feature.device)
+        # (per, W+1): class rankings + a status column, for the owned rows only (pad rows stay 0)
+        packed = vote_packed(merged[:hi - lo], per)
+        gathered = torch.empty((per * self.world_size, W + 1), dtype=torch.int64, device=feature.device)
         dist.all_gather_into_tensor(gathered, packed, group=self.group)
         mark("vote+gather")
-        status = gathered[:B, C]
-        out = gathered[:B, :C].contiguous()
+        status = gathered[:B, W]
+        out = gathered[:B, :W].contiguous()
         worst = int(status.max().item()) if B else 0  # the one host synchronisation of the call
-        if worst & 2:
-            raise RuntimeError("index out of bounds: a feature_labels entry is outside "
-                               f"[0, num_classes={C})")
-        if worst & 4:
-            raise RuntimeError("index out of bounds: neighbour index outside feature_labels")
+        _raise_label_bits(worst, C)
         if worst == 1:
             # identical on every rank -> every rank takes this branch: recompute the starved rows
             # (the ~1e-7 tail of the sampled threshold) without a threshold
             rows = (status == 1).nonzero(as_tuple=False).view(-1)
             sub = feature[rows].contiguous()
             keys = self.ops.merge_keys(self._gather(self.local_keys(sub, knn_k, None)), knn_k)
-            out[rows] = self.ops.vote(keys, self.labels, C, knn_t)
+            pk = vote_packed(keys, rows.numel())
+            out[rows] = pk[:, :W]
+            _raise_label_bits(int(pk[:, W].max().item()), C)
         return out
+
+
+def _raise_label_bits(status: int, C: int) -> None:
+    """The errors of a status word (b200knn_vote_ex): bit 1 label / bit 2 neighbour index out of range."""
+    if status & 2:
+        raise RuntimeError("index out of bounds: a feature_labels entry is outside "
+                           f"[0, num_classes={C})")
+    if status & 4:
+        raise RuntimeError("index out of bounds: neighbour index outside feature_labels")

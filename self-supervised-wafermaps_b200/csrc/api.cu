@@ -531,6 +531,36 @@ int b200knn_vote_ex(const uint64_t* keys, const int64_t* labels, int64_t B, int 
   return e == cudaSuccess ? B200KNN_OK : fail_cuda("vote", e);
 }
 
+int b200knn_vote_multi(const uint64_t* keys, const int64_t* labels, int64_t B, int k_max, int64_t n_labels,
+                       int64_t label_offset, int C, const int* ks, int n_k, const double* ts, int n_t,
+                       int64_t* pred, int64_t pred_ld, int status_col, int32_t* err_flag, void* stream) {
+  if (!keys || !labels || !pred || !err_flag || !ks || !ts || B < 0 || k_max <= 0 || C <= 0 || n_labels <= 0)
+    return fail(B200KNN_E_ARG, "vote_multi: bad argument");
+  if (n_k < 1 || n_k > b200knn::kVoteMaxKs || n_t < 1 || n_t > b200knn::kVoteMaxTs)
+    return fail(B200KNN_E_ARG, "vote_multi: need 1 <= n_k <= 16 and 1 <= n_t <= 8");
+  b200knn::VoteGrid grid{};
+  grid.n_k = n_k;
+  grid.n_t = n_t;
+  for (int i = 0; i < n_k; ++i) {
+    if (ks[i] <= 0 || (i > 0 && ks[i] <= ks[i - 1]))
+      return fail(B200KNN_E_ARG, "vote_multi: ks must be positive and strictly increasing");
+    grid.ks[i] = ks[i];
+  }
+  if (ks[n_k - 1] != k_max) return fail(B200KNN_E_ARG, "vote_multi: ks[n_k-1] must equal k_max");
+  for (int j = 0; j < n_t; ++j) {
+    if (!(ts[j] > 0.0) && !(ts[j] < 0.0)) return fail(B200KNN_E_ARG, "vote_multi: temperature must be non-zero");
+    grid.ts[j] = ts[j];
+  }
+  const int64_t width = int64_t(n_k) * n_t * C;
+  if (pred_ld < width || status_col >= pred_ld || (status_col >= 0 && status_col < width))
+    return fail(B200KNN_E_ARG, "vote_multi: pred_ld / status_col do not describe a (B, >=n_k*n_t*C) output");
+  cudaError_t e = b200knn::launch_vote_multi(keys, labels, B, n_labels, label_offset, C, grid, pred, pred_ld,
+                                             status_col, err_flag, static_cast<cudaStream_t>(stream));
+  if (e == cudaErrorInvalidValue)
+    return fail(B200KNN_E_UNSUPPORTED, "vote_multi: k_max/num_classes/temperatures too large for shared memory");
+  return e == cudaSuccess ? B200KNN_OK : fail_cuda("vote_multi", e);
+}
+
 int b200knn_vote(const uint64_t* keys, const int64_t* labels, int64_t B, int k, int64_t n_labels,
                  int64_t label_offset, int C, double t, int64_t* pred, double* scores,
                  int32_t* err_flag, void* stream) {

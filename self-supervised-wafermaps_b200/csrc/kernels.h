@@ -34,6 +34,17 @@ cudaError_t launch_vote(const uint64_t* keys, const int64_t* labels, int64_t B, 
                         int64_t n_labels, int64_t label_offset, int C, double t, int64_t* pred,
                         int64_t pred_ld, int status_col, double* scores, int32_t* err_flag,
                         cudaStream_t stream);
+// launch_vote for every (ks[i], ts[j]) from one (B, ks[n_k-1]) key list; ks strictly increasing.
+// Passed by value, so a captured launch needs no device-side copy of the grid.
+constexpr int kVoteMaxKs = 16, kVoteMaxTs = 8;
+struct VoteGrid {
+  int n_k, n_t;
+  int ks[kVoteMaxKs];
+  double ts[kVoteMaxTs];
+};
+cudaError_t launch_vote_multi(const uint64_t* keys, const int64_t* labels, int64_t B, int64_t n_labels,
+                              int64_t label_offset, int C, const VoteGrid& grid, int64_t* pred, int64_t pred_ld,
+                              int status_col, int32_t* err_flag, cudaStream_t stream);
 // out[b] = similarity of keys[b, j] (-inf for an empty slot)
 cudaError_t launch_key_sim_column(const uint64_t* keys, int64_t B, int k, int j, float* out,
                                   cudaStream_t stream);

@@ -84,6 +84,94 @@ __global__ void __launch_bounds__(kVoteWarps * 32)
   }
 }
 
+// vote_kernel for a grid of (k, t) settings from one top-k_max list per row: block (i, j) of a
+// row's output is vote_kernel's ranking of its first ks[i] keys at temperature ts[j].  Per t the
+// warp evaluates w[j] = exp(double(sim_j) / t) across its lanes (vote_kernel's expression), then a
+// lane per class accumulates them in rank order j = 0, 1, ... (vote_kernel's order) and, whenever
+// j + 1 reaches ks[i], the warp ranks the accumulators (vote_kernel's rank rule): every block is
+// bitwise vote_kernel's result.  (Evaluating the exps in the lane that owns the class instead
+// leaves most lanes idle at C = 9: the grid call cost 1.089x one k = 200 call at the north
+// star that way, 1.003-1.050x this way; DESIGN §7.)
+__global__ void __launch_bounds__(kVoteWarps * 32)
+    vote_multi_kernel(const uint64_t* __restrict__ keys, const int64_t* __restrict__ labels, int64_t B,
+                      int64_t n_labels, int64_t label_offset, int C, VoteGrid grid,
+                      int64_t* __restrict__ pred, int64_t pred_ld, int status_col,
+                      int32_t* __restrict__ err_flag) {
+  extern __shared__ unsigned char vote_smem[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int k = grid.ks[grid.n_k - 1], n_t = grid.n_t;
+  // per warp: w[k] f64 | sc[C] f64 | sim[k] f32 | lab[k] i32
+  const size_t per_warp = size_t(k) * 16 + size_t(C) * 8;
+  unsigned char* base = vote_smem + size_t(warp) * per_warp;
+  double* w = reinterpret_cast<double*>(base);
+  double* sc = w + k;
+  float* sim = reinterpret_cast<float*>(sc + C);
+  int* lab = reinterpret_cast<int*>(sim + k);
+
+  const int64_t row = int64_t(blockIdx.x) * kVoteWarps + warp;
+  if (row >= B) return;
+
+  int bad = 0;  // vote_kernel's status bits
+  for (int j = lane; j < k; j += 32) {
+    const uint64_t key = keys[row * k + j];
+    int l = -1;
+    if (key != 0) {
+      const int64_t li = key_idx(key) - label_offset;
+      if (li >= 0 && li < n_labels) {
+        const int64_t c = labels[li];
+        if (c >= 0 && c < C) {
+          l = int(c);
+        } else {
+          atomicExch(err_flag, 1);
+          bad |= 2;
+        }
+      } else {
+        atomicExch(err_flag, 2);
+        bad |= 4;
+      }
+    } else if (j == k - 1) {
+      bad |= 1;
+    }
+    lab[j] = l;
+    sim[j] = key_sim(key);
+  }
+  if (status_col >= 0) {
+    bad = __reduce_or_sync(0xffffffffu, bad);
+    if (lane == 0) pred[row * pred_ld + status_col] = bad;
+  }
+  int64_t* out = pred + row * pred_ld;
+  for (int ti = 0; ti < n_t; ++ti) {
+    const double t = grid.ts[ti];
+    __syncwarp();  // lab / sim written; the previous t's ranking is done with w
+    for (int j = lane; j < k; j += 32) w[j] = lab[j] >= 0 ? exp(double(sim[j]) / t) : 0.0;
+    for (int c = lane; c < C; c += 32) sc[c] = 0.0;
+    __syncwarp();
+    int j0 = 0;
+    for (int s = 0; s < grid.n_k; ++s) {
+      const int j1 = grid.ks[s];
+      for (int c = lane; c < C; c += 32) {
+        double acc = sc[c];
+        for (int j = j0; j < j1; ++j)
+          if (lab[j] == c) acc += w[j];
+        sc[c] = acc;
+      }
+      j0 = j1;
+      __syncwarp();
+      int64_t* o = out + (int64_t(s) * n_t + ti) * C;
+      for (int c = lane; c < C; c += 32) {
+        const double v = sc[c];
+        int rank = 0;
+        for (int q = 0; q < C; ++q) {
+          const double sq = sc[q];
+          rank += (sq > v || (sq == v && q < c)) ? 1 : 0;
+        }
+        o[rank] = c;
+      }
+      __syncwarp();  // every lane has read sc before the next segment adds to it
+    }
+  }
+}
+
 // counts[t * C + p] += 1 for every (target t, prediction p): the confusion matrix the
 // reference builds with torchmetrics after each validation epoch
 // (src/ssl_wafermap/models/knn.py:104-129).  Block-private histograms in shared memory
@@ -133,6 +221,24 @@ cudaError_t launch_vote(const uint64_t* keys, const int64_t* labels, int64_t B, 
   const int64_t blocks = (B + kVoteWarps - 1) / kVoteWarps;
   vote_kernel<<<unsigned(blocks), kVoteWarps * 32, smem, stream>>>(
       keys, labels, B, k, n_labels, label_offset, C, t, pred, pred_ld, status_col, scores, err_flag);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_vote_multi(const uint64_t* keys, const int64_t* labels, int64_t B, int64_t n_labels,
+                              int64_t label_offset, int C, const VoteGrid& grid, int64_t* pred, int64_t pred_ld,
+                              int status_col, int32_t* err_flag, cudaStream_t stream) {
+  if (B == 0) return cudaSuccess;
+  const size_t per_warp = size_t(grid.ks[grid.n_k - 1]) * 16 + size_t(C) * 8;
+  const size_t smem = per_warp * kVoteWarps;
+  if (smem > 200 * 1024) return cudaErrorInvalidValue;
+  if (smem > 48 * 1024) {
+    cudaError_t e = cudaFuncSetAttribute(vote_multi_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         int(smem));
+    if (e != cudaSuccess) return e;
+  }
+  const int64_t blocks = (B + kVoteWarps - 1) / kVoteWarps;
+  vote_multi_kernel<<<unsigned(blocks), kVoteWarps * 32, smem, stream>>>(
+      keys, labels, B, n_labels, label_offset, C, grid, pred, pred_ld, status_col, err_flag);
   return cudaGetLastError();
 }
 
