@@ -188,6 +188,17 @@ int b200knn_topk_scatter(int mode, const void* q_hi, const void* q_lo,
 int b200knn_merge(const uint64_t* keys_in, int G, int64_t B, int k_in, int k_out,
                   uint64_t* keys_out, void* stream);
 
+/*
+ * Leave-one-out lists (no counterpart in the reference): row b of a search of bank rows
+ * [self_offset, self_offset + B) against the whole bank, without the row itself.
+ *   keys_in : (B, k_in) uint64, each row sorted descending, k_in >= 2
+ *   keys_out: (B, k_in - 1) uint64, must not overlap keys_in: row b without the key whose bank
+ *             index (the key's index field, idx_offset included) is b + self_offset, or without
+ *             its last key when no key has that index.  Empty (0) keys are copied and never match.
+ */
+int b200knn_drop_self(const uint64_t* keys_in, int64_t B, int k_in, int64_t self_offset,
+                      uint64_t* keys_out, void* stream);
+
 /* keys (B,k) -> sims (B,k) f32 and idx (B,k) int64  (Tensor.topk's two outputs).
  * Empty slots (fewer than k finite candidates) decode to sim=-inf, idx=-1. */
 int b200knn_decode_keys(const uint64_t* keys, int64_t n_keys, float* sims,

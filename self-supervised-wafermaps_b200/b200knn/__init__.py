@@ -5,6 +5,8 @@ faris-k/self-supervised-wafermaps (lightly's ``knn_predict`` as called from
 Public surface (mirrors the reference names for this path):
     knn_predict(feature, feature_bank, feature_labels, num_classes, knn_k=200, knn_t=0.1)
     knn_predict_multi(..., knn_ks, knn_ts)        -> knn_predict over a (k, t) grid, one search
+    knn_predict_loo(feature_bank, feature_labels, num_classes, knn_ks, knn_ts)
+                                                  -> leave-one-out grid of the bank against itself
     knn_topk(feature, feature_bank, k)            -> (sims, idx)
     install() / uninstall()                       -> rebind lightly's symbol
     ShardedBank                                   -> bank row-sharded over the GPUs of a node
@@ -22,6 +24,7 @@ from .knn import (  # noqa: F401
     decode_keys,
     get_default_mode,
     knn_predict,
+    knn_predict_loo,
     knn_predict_multi,
     knn_topk,
     merge_keys,

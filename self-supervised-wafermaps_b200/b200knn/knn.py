@@ -1104,6 +1104,20 @@ def decode_keys(keys: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
     return sims, idx
 
 
+def drop_self(keys: torch.Tensor, self_offset: int) -> torch.Tensor:
+    """(B, k_in) sorted keys of bank rows [self_offset, self_offset + B) searched against their own
+    bank -> (B, k_in - 1): row b without the key of bank row b + self_offset, or without its last
+    key when that row is not in the list (``b200knn_drop_self``)."""
+    _require_cuda("keys", keys)
+    B, k_in = keys.shape
+    keys = keys.contiguous()
+    out = torch.empty((B, max(k_in - 1, 0)), dtype=torch.int64, device=keys.device)
+    with torch.cuda.device(keys.device):
+        _lib.check(_lib.load().b200knn_drop_self(keys.data_ptr(), B, k_in, int(self_offset), out.data_ptr(),
+                                                 _stream()), "drop_self")
+    return out
+
+
 def merge_keys(keys_in: torch.Tensor, k_out: int) -> torch.Tensor:
     """(G,B,k_in) sorted candidate lists -> (B,k_out): the shard-merge step."""
     lib = _lib.load()
@@ -1442,6 +1456,64 @@ def grid_parts(ks_ascending: tuple, mode: str) -> list:
         n_lo = sum(k <= MAX_K for k in ks_ascending)
         return [ks_ascending[:n_lo], ks_ascending[n_lo:]]
     return [ks_ascending]
+
+
+def loo_parts(ks_ascending: tuple, mode: str) -> list:
+    """``grid_parts`` for leave-one-out ks, whose searches run at k + 1: a raw tensor-core mode
+    never asks its kernel for more than MAX_K keys, so its k = MAX_K is served by the exact kernel."""
+    return [tuple(k - 1 for k in part) for part in grid_parts(tuple(k + 1 for k in ks_ascending), mode)]
+
+
+def knn_predict_loo(feature_bank: torch.Tensor, feature_labels: torch.Tensor, num_classes: int,
+                    knn_ks=(200,), knn_ts=(0.1,), batch: int = 75776) -> torch.Tensor:
+    """Leave-one-out kNN class rankings of a labelled bank against itself:
+    (len(knn_ks), len(knn_ts), N, num_classes) int64, where [i, j, r] is bitwise
+    ``knn_predict_multi(feature_bank[:, r:r+1].t(), bank without column r, labels without entry r,
+    num_classes, knn_ks, knn_ts)[i, j, 0]`` in the default mode.
+
+    Neighbours are ordered by (sim desc, index asc) and a pair's similarity does not depend on the
+    other bank rows, so deleting row r leaves the order of the others unchanged: the top-k of the
+    bank without r is the full bank's top-(k+1) list with r's own key removed (by index, so an exact
+    duplicate of r stays), or its first k entries when r is not in it.  One search of the bank's
+    rows at max(knn_ks) + 1 per batch of `batch` rows, one ``drop_self`` and one grid vote; the
+    result does not depend on `batch`.  In a raw tensor-core mode a search at k + 1 > MAX_K comes
+    from the exact kernel (as ``knn_predict`` serves k > MAX_K), so k = MAX_K gives the "exact"
+    mode's leave-one-out result there.  feature_bank (D, N) as ``knn_predict`` takes it;
+    max(knn_ks) < N."""
+    ks, ts, order = check_grid(knn_ks, knn_ts)
+    if feature_bank.dim() != 2:
+        raise RuntimeError("mat2 must be a matrix")
+    N = feature_bank.shape[1]
+    if feature_labels.numel() != N:
+        raise RuntimeError(f"feature_labels has {feature_labels.numel()} entries for a bank of {N}")
+    if max(ks) >= N:  # the bank without the row has N - 1 rows
+        raise RuntimeError("selected index k out of range")
+    if int(batch) <= 0:
+        raise ValueError(f"batch must be positive, got {batch}")
+    _require_cuda("feature_bank", feature_bank)
+    _require_cuda("feature_labels", feature_labels)
+    if feature_labels.device != feature_bank.device:
+        raise RuntimeError("Expected all tensors to be on the same device, but found "
+                           f"{feature_bank.device} and {feature_labels.device}")
+    mode = _default_mode
+    C = int(num_classes)
+    labels = feature_labels.long().contiguous().view(-1)
+    parts = loo_parts(tuple(ks[i] for i in order), mode)
+    pred = torch.empty((N, len(ks) * len(ts) * C), dtype=torch.int64, device=feature_bank.device)
+    with torch.cuda.device(feature_bank.device):
+        flag = torch.zeros((1,), dtype=torch.int32, device=feature_bank.device)
+        for lo in range(0, N, int(batch)):
+            hi = min(N, lo + int(batch))
+            q = feature_bank[:, lo:hi].t()  # bank rows lo..hi-1 as (b, D) queries, values unchanged
+            if q.stride(1) != 1:
+                q = q.contiguous()
+            col = 0
+            for part in parts:
+                keys = drop_self(topk_keys(q, feature_bank, part[-1] + 1, mode), lo)
+                _vote_multi_into(keys, labels, C, part, ts, pred[lo:hi, col:], -1, flag)
+                col += len(part) * len(ts) * C
+        _raise_vote_flag(int(flag.item()), C)
+    return grid_view(pred, order, len(ts), C)
 
 
 def grid_view(pred: torch.Tensor, order, n_t: int, num_classes: int) -> torch.Tensor:

@@ -92,22 +92,18 @@ def knn_graph(rows: torch.Tensor, k: int, normalize: bool = True, mode: Optional
     rows are distinct) is dropped unless include_self."""
     fb = FeatureBank.from_rows(rows, normalize=normalize)
     n = fb.n_rows
+    if not include_self and k >= n:
+        raise RuntimeError("knn_graph: k must be smaller than the number of rows")
     kk = min(n, k if include_self else k + 1)
     sims = torch.empty((n, k), dtype=torch.float32, device=rows.device)
     idx = torch.empty((n, k), dtype=torch.int64, device=rows.device)
     for lo in range(0, n, batch):
         hi = min(n, lo + batch)
-        s, i = fb.knn_topk(fb.rows[lo:hi, :fb.dim], kk, mode=mode)
         if include_self:
+            s, i = fb.knn_topk(fb.rows[lo:hi, :fb.dim], kk, mode=mode)
             sims[lo:hi], idx[lo:hi] = s[:, :k], i[:, :k]
             continue
-        # drop the row itself (wherever it ranks among exact duplicates), keep the first k others
-        own = torch.arange(lo, hi, device=rows.device).view(-1, 1)
-        keep = i != own
-        keep &= keep.cumsum(1) <= k
-        short = keep.sum(1) < k
-        if bool(short.any()):  # k + 1 > n: pad with empty slots
-            raise RuntimeError("knn_graph: k must be smaller than the number of rows")
-        sims[lo:hi] = s[keep].view(hi - lo, k)
-        idx[lo:hi] = i[keep].view(hi - lo, k)
+        # drop the row itself by index (wherever it ranks among exact duplicates), else the last key
+        keys = K.topk_keys(fb.rows[lo:hi, :fb.dim], fb.bank, kk, mode)
+        sims[lo:hi], idx[lo:hi] = K.decode_keys(K.drop_self(keys, lo))
     return sims, idx

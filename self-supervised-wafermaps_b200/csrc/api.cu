@@ -352,6 +352,15 @@ int b200knn_merge(const uint64_t* keys_in, int G, int64_t B, int k_in, int k_out
   return e == cudaSuccess ? B200KNN_OK : fail_cuda("merge", e);
 }
 
+int b200knn_drop_self(const uint64_t* keys_in, int64_t B, int k_in, int64_t self_offset, uint64_t* keys_out,
+                      void* stream) {
+  if (!keys_in || !keys_out || B < 0) return fail(B200KNN_E_ARG, "drop_self: bad argument (null pointer or B < 0)");
+  if (k_in < 2) return fail(B200KNN_E_ARG, "drop_self: need k_in >= 2");
+  cudaError_t e = b200knn::launch_drop_self(keys_in, B, k_in, self_offset, keys_out,
+                                            static_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? B200KNN_OK : fail_cuda("drop_self", e);
+}
+
 int b200knn_row_norm_max(const float* rows_a, const float* rows_b, int64_t n, int dim_pad,
                          float* out_dev, void* stream) {
   if (!rows_a || !out_dev || n < 0 || dim_pad <= 0) return fail(B200KNN_E_ARG, "row_norm_max: bad argument");

@@ -30,6 +30,9 @@ cudaError_t launch_merge(const uint64_t* in, int G, int64_t B, int k_in, int k_o
                          cudaStream_t stream);
 cudaError_t launch_decode(const uint64_t* keys, int64_t n, float* sims, int64_t* idx,
                           cudaStream_t stream);
+// (B, k_in) sorted keys -> (B, k_in - 1) without bank row b + self_offset's key (else the last)
+cudaError_t launch_drop_self(const uint64_t* in, int64_t B, int k_in, int64_t self_offset, uint64_t* out,
+                             cudaStream_t stream);
 cudaError_t launch_vote(const uint64_t* keys, const int64_t* labels, int64_t B, int k,
                         int64_t n_labels, int64_t label_offset, int C, double t, int64_t* pred,
                         int64_t pred_ld, int status_col, double* scores, int32_t* err_flag,

@@ -1,5 +1,6 @@
 // select.cu — candidate-list merge (the exchange step of the sharded mode and
-// of bank splits inside one GPU) and key decoding.
+// of bank splits inside one GPU), the self-exclusion of leave-one-out lists and
+// key decoding.
 //
 // Inputs are lists of 64-bit selection keys sorted descending under the
 // canonical (sim desc, idx asc) order, so merging G lists is itself a top-k of
@@ -288,6 +289,43 @@ __global__ void decode_kernel(const uint64_t* __restrict__ keys, int64_t n, floa
   if (idx) idx[i] = key_idx(key);
 }
 
+// One warp per row: (B, k_in) sorted keys -> (B, k_in - 1) without the key of bank row
+// b + self_offset, or without the last key when that row is not in the list (a row need not be
+// among its own nearest neighbours, and an exact duplicate of lower index ranks before it).
+// A ballot finds the self key's position p; each lane stores its key j at j - (j > p).  Empty (0)
+// keys never match.  HBM-bound: 8 B in and 8 B out per key; kAhead chunks are loaded before the
+// first ballot so that several loads per warp are in flight.
+__global__ void __launch_bounds__(256) drop_self_kernel(const uint64_t* __restrict__ in, int64_t B, int k_in,
+                                                        int64_t self_offset, uint64_t* __restrict__ out) {
+  constexpr int kAhead = 4;
+  const int lane = threadIdx.x & 31;
+  const int64_t row = int64_t(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (row >= B) return;
+  const int64_t self = row + self_offset;
+  const uint64_t* src = in + row * k_in;
+  uint64_t* dst = out + row * (k_in - 1);
+  int p = k_in - 1;  // the position dropped: the self key's once found, the last one otherwise
+  bool found = false;
+  for (int j0 = 0; j0 < k_in; j0 += 32 * kAhead) {
+    uint64_t v[kAhead];
+#pragma unroll
+    for (int u = 0; u < kAhead; ++u) {
+      const int j = j0 + u * 32 + lane;
+      v[u] = j < k_in ? src[j] : 0ull;
+    }
+#pragma unroll
+    for (int u = 0; u < kAhead; ++u) {
+      const int j = j0 + u * 32 + lane;
+      const unsigned m = __ballot_sync(kFull, !found && v[u] != 0ull && key_idx(v[u]) == self);
+      if (m) {
+        p = j0 + u * 32 + __ffs(m) - 1;
+        found = true;
+      }
+      if (j < k_in && j != p) dst[j - (j > p ? 1 : 0)] = v[u];
+    }
+  }
+}
+
 __global__ void key_sim_column_kernel(const uint64_t* __restrict__ keys, int64_t B, int k, int j,
                                       float* __restrict__ out) {
   const int64_t b = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -342,6 +380,14 @@ cudaError_t launch_key_sim_column(const uint64_t* keys, int64_t B, int k, int j,
                                   cudaStream_t stream) {
   if (B == 0) return cudaSuccess;
   key_sim_column_kernel<<<unsigned((B + 255) / 256), 256, 0, stream>>>(keys, B, k, j, out);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_drop_self(const uint64_t* in, int64_t B, int k_in, int64_t self_offset, uint64_t* out,
+                             cudaStream_t stream) {
+  if (B == 0) return cudaSuccess;
+  constexpr int kWarps = 8;
+  drop_self_kernel<<<unsigned((B + kWarps - 1) / kWarps), kWarps * 32, 0, stream>>>(in, B, k_in, self_offset, out);
   return cudaGetLastError();
 }
 
