@@ -214,6 +214,8 @@ int b200knn_decode_keys(const uint64_t* keys, int64_t n_keys, float* sims,
  *   err_flag: device int32, set to 1 if any label is outside [0,C) — the
  *             reference raises from scatter in that case (the host shim checks)
  * Scores are sum_j exp(double(sim_j) / double(t)) accumulated in rank order.
+ * Any k (keys are read in chunks of 1024); C <= (51200 - 8*ceil(12*min(k, 1024) / 8)) / 8, i.e.
+ * 4864 for k >= 1024, 6100 at k = 200; a larger C returns B200KNN_E_UNSUPPORTED.
  */
 int b200knn_vote(const uint64_t* keys, const int64_t* labels, int64_t B, int k,
                  int64_t n_labels, int64_t label_offset, int C, double t,
@@ -237,7 +239,8 @@ int b200knn_vote_ex(const uint64_t* keys, const int64_t* labels, int64_t B, int 
  * pred has row stride pred_ld >= n_k*n_t*C; columns [(i*n_t + j)*C, (i*n_t + j + 1)*C) of a row
  * hold exactly what b200knn_vote writes for that row's first ks[i] keys at t = ts[j].
  * status_col: -1, or a column >= n_k*n_t*C for b200knn_vote_ex's status word (bit 0: the
- * k_max-th slot is empty).
+ * k_max-th slot is empty).  Any k_max; C <= (51200 - 16*min(k_max, 1024)) / 8, i.e. 4352 for
+ * k_max >= 1024, 6000 at k_max = 200; a larger C returns B200KNN_E_UNSUPPORTED.
  */
 int b200knn_vote_multi(const uint64_t* keys, const int64_t* labels, int64_t B, int k_max,
                        int64_t n_labels, int64_t label_offset, int C, const int* ks, int n_k,
@@ -352,7 +355,7 @@ int b200knn_scatter_rows(int64_t* dst, int64_t dst_ld, const int64_t* src, int64
  *
  * b200knn_confusion: counts[t*C + p] += #(target == t, pred == p) — the confusion matrix of
  * src/ssl_wafermap/models/knn.py:121-127; macro accuracy / F1 follow from it.  err_flag is
- * set to 1 if a prediction or target lies outside [0, C).  C <= 64.
+ * set to 1 if a prediction or target lies outside [0, C).
  */
 int b200knn_normalize_rows(const void* src, int src_dtype, int64_t n_vec, int dim, int64_t ld,
                            float eps, float* dst_rows, void* stream);

@@ -539,6 +539,7 @@ def vote_packed(keys: torch.Tensor, feature_labels: torch.Tensor, num_classes: i
     lib = _lib.load()
     B, k = keys.shape
     C = int(num_classes)
+    check_vote_classes(C, k)
     labels = feature_labels if feature_labels.dtype == torch.int64 else feature_labels.long()
     labels = labels.contiguous().view(-1)
     dev = keys.device
@@ -1144,6 +1145,7 @@ def vote(keys: torch.Tensor, feature_labels: torch.Tensor, num_classes: int, knn
         labels = labels.long()
     labels = labels.contiguous().view(-1)
     C = int(num_classes)
+    check_vote_classes(C, k)
     dev = keys.device
     pred = torch.empty((B, C), dtype=torch.int64, device=dev)
     scores = torch.empty((B, C), dtype=torch.float64, device=dev) if return_scores else None
@@ -1162,11 +1164,29 @@ def vote(keys: torch.Tensor, feature_labels: torch.Tensor, num_classes: int, knn
 
 
 MAX_GRID_KS, MAX_GRID_TS = 16, 8  # kVoteMaxKs / kVoteMaxTs of csrc/kernels.h
+VOTE_CHUNK, VOTE_SMEM_BYTES, VOTE_WARPS = 1024, 200 * 1024, 4  # kVoteChunk / kVoteSmemBytes, kVoteWarps
+
+
+def vote_max_classes(k: int, grid: bool = False) -> int:
+    """The largest num_classes the vote kernel (grid: the grid vote kernel) serves for lists of k
+    keys.  Keys pass through shared memory in chunks of at most VOTE_CHUNK, so k itself is not
+    bounded; each of the block's VOTE_WARPS rows also keeps C fp64 scores there."""
+    kc = min(int(k), VOTE_CHUNK)
+    keys_bytes = 16 * kc if grid else (12 * kc + 7) // 8 * 8
+    return (VOTE_SMEM_BYTES // VOTE_WARPS - keys_bytes) // 8
+
+
+def check_vote_classes(num_classes: int, k: int, grid: bool = False) -> None:
+    c_max = vote_max_classes(k, grid)
+    if int(num_classes) > c_max:
+        raise ValueError(f"num_classes={int(num_classes)} is more than the {'grid ' if grid else ''}vote serves "
+                         f"at k={int(k)}: at most {c_max} classes")
 
 
 def _vote_multi_into(keys, feature_labels, num_classes, knn_ks, knn_ts, out, status_col, flag) -> None:
     """b200knn_vote_multi of keys (B, knn_ks[-1]) into the (>= B, ld) int64 tensor `out`."""
     B, k = keys.shape
+    check_vote_classes(num_classes, k, grid=True)
     labels = feature_labels if feature_labels.dtype == torch.int64 else feature_labels.long()
     labels = labels.contiguous().view(-1)
     ks = (ctypes.c_int * len(knn_ks))(*[int(x) for x in knn_ks])
@@ -1396,6 +1416,7 @@ def _predict(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t, m
         _check_feature_bank(feature, feature_bank)
         raise RuntimeError(
             f"feature_labels has {feature_labels.numel()} entries for a bank of {feature_bank.shape[1]}")
+    check_vote_classes(num_classes, knn_k, grid=isinstance(knn_t, tuple))
     if mode == "exact" or int(knn_k) > MAX_K:
         return _vote_checked(topk_keys(feature, feature_bank, knn_k, mode), feature_labels, num_classes, knn_t)
     _check_feature_bank(feature, feature_bank)
@@ -1443,8 +1464,11 @@ def knn_predict_multi(feature: torch.Tensor, feature_bank: torch.Tensor, feature
     similarities themselves do not depend on k.  At most 16 values of k and 8 of t, no duplicates."""
     ks, ts, order = check_grid(knn_ks, knn_ts)
     mode = _default_mode
+    searches = grid_parts(tuple(ks[i] for i in order), mode)
+    for part in searches:  # before the first search
+        check_vote_classes(num_classes, part[-1], grid=True)
     parts = [_predict(feature, feature_bank, feature_labels, num_classes, part[-1], (part, tuple(ts)), mode)
-             for part in grid_parts(tuple(ks[i] for i in order), mode)]
+             for part in searches]
     return grid_view(torch.cat(parts, dim=1) if len(parts) > 1 else parts[0], order, len(ts), num_classes)
 
 
@@ -1490,15 +1514,17 @@ def knn_predict_loo(feature_bank: torch.Tensor, feature_labels: torch.Tensor, nu
         raise RuntimeError("selected index k out of range")
     if int(batch) <= 0:
         raise ValueError(f"batch must be positive, got {batch}")
+    mode = _default_mode
+    parts = loo_parts(tuple(ks[i] for i in order), mode)
+    for part in parts:
+        check_vote_classes(num_classes, part[-1], grid=True)
     _require_cuda("feature_bank", feature_bank)
     _require_cuda("feature_labels", feature_labels)
     if feature_labels.device != feature_bank.device:
         raise RuntimeError("Expected all tensors to be on the same device, but found "
                            f"{feature_bank.device} and {feature_labels.device}")
-    mode = _default_mode
     C = int(num_classes)
     labels = feature_labels.long().contiguous().view(-1)
-    parts = loo_parts(tuple(ks[i] for i in order), mode)
     pred = torch.empty((N, len(ks) * len(ts) * C), dtype=torch.int64, device=feature_bank.device)
     with torch.cuda.device(feature_bank.device):
         flag = torch.zeros((1,), dtype=torch.int32, device=feature_bank.device)

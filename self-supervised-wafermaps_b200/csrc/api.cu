@@ -536,7 +536,7 @@ int b200knn_vote_ex(const uint64_t* keys, const int64_t* labels, int64_t B, int 
   if (!(t > 0.0) && !(t < 0.0)) return fail(B200KNN_E_ARG, "vote: temperature must be non-zero");
   cudaError_t e = b200knn::launch_vote(keys, labels, B, k, n_labels, label_offset, C, t, pred, pred_ld,
                                        status_col, scores, err_flag, static_cast<cudaStream_t>(stream));
-  if (e == cudaErrorInvalidValue) return fail(B200KNN_E_UNSUPPORTED, "vote: k/num_classes too large for shared memory");
+  if (e == cudaErrorInvalidValue) return fail(B200KNN_E_UNSUPPORTED, "vote: num_classes too large for shared memory");
   return e == cudaSuccess ? B200KNN_OK : fail_cuda("vote", e);
 }
 
@@ -566,7 +566,7 @@ int b200knn_vote_multi(const uint64_t* keys, const int64_t* labels, int64_t B, i
   cudaError_t e = b200knn::launch_vote_multi(keys, labels, B, n_labels, label_offset, C, grid, pred, pred_ld,
                                              status_col, err_flag, static_cast<cudaStream_t>(stream));
   if (e == cudaErrorInvalidValue)
-    return fail(B200KNN_E_UNSUPPORTED, "vote_multi: k_max/num_classes/temperatures too large for shared memory");
+    return fail(B200KNN_E_UNSUPPORTED, "vote_multi: num_classes too large for shared memory");
   return e == cudaSuccess ? B200KNN_OK : fail_cuda("vote_multi", e);
 }
 
@@ -597,7 +597,6 @@ int b200knn_row_sqnorms(const void* src, int src_dtype, int64_t n_vec, int dim, 
 int b200knn_confusion(const int64_t* pred, const int64_t* target, int64_t n, int C, int64_t* counts,
                       int32_t* err_flag, void* stream) {
   if (!pred || !target || !counts || !err_flag || n < 0 || C <= 0) return fail(B200KNN_E_ARG, "confusion: bad argument");
-  if (C > 64) return fail(B200KNN_E_UNSUPPORTED, "confusion: at most 64 classes");
   cudaError_t e = b200knn::launch_confusion(pred, target, n, C, counts, err_flag, static_cast<cudaStream_t>(stream));
   return e == cudaSuccess ? B200KNN_OK : fail_cuda("confusion", e);
 }

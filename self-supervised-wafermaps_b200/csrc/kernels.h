@@ -33,6 +33,12 @@ cudaError_t launch_decode(const uint64_t* keys, int64_t n, float* sims, int64_t*
 // (B, k_in) sorted keys -> (B, k_in - 1) without bank row b + self_offset's key (else the last)
 cudaError_t launch_drop_self(const uint64_t* in, int64_t B, int k_in, int64_t self_offset, uint64_t* out,
                              cudaStream_t stream);
+// The vote kernels stream a row's keys through shared memory in chunks of at most kVoteChunk, so
+// k is unbounded; the per-warp fp64 score array of C classes is not.  A launch whose shared
+// memory, 4 warps x (chunk arrays + 8 C bytes), exceeds kVoteSmemBytes returns
+// cudaErrorInvalidValue (b200knn/knn.py restates the bound as vote_max_classes).
+constexpr int kVoteChunk = 1024;
+constexpr int kVoteSmemBytes = 200 * 1024;
 cudaError_t launch_vote(const uint64_t* keys, const int64_t* labels, int64_t B, int k,
                         int64_t n_labels, int64_t label_offset, int C, double t, int64_t* pred,
                         int64_t pred_ld, int status_col, double* scores, int32_t* err_flag,
@@ -59,7 +65,7 @@ cudaError_t launch_normalize_rows(const void* src, int src_dtype, int64_t n_vec,
                                   float eps, float* dst, cudaStream_t stream);
 cudaError_t launch_row_sqnorm(const void* src, int src_dtype, int64_t n_vec, int dim, int64_t ld, float* out,
                               cudaStream_t stream);
-// confusion-matrix counts (vote.cu): counts (C,C) int64 += histogram of (target, pred)
+// confusion-matrix counts (vote.cu): counts (C,C) int64 += histogram of (target, pred); any C
 cudaError_t launch_confusion(const int64_t* pred, const int64_t* target, int64_t n, int C, int64_t* counts,
                              int32_t* err_flag, cudaStream_t stream);
 

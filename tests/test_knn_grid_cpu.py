@@ -63,6 +63,32 @@ def test_python_argument_errors(ks, ts, match):
         b200knn.ShardedBank(bank, lab, bank.shape[1], ops=_GridOps).knn_predict_multi(f, c["C"], ks, ts)
 
 
+@pytest.mark.parametrize("k", [1, 200, 1023, 1024, 5000])
+def test_vote_class_bound_without_gpu(k):
+    """One class past vote_max_classes: B200KNN_E_UNSUPPORTED from the C ABI (refused before any CUDA
+    call), a ValueError naming the bound from Python before any tensor reaches the device."""
+    from b200knn import knn as K
+
+    lib = _lib.load()
+    for grid in (False, True):
+        C = K.vote_max_classes(k, grid) + 1
+        if grid:
+            rc = lib.b200knn_vote_multi(1, 1, 4, k, 10, 0, C, *_grid_args((k,), (0.1,)), 1, C, -1, 1, None)
+        else:
+            rc = lib.b200knn_vote(1, 1, 4, k, 10, 0, C, 0.1, 1, None, 1, None)
+        assert rc == -4 and b"num_classes too large" in lib.b200knn_last_error(), (grid, rc)
+    # the figures include/b200knn.h and DESIGN.md quote
+    assert [K.vote_max_classes(kk, g) for g in (False, True) for kk in (200, 5000)] == [6100, 4864, 6000, 4352]
+    c = datagen.make_case("ragged")
+    f, bank, lab = (torch.from_numpy(c[n]) for n in ("feature", "bank", "labels"))
+    g1 = K.vote_max_classes(k, True) + 1
+    if k < bank.shape[1]:
+        with pytest.raises(ValueError, match=f"at most {g1 - 1} classes"):
+            b200knn.knn_predict_multi(f, bank, lab, g1, (k,), (0.1,))
+        with pytest.raises(ValueError, match=f"at most {g1 - 1} classes"):
+            b200knn.knn_predict_loo(bank, lab, g1, (k,), (0.1,))
+
+
 def test_cpu_tensors_raise():
     c = datagen.make_case("ragged")
     f, bank, lab = (torch.from_numpy(c[n]) for n in ("feature", "bank", "labels"))
