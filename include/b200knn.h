@@ -199,6 +199,25 @@ int b200knn_merge(const uint64_t* keys_in, int G, int64_t B, int k_in, int k_out
 int b200knn_drop_self(const uint64_t* keys_in, int64_t B, int k_in, int64_t self_offset,
                       uint64_t* keys_out, void* stream);
 
+/*
+ * Leave-one-group-out lists (no counterpart in the reference; replaces one bank preparation and
+ * search per group): row b of a search of bank row row_ids[b] against the whole bank, without
+ * every row of that row's group.
+ *   keys_in  : (B, k_in) uint64, each row sorted descending, k_in >= k_out
+ *   row_ids  : (B,) int64, the bank row each list belongs to
+ *   group_ids: (N,) int32, the group of every bank row (the key's index field, idx_offset included)
+ *   keys_out : (B, k_out) uint64, must not overlap keys_in: the first k_out keys of row b whose
+ *              group_ids entry differs from group_ids[row_ids[b]], in order; zero-filled when fewer
+ *              survive.  Empty (0) keys are never dropped.
+ *   err_flag : int32[1], set to 2 when a key index or row id is outside [0, N); such a key is
+ *              kept, and a row id outside [0, N) drops nothing.  Keys after the k_out-th survivor
+ *              may be left unread (and unchecked).
+ * k_out >= 1; B == 0 launches nothing.
+ */
+int b200knn_drop_group(const uint64_t* keys_in, int64_t B, int k_in, const int64_t* row_ids,
+                       const int32_t* group_ids, int64_t N, int k_out, uint64_t* keys_out,
+                       int32_t* err_flag, void* stream);
+
 /* keys (B,k) -> sims (B,k) f32 and idx (B,k) int64  (Tensor.topk's two outputs).
  * Empty slots (fewer than k finite candidates) decode to sim=-inf, idx=-1. */
 int b200knn_decode_keys(const uint64_t* keys, int64_t n_keys, float* sims,

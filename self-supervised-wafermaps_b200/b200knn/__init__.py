@@ -5,8 +5,9 @@ faris-k/self-supervised-wafermaps (lightly's ``knn_predict`` as called from
 Public surface (mirrors the reference names for this path):
     knn_predict(feature, feature_bank, feature_labels, num_classes, knn_k=200, knn_t=0.1)
     knn_predict_multi(..., knn_ks, knn_ts)        -> knn_predict over a (k, t) grid, one search
-    knn_predict_loo(feature_bank, feature_labels, num_classes, knn_ks, knn_ts)
-                                                  -> leave-one-out grid of the bank against itself
+    knn_predict_loo(feature_bank, feature_labels, num_classes, knn_ks, knn_ts, groups=None)
+                                                  -> leave-one-out (or leave-one-group-out) grid of the
+                                                     bank against itself
     knn_topk(feature, feature_bank, k)            -> (sims, idx)
     install() / uninstall()                       -> rebind lightly's symbol
     ShardedBank                                   -> bank row-sharded over the GPUs of a node

@@ -115,12 +115,14 @@ class FeatureBank:
         return K.knn_predict_multi(self._queries(feature, normalize), self.bank, self.labels, num_classes,
                                    knn_ks, knn_ts)
 
-    def knn_predict_loo(self, num_classes: int, knn_ks=(200,), knn_ts=(0.1,), batch: int = 75776) -> torch.Tensor:
+    def knn_predict_loo(self, num_classes: int, knn_ks=(200,), knn_ts=(0.1,), batch: int = 75776,
+                        groups: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Leave-one-out class rankings of the bank's own rows and labels (``K.knn_predict_loo``):
-        (len(knn_ks), len(knn_ts), N, C).  The queries are views of the padded rows, no copy."""
+        (len(knn_ks), len(knn_ts), N, C).  The queries are views of the padded rows, no copy.
+        groups: (N,) integer ids, each row's whole group left out of its vote."""
         if self.labels is None:
             raise RuntimeError("this FeatureBank was built without labels")
-        return K.knn_predict_loo(self.bank, self.labels, num_classes, knn_ks, knn_ts, batch)
+        return K.knn_predict_loo(self.bank, self.labels, num_classes, knn_ks, knn_ts, batch, groups)
 
     def knn_topk(self, feature: torch.Tensor, k: int, normalize: bool = False, mode: Optional[str] = None):
         return K.knn_topk(self._queries(feature, normalize), self.bank, k, mode)

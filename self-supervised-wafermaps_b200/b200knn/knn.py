@@ -1119,6 +1119,39 @@ def drop_self(keys: torch.Tensor, self_offset: int) -> torch.Tensor:
     return out
 
 
+def drop_group(keys: torch.Tensor, row_ids: torch.Tensor, group_ids: torch.Tensor, k_out: int,
+               flag: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """(B, k_in) sorted keys of bank rows row_ids (B,) searched against their own bank, group_ids
+    (N,) int32 the group of every bank row -> (B, k_out): the first k_out keys of row b outside the
+    group of bank row row_ids[b], zero-filled when fewer survive (``b200knn_drop_group``).  A key
+    index or row id outside [0, N) sets the device int32[1] `flag` to 2; without a flag it raises."""
+    _require_cuda("keys", keys)
+    if group_ids.dtype != torch.int32:
+        raise ValueError(f"group_ids must be int32, got {group_ids.dtype}")
+    B, k_in = keys.shape
+    if row_ids.numel() != B:
+        raise RuntimeError(f"row_ids has {row_ids.numel()} entries for {B} rows of keys")
+    if flag is not None and (flag.dtype != torch.int32 or flag.numel() < 1):
+        raise ValueError("flag must be a device int32 tensor of at least one element")
+    for t in (row_ids, group_ids) + (() if flag is None else (flag,)):
+        if t.device != keys.device:
+            raise RuntimeError(f"Expected all tensors to be on the same device, but found {keys.device} and {t.device}")
+    keys = keys.contiguous()
+    row_ids = row_ids.to(torch.int64).contiguous().view(-1)
+    group_ids = group_ids.contiguous().view(-1)
+    out = torch.empty((B, int(k_out)), dtype=torch.int64, device=keys.device)
+    check = flag is None
+    with torch.cuda.device(keys.device):
+        if check:
+            flag = torch.zeros((1,), dtype=torch.int32, device=keys.device)
+        _lib.check(_lib.load().b200knn_drop_group(keys.data_ptr(), B, k_in, row_ids.data_ptr(), group_ids.data_ptr(),
+                                                  group_ids.numel(), int(k_out), out.data_ptr(), flag.data_ptr(),
+                                                  _stream()), "drop_group")
+        if check and int(flag.item()):
+            raise RuntimeError("drop_group: a key index or row id is outside the group ids")
+    return out
+
+
 def merge_keys(keys_in: torch.Tensor, k_out: int) -> torch.Tensor:
     """(G,B,k_in) sorted candidate lists -> (B,k_out): the shard-merge step."""
     lib = _lib.load()
@@ -1488,8 +1521,76 @@ def loo_parts(ks_ascending: tuple, mode: str) -> list:
     return [tuple(k - 1 for k in part) for part in grid_parts(tuple(k + 1 for k in ks_ascending), mode)]
 
 
+def logo_parts(ks_ascending: tuple, p: int, n: int, mode: str) -> list:
+    """The searches of the leave-one-group-out rows whose group size g has p = the smallest power of
+    two >= g, in a bank of n rows: k is searched at depth min(n, k + p), and the ks are split by
+    ``grid_parts``' rule applied to those depths, so a raw tensor-core mode never asks its kernel for
+    more than MAX_K keys.  p = 1 is ``loo_parts``."""
+    n_lo = len(grid_parts(tuple(min(n, k + p) for k in ks_ascending), mode)[0])
+    return [tuple(ks_ascending)] if n_lo == len(ks_ascending) else [tuple(ks_ascending[:n_lo]),
+                                                                    tuple(ks_ascending[n_lo:])]
+
+
+_GROUP_DTYPES = (torch.uint8, torch.int8, torch.int16, torch.int32, torch.int64)
+_GROUP_DTYPES_WIDENED = (torch.uint16, torch.uint32)  # to int64, losslessly
+
+
+def _group_plan(groups: torch.Tensor, n: int, device: torch.device):
+    """The buckets of a leave-one-group-out search: (dense int32 group ids (n,), largest group size,
+    rows (n,) int64 in bucket order, [(p, lo, hi)]) where positions [lo, hi) of `rows` hold, in
+    ascending order, the rows whose group size g has p = the smallest power of two >= g, p
+    ascending.  One torch.unique and one host read of the group statistics."""
+    if groups.numel() != n:
+        raise RuntimeError(f"groups has {groups.numel()} entries for a bank of {n}")
+    if groups.dtype not in _GROUP_DTYPES + _GROUP_DTYPES_WIDENED + (torch.uint64,):
+        raise ValueError(f"groups must be an integer tensor, got {groups.dtype}")
+    if groups.device != device:
+        raise RuntimeError(f"Expected all tensors to be on the same device, but found {device} and {groups.device}")
+    groups = groups.reshape(-1)
+    if groups.dtype in _GROUP_DTYPES_WIDENED:
+        groups = groups.to(torch.int64)
+    elif groups.dtype == torch.uint64:  # the same bits as int64: equal ids stay equal, distinct ones distinct
+        groups = groups.view(torch.int64)
+    _, inv, cnt = torch.unique(groups, return_inverse=True, return_counts=True)
+    e_group = torch.frexp((cnt - 1).double()).exponent.long()  # the bit length of g - 1: p = 2**e
+    rows = torch.sort(e_group[inv], stable=True).indices
+    rows_per_e = torch.zeros((64,), dtype=torch.int64, device=cnt.device).scatter_add_(0, e_group, cnt)
+    stats = torch.cat([cnt.max().view(1), rows_per_e]).tolist()
+    buckets, lo = [], 0
+    for e, m in enumerate(stats[1:]):
+        if m:
+            buckets.append((1 << e, lo, lo + m))
+            lo += m
+    return inv.to(torch.int32), stats[0], rows, buckets
+
+
+def _group_searches(feature_bank: torch.Tensor, plan, ks_ascending: tuple, mode: str, batch: int,
+                    flag: torch.Tensor):
+    """Yields (part, lo, hi, keys) for every search of a leave-one-group-out pass over the bank's own
+    rows: keys (hi - lo, part[-1]) are the lists of rows plan[2][lo:hi] without their groups.  Each
+    search runs one ``topk_keys`` at depth min(N, part[-1] + p) (every mode, cascade and repair) and
+    one ``drop_group``; it takes max(1, min(batch, batch * (part[-1] + 1) // depth)) rows, so its key
+    buffer is no larger than that of a leave-one-out search of `batch` rows."""
+    gid, _, rows, buckets = plan
+    n = feature_bank.shape[1]
+    bank_rows = feature_bank.t()
+    whole = len(buckets) == 1  # rows is arange(n): the queries are views
+    for p, b_lo, b_hi in buckets:
+        for part in logo_parts(ks_ascending, p, n, mode):
+            depth = min(n, part[-1] + p)
+            step = max(1, min(batch, batch * (part[-1] + 1) // depth))
+            for lo in range(b_lo, b_hi, step):
+                hi = min(b_hi, lo + step)
+                q = bank_rows[lo:hi] if whole else bank_rows.index_select(0, rows[lo:hi])
+                if q.stride(1) != 1:
+                    q = q.contiguous()
+                yield part, lo, hi, drop_group(topk_keys(q, feature_bank, depth, mode), rows[lo:hi], gid, part[-1],
+                                               flag)
+
+
 def knn_predict_loo(feature_bank: torch.Tensor, feature_labels: torch.Tensor, num_classes: int,
-                    knn_ks=(200,), knn_ts=(0.1,), batch: int = 75776) -> torch.Tensor:
+                    knn_ks=(200,), knn_ts=(0.1,), batch: int = 75776,
+                    groups: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Leave-one-out kNN class rankings of a labelled bank against itself:
     (len(knn_ks), len(knn_ts), N, num_classes) int64, where [i, j, r] is bitwise
     ``knn_predict_multi(feature_bank[:, r:r+1].t(), bank without column r, labels without entry r,
@@ -1503,13 +1604,20 @@ def knn_predict_loo(feature_bank: torch.Tensor, feature_labels: torch.Tensor, nu
     result does not depend on `batch`.  In a raw tensor-core mode a search at k + 1 > MAX_K comes
     from the exact kernel (as ``knn_predict`` serves k > MAX_K), so k = MAX_K gives the "exact"
     mode's leave-one-out result there.  feature_bank (D, N) as ``knn_predict`` takes it;
-    max(knn_ks) < N."""
+    max(knn_ks) < N.
+
+    groups: optional (N,) integer ids (any values and integer dtype, on the bank's device) for
+    leave-one-group-out: [i, j, r] is then the same call against the bank without every column c
+    with groups[c] == groups[r] (``_knn_predict_logo``); groups=None is the path above, and
+    groups=torch.arange(N) gives its result bitwise."""
     ks, ts, order = check_grid(knn_ks, knn_ts)
     if feature_bank.dim() != 2:
         raise RuntimeError("mat2 must be a matrix")
     N = feature_bank.shape[1]
     if feature_labels.numel() != N:
         raise RuntimeError(f"feature_labels has {feature_labels.numel()} entries for a bank of {N}")
+    if groups is not None:
+        return _knn_predict_logo(feature_bank, feature_labels, num_classes, ks, ts, order, batch, groups)
     if max(ks) >= N:  # the bank without the row has N - 1 rows
         raise RuntimeError("selected index k out of range")
     if int(batch) <= 0:
@@ -1538,6 +1646,46 @@ def knn_predict_loo(feature_bank: torch.Tensor, feature_labels: torch.Tensor, nu
                 keys = drop_self(topk_keys(q, feature_bank, part[-1] + 1, mode), lo)
                 _vote_multi_into(keys, labels, C, part, ts, pred[lo:hi, col:], -1, flag)
                 col += len(part) * len(ts) * C
+        _raise_vote_flag(int(flag.item()), C)
+    return grid_view(pred, order, len(ts), C)
+
+
+def _knn_predict_logo(feature_bank, feature_labels, num_classes, ks, ts, order, batch, groups) -> torch.Tensor:
+    """``knn_predict_loo`` with every row's whole group left out.  Deleting G(r), the rows of r's
+    group, leaves the (sim desc, index asc) order of the others unchanged, and at most g(r) = |G(r)|
+    keys of a list are in G(r), so the top-k of the bank without G(r) is the full bank's
+    top-(k + g(r)) list without the members of G(r), cut to k.  The search depth is min(N, k + p) with p the smallest
+    power of two >= g(r), a function of the row alone, so the result does not depend on `batch`:
+    rows are searched in buckets of equal p (``logo_parts``, ``_group_searches``) and voted into a
+    bucket-ordered buffer that one permutation puts back in row order.  In a raw tensor-core mode a
+    search deeper than MAX_K comes from the exact kernel, so such rows get the "exact" mode's
+    result.  max(knn_ks) <= N - (largest group size).  One host read of the group statistics after
+    torch.unique and one of the label flag."""
+    N = feature_bank.shape[1]
+    if int(batch) <= 0:
+        raise ValueError(f"batch must be positive, got {batch}")
+    # the class bound falls with k, so the search ending at max(knn_ks) is the worst part of any bucket
+    check_vote_classes(num_classes, max(ks), grid=True)
+    plan = _group_plan(groups, N, feature_bank.device)
+    if max(ks) > N - plan[1]:  # the bank without the largest group has N - g_max rows
+        raise RuntimeError("selected index k out of range")
+    mode = _default_mode
+    ks_ascending = tuple(ks[i] for i in order)
+    _require_cuda("feature_bank", feature_bank)
+    _require_cuda("feature_labels", feature_labels)
+    if feature_labels.device != feature_bank.device:
+        raise RuntimeError("Expected all tensors to be on the same device, but found "
+                           f"{feature_bank.device} and {feature_labels.device}")
+    C = int(num_classes)
+    labels = feature_labels.long().contiguous().view(-1)
+    pred = torch.empty((N, len(ks) * len(ts) * C), dtype=torch.int64, device=feature_bank.device)
+    with torch.cuda.device(feature_bank.device):
+        flag = torch.zeros((1,), dtype=torch.int32, device=feature_bank.device)
+        for part, lo, hi, keys in _group_searches(feature_bank, plan, ks_ascending, mode, int(batch), flag):
+            col = ks_ascending.index(part[0]) * len(ts) * C
+            _vote_multi_into(keys, labels, C, part, ts, pred[lo:hi, col:], -1, flag)
+        if len(plan[3]) > 1:  # bucket order -> row order
+            pred = torch.empty_like(pred).index_copy_(0, plan[2], pred)
         _raise_vote_flag(int(flag.item()), C)
     return grid_view(pred, order, len(ts), C)
 

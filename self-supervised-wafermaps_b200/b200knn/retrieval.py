@@ -84,14 +84,36 @@ def l2_topk(data_rows: torch.Tensor, queries: torch.Tensor, k: int, mode: Option
 
 
 def knn_graph(rows: torch.Tensor, k: int, normalize: bool = True, mode: Optional[str] = None,
-              batch: int = 75776, include_self: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
+              batch: int = 75776, include_self: bool = False,
+              groups: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
     """k nearest neighbours (cosine when normalize=True) of EVERY row among all rows — the graph
     UMAP / HDBSCAN build from the embeddings (``notebooks/3.0-Embeddings-inference.ipynb:208-216``,
     ``3.2-Embeddings-SSL-categories.ipynb:51-53``; BASELINE.json config "811k x 512, top-10 for all
     811k queries").  Returns (sims (N,k) fp32, idx (N,k) int64); a row's own entry (rank 0 when
-    rows are distinct) is dropped unless include_self."""
+    rows are distinct) is dropped unless include_self.  groups: optional (N,) integer ids (lots,
+    duplicate hashes); a row's k neighbours then exclude every row of its group, through the
+    leave-one-group-out search of ``knn_predict_loo``; k <= N - (largest group size)."""
+    if groups is not None:
+        if include_self:
+            raise ValueError("knn_graph: groups leaves a row's whole group out, so include_self must be False")
+        plan = K._group_plan(groups, rows.shape[0], rows.device)
+        if k > rows.shape[0] - plan[1]:
+            raise RuntimeError("knn_graph: k must be smaller than the number of rows outside a row's group")
     fb = FeatureBank.from_rows(rows, normalize=normalize)
     n = fb.n_rows
+    if groups is not None:
+        sims = torch.empty((n, k), dtype=torch.float32, device=rows.device)
+        idx = torch.empty((n, k), dtype=torch.int64, device=rows.device)
+        flag = torch.zeros((1,), dtype=torch.int32, device=rows.device)
+        for _, lo, hi, keys in K._group_searches(fb.bank, plan, (int(k),), mode or K.get_default_mode(), batch,
+                                                 flag):
+            sims[lo:hi], idx[lo:hi] = K.decode_keys(keys)
+        if len(plan[3]) > 1:  # bucket order -> row order
+            sims = torch.empty_like(sims).index_copy_(0, plan[2], sims)
+            idx = torch.empty_like(idx).index_copy_(0, plan[2], idx)
+        if int(flag.item()):
+            raise RuntimeError("knn_graph: a neighbour index is outside the group ids")
+        return sims, idx
     if not include_self and k >= n:
         raise RuntimeError("knn_graph: k must be smaller than the number of rows")
     kk = min(n, k if include_self else k + 1)

@@ -361,6 +361,17 @@ int b200knn_drop_self(const uint64_t* keys_in, int64_t B, int k_in, int64_t self
   return e == cudaSuccess ? B200KNN_OK : fail_cuda("drop_self", e);
 }
 
+int b200knn_drop_group(const uint64_t* keys_in, int64_t B, int k_in, const int64_t* row_ids,
+                       const int32_t* group_ids, int64_t N, int k_out, uint64_t* keys_out, int32_t* err_flag,
+                       void* stream) {
+  if (!keys_in || !row_ids || !group_ids || !keys_out || !err_flag || B < 0 || N < 0)
+    return fail(B200KNN_E_ARG, "drop_group: bad argument (null pointer, B < 0 or N < 0)");
+  if (k_out < 1 || k_in < k_out) return fail(B200KNN_E_ARG, "drop_group: need 1 <= k_out <= k_in");
+  cudaError_t e = b200knn::launch_drop_group(keys_in, B, k_in, row_ids, group_ids, N, k_out, keys_out, err_flag,
+                                             static_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? B200KNN_OK : fail_cuda("drop_group", e);
+}
+
 int b200knn_row_norm_max(const float* rows_a, const float* rows_b, int64_t n, int dim_pad,
                          float* out_dev, void* stream) {
   if (!rows_a || !out_dev || n < 0 || dim_pad <= 0) return fail(B200KNN_E_ARG, "row_norm_max: bad argument");

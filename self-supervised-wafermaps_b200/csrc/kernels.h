@@ -33,6 +33,11 @@ cudaError_t launch_decode(const uint64_t* keys, int64_t n, float* sims, int64_t*
 // (B, k_in) sorted keys -> (B, k_in - 1) without bank row b + self_offset's key (else the last)
 cudaError_t launch_drop_self(const uint64_t* in, int64_t B, int k_in, int64_t self_offset, uint64_t* out,
                              cudaStream_t stream);
+// (B, k_in) sorted keys -> (B, k_out): the first k_out keys outside row row_ids[b]'s group
+// (group_ids (N,)), zero-filled; err_flag = 2 on a key index or row id outside [0, N)
+cudaError_t launch_drop_group(const uint64_t* in, int64_t B, int k_in, const int64_t* row_ids,
+                              const int32_t* group_ids, int64_t N, int k_out, uint64_t* out, int32_t* err_flag,
+                              cudaStream_t stream);
 // The vote kernels stream a row's keys through shared memory in chunks of at most kVoteChunk, so
 // k is unbounded; the per-warp fp64 score array of C classes is not.  A launch whose shared
 // memory, 4 warps x (chunk arrays + 8 C bytes), exceeds kVoteSmemBytes returns

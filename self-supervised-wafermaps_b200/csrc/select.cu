@@ -1,6 +1,6 @@
 // select.cu — candidate-list merge (the exchange step of the sharded mode and
-// of bank splits inside one GPU), the self-exclusion of leave-one-out lists and
-// key decoding.
+// of bank splits inside one GPU), the self- and group-exclusion of leave-one-out
+// lists and key decoding.
 //
 // Inputs are lists of 64-bit selection keys sorted descending under the
 // canonical (sim desc, idx asc) order, so merging G lists is itself a top-k of
@@ -326,6 +326,62 @@ __global__ void __launch_bounds__(256) drop_self_kernel(const uint64_t* __restri
   }
 }
 
+// One warp per row: (B, k_in) sorted keys -> (B, k_out), the first k_out keys whose bank row is
+// not in the group of bank row row_ids[b], in order, zero-filled when fewer survive (leave-one-
+// group-out lists).  Each lane gathers group_ids[key index] (4 B per bank row: 3.2 MB at
+// N = 811k, so L2-resident) and compares it with the row's own id; a ballot plus a prefix
+// popcount gives each survivor its output position.  Empty (0) keys are never dropped.  A key
+// index or row id outside [0, N) sets *err_flag = 2 (the vote's "index outside the labels"); such
+// a key is kept, such a row drops nothing.  kAhead chunks (and their group gathers) are issued
+// before the first ballot, as in drop_self_kernel.  The warp stops after the chunk group in which
+// the k_out-th survivor appears (a row of a large group searched at k + p keeps k keys): keys past
+// it are neither read nor checked.
+__global__ void __launch_bounds__(256) drop_group_kernel(const uint64_t* __restrict__ in, int64_t B, int k_in,
+                                                         const int64_t* __restrict__ row_ids,
+                                                         const int32_t* __restrict__ group_ids, int64_t N,
+                                                         int k_out, uint64_t* __restrict__ out,
+                                                         int32_t* __restrict__ err_flag) {
+  constexpr int kAhead = 4;
+  const int lane = threadIdx.x & 31;
+  const int64_t row = int64_t(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (row >= B) return;
+  const uint64_t* src = in + row * k_in;
+  uint64_t* dst = out + row * k_out;
+  const int64_t self = row_ids[row];
+  const bool self_ok = self >= 0 && self < N;
+  const int32_t own = self_ok ? group_ids[self] : 0;
+  bool bad = !self_ok;
+  const unsigned lt_mask = (1u << lane) - 1u;
+  int n = 0;  // survivors so far (warp-uniform)
+  for (int j0 = 0; j0 < k_in && n < k_out; j0 += 32 * kAhead) {
+    uint64_t v[kAhead];
+#pragma unroll
+    for (int u = 0; u < kAhead; ++u) {
+      const int j = j0 + u * 32 + lane;
+      v[u] = j < k_in ? src[j] : 0ull;
+    }
+    bool keep[kAhead];
+#pragma unroll
+    for (int u = 0; u < kAhead; ++u) {
+      keep[u] = j0 + u * 32 + lane < k_in;
+      if (v[u] != 0ull) {
+        const int64_t i = key_idx(v[u]);
+        if (i < N) keep[u] &= !(self_ok && group_ids[i] == own);  // key_idx of a non-empty key is >= 0
+        else bad = true;
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < kAhead; ++u) {
+      const unsigned m = __ballot_sync(kFull, keep[u]);
+      const int pos = n + __popc(m & lt_mask);
+      if (keep[u] && pos < k_out) dst[pos] = v[u];
+      n += __popc(m);
+    }
+  }
+  for (int j = n + lane; j < k_out; j += 32) dst[j] = 0ull;
+  if (bad) atomicExch(err_flag, 2);
+}
+
 __global__ void key_sim_column_kernel(const uint64_t* __restrict__ keys, int64_t B, int k, int j,
                                       float* __restrict__ out) {
   const int64_t b = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -388,6 +444,16 @@ cudaError_t launch_drop_self(const uint64_t* in, int64_t B, int k_in, int64_t se
   if (B == 0) return cudaSuccess;
   constexpr int kWarps = 8;
   drop_self_kernel<<<unsigned((B + kWarps - 1) / kWarps), kWarps * 32, 0, stream>>>(in, B, k_in, self_offset, out);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_drop_group(const uint64_t* in, int64_t B, int k_in, const int64_t* row_ids,
+                              const int32_t* group_ids, int64_t N, int k_out, uint64_t* out, int32_t* err_flag,
+                              cudaStream_t stream) {
+  if (B == 0) return cudaSuccess;
+  constexpr int kWarps = 8;
+  drop_group_kernel<<<unsigned((B + kWarps - 1) / kWarps), kWarps * 32, 0, stream>>>(
+      in, B, k_in, row_ids, group_ids, N, k_out, out, err_flag);
   return cudaGetLastError();
 }
 
