@@ -134,6 +134,30 @@ int b200knn_topk_exact_below(const void* q, int q_dtype, int64_t q_ld, const voi
                              int64_t idx_offset, const uint64_t* upper_keys, uint64_t* out_keys,
                              void* workspace, size_t workspace_bytes, void* stream);
 
+/*
+ * Group-excluding searches (no counterpart in the reference; k-fold cross-validation and held-out
+ * queries whose group also has rows in the bank): b200knn_topk, except that bank row n is never
+ * admitted to query row b's list when bank_groups[n] == q_groups[b].  Order, key format and indices
+ * (idx_offset included) are unchanged; a row with fewer than k eligible bank rows gets empty (0)
+ * trailing slots.
+ *   q_groups   : (B,) int32 group id of every query row
+ *   bank_groups: (N,) int32 group id of every bank row, indexed before idx_offset
+ * Both must be non-null (B200KNN_E_ARG otherwise).
+ * b200knn_topk_excl      : the tensor-core modes (operands as b200knn_topk_ex; no sampling
+ *                          threshold, no row stride).
+ * b200knn_topk_exact_excl: MODE_EXACT, arguments as b200knn_topk_exact_below (upper_keys may be
+ *                          NULL), so peeled passes for k > 992 exclude the groups too.
+ */
+int b200knn_topk_excl(int mode, const void* q_hi, const void* q_lo, const void* bank_hi,
+                      const void* bank_lo, int64_t B, int64_t N, int dim, int k, int64_t idx_offset,
+                      const int32_t* q_groups, const int32_t* bank_groups, uint64_t* out_keys,
+                      void* workspace, size_t workspace_bytes, void* stream);
+int b200knn_topk_exact_excl(const void* q, int q_dtype, int64_t q_ld, const void* bank, int bank_dtype,
+                            int bank_layout, int64_t bank_ld, int64_t B, int64_t N, int dim, int k,
+                            int64_t idx_offset, const int32_t* q_groups, const int32_t* bank_groups,
+                            const uint64_t* upper_keys, uint64_t* out_keys, void* workspace,
+                            size_t workspace_bytes, void* stream);
+
 int b200knn_topk_ex(int mode, const void* q_hi, const void* q_lo,
                     const void* bank_hi, const void* bank_lo, int64_t B,
                     int64_t n_visit, int dim, int k, int64_t idx_offset,

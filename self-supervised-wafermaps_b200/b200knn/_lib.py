@@ -41,6 +41,16 @@ SIGNATURES = {
         [c_void_p, c_int, c_int64, c_void_p, c_int, c_int, c_int64, c_int64, c_int64, c_int, c_int, c_int64,
          c_void_p, c_void_p, c_void_p, c_size_t, c_void_p],
     ),
+    "b200knn_topk_excl": (
+        c_int,
+        [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_int64, c_void_p, c_void_p,
+         c_void_p, c_void_p, c_size_t, c_void_p],
+    ),
+    "b200knn_topk_exact_excl": (
+        c_int,
+        [c_void_p, c_int, c_int64, c_void_p, c_int, c_int, c_int64, c_int64, c_int64, c_int, c_int, c_int64,
+         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p],
+    ),
     "b200knn_topk_ex": (
         c_int,
         [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_int64, c_int64,
@@ -129,6 +139,7 @@ KERNELS_PER_CALL = {
     "b200knn_merge": 1, "b200knn_decode_keys": 1, "b200knn_drop_self": 1, "b200knn_drop_group": 1, "b200knn_vote": 1, "b200knn_vote_ex": 1, "b200knn_vote_multi": 1,
     "b200knn_key_sim_column": 1, "b200knn_normalize_rows": 1, "b200knn_confusion": 1, "b200knn_row_sqnorms": 1, "b200knn_rescore": 2, "b200knn_route_keys": 1, "b200knn_certify": 1,
     "b200knn_row_norm_max": 1, "b200knn_debug_topk_dump": 1, "b200knn_topk_exact_below": 1,
+    "b200knn_topk_excl": 1, "b200knn_topk_exact_excl": 1,
     "b200knn_topk_sample_scatter": 1, "b200knn_broadcast_f32": 1,
     "b200knn_route_scatter": 1, "b200knn_rescore_scatter": 2, "b200knn_compact_rows": 1, "b200knn_scatter_rows": 1,
 }

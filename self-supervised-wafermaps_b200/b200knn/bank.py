@@ -107,13 +107,15 @@ class FeatureBank:
         return K.knn_predict(self._queries(feature, normalize), self.bank, self.labels, num_classes, knn_k, knn_t)
 
     def knn_predict_multi(self, feature: torch.Tensor, num_classes: int, knn_ks=(200,), knn_ts=(0.1,),
-                          normalize: bool = False) -> torch.Tensor:
+                          normalize: bool = False, query_groups: Optional[torch.Tensor] = None,
+                          bank_groups: Optional[torch.Tensor] = None) -> torch.Tensor:
         """``knn_predict`` over a (knn_ks, knn_ts) grid from one neighbour search (``K.knn_predict_multi``):
-        (len(knn_ks), len(knn_ts), B, C); normalize=True fuses the query ``F.normalize``."""
+        (len(knn_ks), len(knn_ts), B, C); normalize=True fuses the query ``F.normalize``.
+        query_groups (B,) / bank_groups (N,): each query's group left out of its search."""
         if self.labels is None:
             raise RuntimeError("this FeatureBank was built without labels")
         return K.knn_predict_multi(self._queries(feature, normalize), self.bank, self.labels, num_classes,
-                                   knn_ks, knn_ts)
+                                   knn_ks, knn_ts, query_groups, bank_groups)
 
     def knn_predict_loo(self, num_classes: int, knn_ks=(200,), knn_ts=(0.1,), batch: int = 75776,
                         groups: Optional[torch.Tensor] = None) -> torch.Tensor:
@@ -124,5 +126,6 @@ class FeatureBank:
             raise RuntimeError("this FeatureBank was built without labels")
         return K.knn_predict_loo(self.bank, self.labels, num_classes, knn_ks, knn_ts, batch, groups)
 
-    def knn_topk(self, feature: torch.Tensor, k: int, normalize: bool = False, mode: Optional[str] = None):
-        return K.knn_topk(self._queries(feature, normalize), self.bank, k, mode)
+    def knn_topk(self, feature: torch.Tensor, k: int, normalize: bool = False, mode: Optional[str] = None,
+                 query_groups: Optional[torch.Tensor] = None, bank_groups: Optional[torch.Tensor] = None):
+        return K.knn_topk(self._queries(feature, normalize), self.bank, k, mode, query_groups, bank_groups)

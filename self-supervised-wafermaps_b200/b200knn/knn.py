@@ -498,7 +498,7 @@ def prepass_stride(n_rows: int, k: int, batch: Optional[int] = None) -> int:
 
 
 def _tc_call(mode, pq, pb, B, n_visit, D, k, idx_offset, stride, tau0, dev, timed=False, sample=False,
-             out=None):
+             out=None, exclude=None):
     lib = _lib.load()
     if out is not None:
         assert out.shape == (B, k) and out.dtype == torch.int64 and out.is_contiguous()
@@ -511,6 +511,13 @@ def _tc_call(mode, pq, pb, B, n_visit, D, k, idx_offset, stride, tau0, dev, time
         _lib.check(lib.b200knn_topk_sample(_lib.MODES[mode], pq.hi.data_ptr(), _ptr(pq.lo), pb.hi.data_ptr(),
                                            _ptr(pb.lo), B, n_visit, D, stride, keys.data_ptr(), ws.data_ptr(),
                                            ws_bytes, _stream()), "topk_sample")
+        return keys
+    if exclude is not None:
+        with _Timed("topk", timed):
+            rc = lib.b200knn_topk_excl(_lib.MODES[mode], pq.hi.data_ptr(), _ptr(pq.lo), pb.hi.data_ptr(), _ptr(pb.lo),
+                                       B, n_visit, D, k, idx_offset, exclude[0].data_ptr(), exclude[1].data_ptr(),
+                                       keys.data_ptr(), ws.data_ptr(), ws_bytes, _stream())
+        _lib.check(rc, "topk_excl")
         return keys
     with _Timed("topk", timed):
         rc = lib.b200knn_topk_ex(_lib.MODES[mode], pq.hi.data_ptr(), _ptr(pq.lo), pb.hi.data_ptr(), _ptr(pb.lo),
@@ -620,27 +627,60 @@ def broadcast_f32(src: torch.Tensor, peer_ptrs, dst_offset: int) -> None:
                                                          len(peer_ptrs), dst_offset, _stream()), "broadcast_f32")
 
 
+def _exclusion(exclude, B: int, N: int, device: torch.device):
+    """``topk_keys``' exclude argument -> (query ids (B,) int32, bank ids (N,) int32, m) with m the
+    largest number of bank rows that share one query row's id.  A 3-tuple is taken as already
+    checked (the internal form: callers that know m pass it and save the host read here)."""
+    if len(exclude) == 3:
+        return exclude
+    qg, bg = exclude
+    for name, t, n in (("query group ids", qg, B), ("bank group ids", bg, N)):
+        if not isinstance(t, torch.Tensor) or t.dtype != torch.int32:
+            raise ValueError(f"{name} must be an int32 tensor of dense ids")
+        if t.numel() != n:
+            raise RuntimeError(f"{name} have {t.numel()} entries for {n} rows")
+        if t.device != device:
+            raise RuntimeError(f"Expected all tensors to be on the same device, but found {device} and {t.device}")
+    qg, bg = qg.contiguous().view(-1), bg.contiguous().view(-1)
+    m = 0
+    if B and N:
+        n_ids = max(int(qg.max()), int(bg.max())) + 1
+        m = int(torch.bincount(bg, minlength=n_ids)[qg.long()].max())
+    return qg, bg, m
+
+
 def topk_keys(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, mode: Optional[str] = None,
               idx_offset: int = 0, tau0: Optional[torch.Tensor] = None, repair: bool = True,
-              out: Optional[torch.Tensor] = None) -> torch.Tensor:
+              out: Optional[torch.Tensor] = None, exclude=None) -> torch.Tensor:
     """(B,k) selection keys (uint64 bit patterns in an int64 tensor), sorted descending under
     the canonical (sim desc, bank index asc) order; bank indices are offset by idx_offset.
 
     tau0 (tensor-core modes): caller-supplied (B,) admission thresholds — then no pre-pass and
     no validation happen here and rows may come back with empty (0) slots (sharded driver).
     repair=False (tensor-core modes): skip the host-synchronising check for rows the sampled
-    threshold starved (empty k-th slot); the caller detects and repairs them (``repair_rows``)."""
+    threshold starved (empty k-th slot); the caller detects and repairs them (``repair_rows``).
+    exclude: optional (query_gids (B,), bank_gids (N,)), dense non-negative int32 ids on the device:
+    bank row n is left out of query row b's search when bank_gids[n] == query_gids[b], in every mode
+    and path (no sampling pre-pass then).  Keys keep the full bank's indices; k must not exceed
+    N minus the largest number of bank rows sharing one query row's id."""
     lib = _lib.load()
     mode = mode or _default_mode
     if mode not in _lib.MODES and mode not in RESCORED_MODES:
         raise ValueError(f"unknown mode {mode!r}")
+    if exclude is not None:
+        _check_feature_bank(feature, feature_bank)
+        if tau0 is not None:
+            raise ValueError("topk_keys: exclude runs without an admission threshold (tau0)")
+        exclude = _exclusion(exclude, feature.shape[0], feature_bank.shape[1], feature.device)
+        if int(k) > feature_bank.shape[1] - exclude[2]:
+            raise RuntimeError("selected index k out of range")
     if int(k) > MAX_K:
         # Tensor.topk takes any k <= N; the streaming lists hold MAX_K keys.  Larger k is served by
         # the exact kernel in passes of <= MAX_K (a completeness path, whatever the mode).
         _check_feature_bank(feature, feature_bank)
-        return _topk_keys_peeled(feature, feature_bank, int(k), idx_offset)
+        return _topk_keys_peeled(feature, feature_bank, int(k), idx_offset, exclude)
     if mode in RESCORED_MODES:
-        return _topk_keys_rescored(feature, feature_bank, k, mode, idx_offset)
+        return _topk_keys_rescored(feature, feature_bank, k, mode, idx_offset, exclude=exclude)
     _check_feature_bank(feature, feature_bank)
     B, D = feature.shape
     mode = effective_mode(mode, D)
@@ -664,14 +704,24 @@ def topk_keys(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, mode: O
             bank = feature_bank if feature_bank.dtype in _DTYPES else feature_bank.float()
             bank, layout, ld = _layout_of(bank, vectors_are_columns=True)
             with _Timed("topk"):
-                rc = lib.b200knn_topk(_lib.MODE_EXACT, q.data_ptr(), None, _DTYPES[q.dtype], q.stride(0),
-                                      bank.data_ptr(), None, _DTYPES[bank.dtype], layout, ld,
-                                      B, N, D, k, idx_offset, keys.data_ptr(), ws.data_ptr(), ws_bytes,
-                                      _stream())
+                if exclude is not None:
+                    rc = lib.b200knn_topk_exact_excl(q.data_ptr(), _DTYPES[q.dtype], q.stride(0), bank.data_ptr(),
+                                                     _DTYPES[bank.dtype], layout, ld, B, N, D, k, idx_offset,
+                                                     exclude[0].data_ptr(), exclude[1].data_ptr(), None,
+                                                     keys.data_ptr(), ws.data_ptr(), ws_bytes, _stream())
+                else:
+                    rc = lib.b200knn_topk(_lib.MODE_EXACT, q.data_ptr(), None, _DTYPES[q.dtype], q.stride(0),
+                                          bank.data_ptr(), None, _DTYPES[bank.dtype], layout, ld,
+                                          B, N, D, k, idx_offset, keys.data_ptr(), ws.data_ptr(), ws_bytes,
+                                          _stream())
             _lib.check(rc, "topk")
             return keys
         pb = bank_cache.get(feature_bank, mode)
         pq = query_cache.get(feature, mode)
+        if exclude is not None:
+            # no sampling pre-pass: a threshold sampled from the whole bank may come from the row's
+            # own group and would starve the row
+            return _tc_call(mode, pq, pb, B, N, D, k, idx_offset, 1, None, dev, timed=True, exclude=exclude)
         if tau0 is not None:  # `out`: write the keys straight into a caller buffer (sharded exchange)
             return _tc_call(mode, pq, pb, B, N, D, k, idx_offset, 1, tau0.contiguous(), dev, timed=True, out=out)
         sk = sample_keys(feature, feature_bank, k, mode)
@@ -684,9 +734,11 @@ def topk_keys(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, mode: O
                                                         idx_offset, 1, None, dev))
 
 
-def _topk_keys_peeled(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, idx_offset: int) -> torch.Tensor:
+def _topk_keys_peeled(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, idx_offset: int,
+                      exclude=None) -> torch.Tensor:
     """Exact keys for k > MAX_K: pass i selects the best min(MAX_K, remaining) keys strictly below
-    the last key of pass i-1 (b200knn_topk_exact_below); ceil(k / MAX_K) scans of the bank."""
+    the last key of pass i-1 (b200knn_topk_exact_below, or b200knn_topk_exact_excl with
+    ``topk_keys``' checked exclusion); ceil(k / MAX_K) scans of the bank."""
     lib = _lib.load()
     B, D = feature.shape
     N = feature_bank.shape[1]
@@ -711,10 +763,17 @@ def _topk_keys_peeled(feature: torch.Tensor, feature_bank: torch.Tensor, k: int,
             if ws_bytes == 0:
                 raise RuntimeError(f"b200knn: unsupported problem (B={B}, N={N}, D={D}, k={kp})")
             ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
-            _lib.check(lib.b200knn_topk_exact_below(q.data_ptr(), _DTYPES[q.dtype], q.stride(0), bank.data_ptr(),
-                                                    _DTYPES[bank.dtype], layout, ld, B, N, D, kp, idx_offset,
-                                                    _ptr(upper), part.data_ptr(), ws.data_ptr(), ws_bytes,
-                                                    _stream()), "topk_exact_below")
+            if exclude is not None:
+                _lib.check(lib.b200knn_topk_exact_excl(q.data_ptr(), _DTYPES[q.dtype], q.stride(0), bank.data_ptr(),
+                                                       _DTYPES[bank.dtype], layout, ld, B, N, D, kp, idx_offset,
+                                                       exclude[0].data_ptr(), exclude[1].data_ptr(), _ptr(upper),
+                                                       part.data_ptr(), ws.data_ptr(), ws_bytes, _stream()),
+                           "topk_exact_excl")
+            else:
+                _lib.check(lib.b200knn_topk_exact_below(q.data_ptr(), _DTYPES[q.dtype], q.stride(0), bank.data_ptr(),
+                                                        _DTYPES[bank.dtype], layout, ld, B, N, D, kp, idx_offset,
+                                                        _ptr(upper), part.data_ptr(), ws.data_ptr(), ws_bytes,
+                                                        _stream()), "topk_exact_below")
             keys[:, done:done + kp] = part
             upper = part[:, -1].contiguous()
             done += kp
@@ -758,9 +817,13 @@ def topk_scatter(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, mode
 
 
 def recompute_rows(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, mode: str, rows: torch.Tensor,
-                   idx_offset: int = 0) -> torch.Tensor:
+                   idx_offset: int = 0, exclude=None) -> torch.Tensor:
     """Keys of the given query rows computed without any admission threshold."""
     sub = feature[rows].contiguous()
+    if exclude is not None:
+        exclude = _exclusion(exclude, feature.shape[0], feature_bank.shape[1], feature.device)
+        return topk_keys(sub, feature_bank, k, "exact" if mode in RESCORED_MODES else mode, idx_offset,
+                         exclude=(exclude[0][rows], exclude[1], exclude[2]))
     if mode == "exact" or mode in RESCORED_MODES:
         return topk_keys(sub, feature_bank, k, "exact", idx_offset)
     B, D = sub.shape
@@ -793,9 +856,10 @@ last_prepass_stats = {"rows": 0, "repaired": 0}
 
 
 def _rescored_level(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, level: str, idx_offset: int,
-                    n_bad: Optional[torch.Tensor] = None):
+                    n_bad: Optional[torch.Tensor] = None, exclude=None):
     """One cascade level, nothing synchronises: (keys (B,k), uncertified flags (B,) int32, count int32[1]).
-    n_bad: optional zeroed int32[1] the count is accumulated into (the caller's status word)."""
+    n_bad: optional zeroed int32[1] the count is accumulated into (the caller's status word).
+    exclude: ``topk_keys``' checked (query ids, bank ids, m) for these rows."""
     lib = _lib.load()
     B, D = feature.shape
     cfg = level_config(level, D)
@@ -803,10 +867,15 @@ def _rescored_level(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, l
     # the streaming lists hold at most MAX_K keys: near that limit the margin shrinks (and with it
     # the chance to certify; uncertified rows still end up exact through the next level)
     k_in = min(N, k + cfg["margin"], max(k, MAX_K))
+    if exclude is not None:
+        # every row keeps at least k_in eligible bank rows, so no candidate slot stays empty (the
+        # re-scoring kernel would read an empty k_in-th slot as uncertified).  The certificate's
+        # max row norm of the whole bank still bounds the reduced bank's.
+        k_in = min(k_in, N - exclude[2])
     dev = feature.device
     # no repair pass on the candidates: a row its sampled threshold starved has an empty k_in-th
     # slot, which the re-scoring kernel reports as uncertified
-    cand = topk_keys(feature, feature_bank, k_in, cfg["cand"], idx_offset, repair=False)
+    cand = topk_keys(feature, feature_bank, k_in, cfg["cand"], idx_offset, repair=False, exclude=exclude)
     pb = bank_cache.get(feature_bank, cfg["cand"])
     rows_a, rows_b = pb.rescore_rows()
     max_norm = pb.max_norm()
@@ -1026,19 +1095,22 @@ def _cascade_levels(feature_bank: torch.Tensor, mode: str, track: bool = True, b
 
 
 def _cascade_fix(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, levels, rows: torch.Tensor,
-                 idx_offset: int) -> torch.Tensor:
-    """Keys of `rows` (uncertified at the previous level) from the remaining levels, then exact."""
+                 idx_offset: int, exclude=None) -> torch.Tensor:
+    """Keys of `rows` (uncertified at the previous level) from the remaining levels, then exact.
+    exclude: ``topk_keys``' checked (query ids, bank ids, m) of `feature`'s rows."""
     sub = feature[rows].contiguous()
+    if exclude is not None:
+        exclude = (exclude[0][rows], exclude[1], exclude[2])
     for level in levels:
-        out, flags, n_bad = _rescored_level(sub, feature_bank, k, level, idx_offset)
+        out, flags, n_bad = _rescored_level(sub, feature_bank, k, level, idx_offset, exclude=exclude)
         last_rescore_stats["levels"].append((level, int(rows.numel()), int(n_bad.item())))
         if int(n_bad.item()) == 0:
             return out
         left = flags.nonzero(as_tuple=False).view(-1)
-        out[left] = _cascade_fix(sub, feature_bank, k, levels[levels.index(level) + 1:], left, idx_offset)
+        out[left] = _cascade_fix(sub, feature_bank, k, levels[levels.index(level) + 1:], left, idx_offset, exclude)
         return out
     last_rescore_stats["levels"].append(("exact", int(rows.numel()), 0))
-    return topk_keys(sub, feature_bank, k, "exact", idx_offset)
+    return topk_keys(sub, feature_bank, k, "exact", idx_offset, exclude=exclude)
 
 
 def _note_first_level(feature_bank: torch.Tensor, mode: str, levels, rows: int, uncertified: int,
@@ -1058,7 +1130,7 @@ def _note_first_level(feature_bank: torch.Tensor, mode: str, levels, rows: int, 
 
 def _topk_keys_rescored(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, mode: str,
                         idx_offset: int = 0, defer: bool = False, track: bool = True, boost: int = 1,
-                        n_bad: Optional[torch.Tensor] = None):
+                        n_bad: Optional[torch.Tensor] = None, exclude=None):
     """Tensor-core candidates -> exact sequential-fma re-scoring -> best k, with a per-row
     certificate; rows a level cannot certify go to the next level and finally to the "exact"
     kernel, so the keys are bitwise those of mode "exact".
@@ -1075,13 +1147,15 @@ def _topk_keys_rescored(feature: torch.Tensor, feature_bank: torch.Tensor, k: in
         out = torch.empty((B, k), dtype=torch.int64, device=dev)
         return (out, None, None, None) if defer else out
     levels = _cascade_levels(feature_bank, mode, track, boost)
-    out, flags, n_bad = _rescored_level(feature, feature_bank, k, levels[0], idx_offset, n_bad)
+    if exclude is not None:
+        exclude = _exclusion(exclude, B, N, dev)
+    out, flags, n_bad = _rescored_level(feature, feature_bank, k, levels[0], idx_offset, n_bad, exclude)
 
     def fix(rows, n_rows_bad):
         _note_first_level(feature_bank, mode, levels, B, n_rows_bad, track)
         if rows is None:
             return None
-        return _cascade_fix(feature, feature_bank, k, levels[1:], rows, idx_offset)
+        return _cascade_fix(feature, feature_bank, k, levels[1:], rows, idx_offset, exclude)
 
     if defer:
         return out, flags, n_bad, fix
@@ -1306,7 +1380,8 @@ def _vote_step(keys, feature_labels, num_classes, knn_t, flag):
     return vote(keys, feature_labels, num_classes, knn_t, check_labels=False, return_flag=True, flag=flag)[0]
 
 
-def _predict_enqueue(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t, mode, track=True, boost=1):
+def _predict_enqueue(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t, mode, track=True, boost=1,
+                     exclude=None):
     """Everything of one tensor-core-mode call, enqueued without a host synchronisation (so it can
     be captured into a CUDA graph): (pred (B,C), status int32[2] = [vote flag, rows to recompute],
     bad_rows (B,) mask/flags, fix).  status[0]: 1 label / 2 neighbour index out of range;
@@ -1316,9 +1391,9 @@ def _predict_enqueue(feature, feature_bank, feature_labels, num_classes, knn_k, 
     status = torch.zeros((2,), dtype=torch.int32, device=feature.device)
     if mode in RESCORED_MODES:
         keys, bad_rows, _, fix = _topk_keys_rescored(feature, feature_bank, knn_k, mode, defer=True,
-                                                     track=track, boost=boost, n_bad=status[1:2])
+                                                     track=track, boost=boost, n_bad=status[1:2], exclude=exclude)
     else:
-        keys = topk_keys(feature, feature_bank, knn_k, mode, repair=False)
+        keys = topk_keys(feature, feature_bank, knn_k, mode, repair=False, exclude=exclude)
         bad_rows = keys[:, -1] == 0
         status[1:2] = bad_rows.sum().to(torch.int32)
         fix = None
@@ -1327,7 +1402,7 @@ def _predict_enqueue(feature, feature_bank, feature_labels, num_classes, knn_k, 
 
 
 def _predict_finish(pred, status, bad_rows, fix, feature, feature_bank, feature_labels, num_classes, knn_k,
-                    knn_t, mode):
+                    knn_t, mode, exclude=None):
     """The host side of a call after its one synchronisation (`status` is a host list here)."""
     n_fix = int(status[1])
     if mode not in RESCORED_MODES:
@@ -1337,7 +1412,7 @@ def _predict_finish(pred, status, bad_rows, fix, feature, feature_bank, feature_
     if n_fix:
         rows = bad_rows.nonzero(as_tuple=False).view(-1)
         fixed = fix(rows, n_fix) if mode in RESCORED_MODES else \
-            recompute_rows(feature, feature_bank, knn_k, mode, rows)
+            recompute_rows(feature, feature_bank, knn_k, mode, rows, exclude=exclude)
         flag2 = torch.zeros((1,), dtype=torch.int32, device=pred.device)
         pred[rows] = _vote_step(fixed, feature_labels, num_classes, knn_t, flag2)
         status[0] = max(int(status[0]), int(flag2.item()))
@@ -1441,9 +1516,10 @@ def _vote_checked(keys, feature_labels, num_classes, knn_t):
     return vote(keys, feature_labels, num_classes, knn_t)
 
 
-def _predict(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t, mode):
+def _predict(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t, mode, exclude=None):
     """knn_predict in `mode`; knn_t a temperature, or a (ks, ts) grid with ks ascending and
-    ks[-1] == knn_k (``_vote_step``)."""
+    ks[-1] == knn_k (``_vote_step``).  exclude: ``topk_keys``' group exclusion (such calls are
+    never captured into a CUDA graph)."""
     _require_cuda("feature_labels", feature_labels)
     if feature_labels.numel() != feature_bank.shape[1]:
         _check_feature_bank(feature, feature_bank)
@@ -1451,7 +1527,8 @@ def _predict(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t, m
             f"feature_labels has {feature_labels.numel()} entries for a bank of {feature_bank.shape[1]}")
     check_vote_classes(num_classes, knn_k, grid=isinstance(knn_t, tuple))
     if mode == "exact" or int(knn_k) > MAX_K:
-        return _vote_checked(topk_keys(feature, feature_bank, knn_k, mode), feature_labels, num_classes, knn_t)
+        return _vote_checked(topk_keys(feature, feature_bank, knn_k, mode, exclude=exclude), feature_labels,
+                             num_classes, knn_t)
     _check_feature_bank(feature, feature_bank)
     knn_k = int(knn_k)
     if knn_k <= 0 or knn_k > feature_bank.shape[1]:
@@ -1462,7 +1539,8 @@ def _predict(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t, m
     # Tensor-core modes: everything is enqueued first and ONE host synchronisation reads the
     # status word (vote flag; rows to recompute: rows a sampled threshold starved, or rows whose
     # exact re-scoring could not be certified).
-    if GRAPHS["enabled"] and feature.shape[0] <= GRAPH_MAX_BATCH and feature_labels.dtype == torch.int64 \
+    if GRAPHS["enabled"] and exclude is None and feature.shape[0] <= GRAPH_MAX_BATCH \
+            and feature_labels.dtype == torch.int64 \
             and feature_labels.is_contiguous() and not torch.cuda.is_current_stream_capturing():
         with torch.cuda.device(feature.device):
             g = _graph_for(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t, mode)
@@ -1483,25 +1561,34 @@ def _predict(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t, m
             return _predict_finish(pred, g.status_host.tolist(), g.bad_rows, g.fix, g.q_static, feature_bank,
                                    feature_labels, num_classes, knn_k, knn_t, mode)
     pred, status, bad_rows, fix = _predict_enqueue(feature, feature_bank, feature_labels, num_classes, knn_k,
-                                                   knn_t, mode)
+                                                   knn_t, mode, exclude=exclude)
     return _predict_finish(pred, status.tolist(), bad_rows, fix, feature, feature_bank, feature_labels,
-                           num_classes, knn_k, knn_t, mode)
+                           num_classes, knn_k, knn_t, mode, exclude)
 
 
 def knn_predict_multi(feature: torch.Tensor, feature_bank: torch.Tensor, feature_labels: torch.Tensor,
-                      num_classes: int, knn_ks=(200,), knn_ts=(0.1,)) -> torch.Tensor:
+                      num_classes: int, knn_ks=(200,), knn_ts=(0.1,), query_groups: Optional[torch.Tensor] = None,
+                      bank_groups: Optional[torch.Tensor] = None) -> torch.Tensor:
     """``knn_predict`` for every (knn_k, knn_t) of a grid from ONE neighbour search at
     k_max = max(knn_ks) and one vote kernel: (len(knn_ks), len(knn_ts), B, num_classes) int64, where
     [i, j] is bitwise ``knn_predict(..., knn_ks[i], knn_ts[j])`` in the default mode.  The top-k list
     is the first k entries of the top-k_max list: the (sim desc, index asc) order and the
-    similarities themselves do not depend on k.  At most 16 values of k and 8 of t, no duplicates."""
+    similarities themselves do not depend on k.  At most 16 values of k and 8 of t, no duplicates.
+
+    query_groups (B,) and bank_groups (N,): optional integer ids (any integer dtype, compared by
+    value, on the bank's device), both or neither.  [i, j, b] is then the same call for query b
+    against the bank without every column c with bank_groups[c] == query_groups[b] (labels
+    likewise): a held-out query never votes with rows of its own group (a lot, a wafer's repeats).
+    The search skips those columns itself, at depth max(knn_ks); max(knn_ks) must not exceed the
+    smallest number of bank rows left to any query."""
     ks, ts, order = check_grid(knn_ks, knn_ts)
     mode = _default_mode
     searches = grid_parts(tuple(ks[i] for i in order), mode)
     for part in searches:  # before the first search
         check_vote_classes(num_classes, part[-1], grid=True)
-    parts = [_predict(feature, feature_bank, feature_labels, num_classes, part[-1], (part, tuple(ts)), mode)
-             for part in searches]
+    exclude = _query_bank_exclusion(feature, feature_bank, query_groups, bank_groups, max(ks))
+    parts = [_predict(feature, feature_bank, feature_labels, num_classes, part[-1], (part, tuple(ts)), mode,
+                      exclude) for part in searches]
     return grid_view(torch.cat(parts, dim=1) if len(parts) > 1 else parts[0], order, len(ts), num_classes)
 
 
@@ -1535,6 +1622,44 @@ _GROUP_DTYPES = (torch.uint8, torch.int8, torch.int16, torch.int32, torch.int64)
 _GROUP_DTYPES_WIDENED = (torch.uint16, torch.uint32)  # to int64, losslessly
 
 
+def _query_bank_exclusion(feature, feature_bank, query_groups, bank_groups, k_max: int):
+    """``topk_keys``' exclusion (query ids, bank ids, m) for query_groups (B,) / bank_groups (N,) of
+    any integer dtype, made dense by one torch.unique over both; None when both are None.  Raises,
+    before any search, on one missing id tensor, a length or device mismatch, a non-integer dtype,
+    and k_max above the smallest number of bank rows outside a query's group."""
+    if query_groups is None and bank_groups is None:
+        return None
+    if query_groups is None or bank_groups is None:
+        raise ValueError("query_groups and bank_groups go together: pass both or neither")
+    if feature.dim() != 2 or feature_bank.dim() != 2:
+        _check_feature_bank(feature, feature_bank)
+    B, N = feature.shape[0], feature_bank.shape[1]
+    ids = []
+    for name, g, n in (("query_groups", query_groups, B), ("bank_groups", bank_groups, N)):
+        if not isinstance(g, torch.Tensor):
+            raise TypeError(f"{name} must be a torch.Tensor, got {type(g).__name__}")
+        if g.numel() != n:
+            raise RuntimeError(f"{name} has {g.numel()} entries for {n} {'queries' if n == B else 'bank rows'}")
+        if g.dtype not in _GROUP_DTYPES + _GROUP_DTYPES_WIDENED + (torch.uint64,):
+            raise ValueError(f"{name} must be an integer tensor, got {g.dtype}")
+        if g.device != feature_bank.device:
+            raise RuntimeError("Expected all tensors to be on the same device, but found "
+                               f"{feature_bank.device} and {g.device}")
+        g = g.reshape(-1)
+        if g.dtype in _GROUP_DTYPES_WIDENED:
+            g = g.to(torch.int64)
+        elif g.dtype == torch.uint64:  # the same bits as int64: equal ids stay equal, distinct ones distinct
+            g = g.view(torch.int64)
+        ids.append(g.to(torch.int64))
+    _, inv = torch.unique(torch.cat(ids), return_inverse=True)
+    inv = inv.to(torch.int32)
+    qg, bg = inv[:B].contiguous(), inv[B:].contiguous()
+    m = int(torch.bincount(bg, minlength=B + N)[qg.long()].max()) if B and N else 0
+    if int(k_max) > N - m:  # the bank without the query's group has N - m rows for some query
+        raise RuntimeError("selected index k out of range")
+    return qg, bg, m
+
+
 def _group_plan(groups: torch.Tensor, n: int, device: torch.device):
     """The buckets of a leave-one-group-out search: (dense int32 group ids (n,), largest group size,
     rows (n,) int64 in bucket order, [(p, lo, hi)]) where positions [lo, hi) of `rows` hold, in
@@ -1564,26 +1689,44 @@ def _group_plan(groups: torch.Tensor, n: int, device: torch.device):
     return inv.to(torch.int32), stats[0], rows, buckets
 
 
+def logo_excludes(k: int, p: int, n: int) -> bool:
+    """Whether the leave-one-group-out rows of bucket p (group sizes in (p/2, p]) search for a list
+    of k neighbours by skipping their group inside the search (at depth k) instead of searching
+    deeper and dropping the group's keys afterwards: when that deeper search, min(n, k + p), would
+    not fit the streaming lists (MAX_K)."""
+    return min(n, int(k) + int(p)) > MAX_K
+
+
 def _group_searches(feature_bank: torch.Tensor, plan, ks_ascending: tuple, mode: str, batch: int,
                     flag: torch.Tensor):
     """Yields (part, lo, hi, keys) for every search of a leave-one-group-out pass over the bank's own
     rows: keys (hi - lo, part[-1]) are the lists of rows plan[2][lo:hi] without their groups.  Each
     search runs one ``topk_keys`` at depth min(N, part[-1] + p) (every mode, cascade and repair) and
     one ``drop_group``; it takes max(1, min(batch, batch * (part[-1] + 1) // depth)) rows, so its key
-    buffer is no larger than that of a leave-one-out search of `batch` rows."""
-    gid, _, rows, buckets = plan
+    buffer is no larger than that of a leave-one-out search of `batch` rows.  A part deeper than
+    MAX_K (``logo_excludes``) instead runs one group-excluding ``topk_keys`` at depth part[-1] on
+    `batch` rows: the mode's own path, or in a raw tensor-core mode the exact kernel, whose result
+    the deeper search gave such rows."""
+    gid, g_max, rows, buckets = plan
     n = feature_bank.shape[1]
     bank_rows = feature_bank.t()
     whole = len(buckets) == 1  # rows is arange(n): the queries are views
     for p, b_lo, b_hi in buckets:
         for part in logo_parts(ks_ascending, p, n, mode):
-            depth = min(n, part[-1] + p)
+            excl = logo_excludes(part[-1], p, n)
+            depth = part[-1] if excl else min(n, part[-1] + p)
             step = max(1, min(batch, batch * (part[-1] + 1) // depth))
             for lo in range(b_lo, b_hi, step):
                 hi = min(b_hi, lo + step)
                 q = bank_rows[lo:hi] if whole else bank_rows.index_select(0, rows[lo:hi])
                 if q.stride(1) != 1:
                     q = q.contiguous()
+                if excl:
+                    # a row's own id is its group's, so the row itself is skipped with it
+                    qg = gid[lo:hi] if whole else gid.index_select(0, rows[lo:hi])
+                    yield part, lo, hi, topk_keys(q, feature_bank, depth, "exact" if mode in TC_MODES else mode,
+                                                  exclude=(qg, gid, g_max))
+                    continue
                 yield part, lo, hi, drop_group(topk_keys(q, feature_bank, depth, mode), rows[lo:hi], gid, part[-1],
                                                flag)
 
@@ -1700,11 +1843,15 @@ def grid_view(pred: torch.Tensor, order, n_t: int, num_classes: int) -> torch.Te
     return g[torch.tensor(inv, device=pred.device)] if inv != list(range(len(order))) else g.contiguous()
 
 
-def knn_topk(feature: torch.Tensor, feature_bank: torch.Tensor, k: int,
-             mode: Optional[str] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+def knn_topk(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, mode: Optional[str] = None,
+             query_groups: Optional[torch.Tensor] = None,
+             bank_groups: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
     """``torch.mm(feature, feature_bank).topk(k, dim=-1)`` without materialising the
-    similarity matrix: (sims fp32 (B,k) sorted desc, idx int64 (B,k)), ties by lowest index."""
-    return decode_keys(topk_keys(feature, feature_bank, k, mode))
+    similarity matrix: (sims fp32 (B,k) sorted desc, idx int64 (B,k)), ties by lowest index.
+    query_groups / bank_groups: as ``knn_predict_multi``; query b's list then skips every bank
+    column of its group, and the indices are still those of the full bank."""
+    exclude = _query_bank_exclusion(feature, feature_bank, query_groups, bank_groups, k)
+    return decode_keys(topk_keys(feature, feature_bank, k, mode, exclude=exclude))
 
 
 def plan_info(B: int, N: int, D: int, k: int, mode: Optional[str] = None) -> dict:

@@ -109,7 +109,8 @@ static int topk_impl(int mode, const void* q_hi, const void* q_lo, int q_dtype, 
                      float* dump, int32_t* diag, int flags, int64_t bank_row_stride = 1,
                      const float* tau0 = nullptr, bool sample = false,
                      const void* const* host_peer_out = nullptr, int n_peers = 0, int my_rank = 0,
-                     int64_t rows_per_owner = 0, const uint64_t* upper = nullptr) {
+                     int64_t rows_per_owner = 0, const uint64_t* upper = nullptr,
+                     const int32_t* q_gid = nullptr, const int32_t* bank_gid = nullptr) {
   if (B < 0 || N <= 0 || dim <= 0) return fail(B200KNN_E_ARG, "topk: bad shape");
   if (k <= 0 || k > N) return fail(B200KNN_E_ARG, "topk: selected index k out of range");
   if (N + idx_offset >= 0xFFFFFFFFll || idx_offset < 0)
@@ -160,6 +161,8 @@ static int topk_impl(int mode, const void* q_hi, const void* q_lo, int q_dtype, 
     p.lists = lists;
     p.out = partial;
     p.upper = upper;
+    p.q_gid = q_gid;
+    p.bank_gid = bank_gid;
     e = b200knn::launch_exact(p, plan.grid, plan.cap, st);
     if (e != cudaSuccess) return fail_cuda("topk(exact)", e);
   } else if (is_tc_mode(mode)) {
@@ -195,6 +198,8 @@ static int topk_impl(int mode, const void* q_hi, const void* q_lo, int q_dtype, 
     p.rows_per_owner = rows_per_owner;
     for (int g = 0; g < n_peers; ++g)
       p.peer_out[g] = static_cast<uint64_t*>(const_cast<void*>(host_peer_out[g]));
+    p.q_gid = q_gid;
+    p.bank_gid = bank_gid;
     const char* why = "";
     e = b200knn::launch_tc(p, plan.grid, plan.cap, st, dump, diag, flags, &why);
     if (e == cudaErrorNotSupported) return fail(B200KNN_E_UNSUPPORTED, "topk(tc): %s", why);
@@ -228,6 +233,28 @@ int b200knn_topk_exact_below(const void* q, int q_dtype, int64_t q_ld, const voi
   return topk_impl(B200KNN_MODE_EXACT, q, nullptr, q_dtype, q_ld, bank, nullptr, bank_dtype, bank_layout,
                    bank_ld, B, N, dim, k, idx_offset, out_keys, workspace, workspace_bytes, stream, nullptr,
                    nullptr, 0, 1, nullptr, false, nullptr, 0, 0, 0, upper_keys);
+}
+
+int b200knn_topk_excl(int mode, const void* q_hi, const void* q_lo, const void* bank_hi, const void* bank_lo,
+                      int64_t B, int64_t N, int dim, int k, int64_t idx_offset, const int32_t* q_groups,
+                      const int32_t* bank_groups, uint64_t* out_keys, void* workspace, size_t workspace_bytes,
+                      void* stream) {
+  if (!is_tc_mode(mode)) return fail(B200KNN_E_ARG, "topk_excl: tensor-core modes only");
+  if (!q_groups || !bank_groups) return fail(B200KNN_E_ARG, "topk_excl: null group ids");
+  return topk_impl(mode, q_hi, q_lo, 0, 0, bank_hi, bank_lo, 0, 0, 0, B, N, dim, k, idx_offset, out_keys,
+                   workspace, workspace_bytes, stream, nullptr, nullptr, 0, 1, nullptr, false, nullptr, 0, 0, 0,
+                   nullptr, q_groups, bank_groups);
+}
+
+int b200knn_topk_exact_excl(const void* q, int q_dtype, int64_t q_ld, const void* bank, int bank_dtype,
+                            int bank_layout, int64_t bank_ld, int64_t B, int64_t N, int dim, int k,
+                            int64_t idx_offset, const int32_t* q_groups, const int32_t* bank_groups,
+                            const uint64_t* upper_keys, uint64_t* out_keys, void* workspace,
+                            size_t workspace_bytes, void* stream) {
+  if (!q_groups || !bank_groups) return fail(B200KNN_E_ARG, "topk_exact_excl: null group ids");
+  return topk_impl(B200KNN_MODE_EXACT, q, nullptr, q_dtype, q_ld, bank, nullptr, bank_dtype, bank_layout,
+                   bank_ld, B, N, dim, k, idx_offset, out_keys, workspace, workspace_bytes, stream, nullptr,
+                   nullptr, 0, 1, nullptr, false, nullptr, 0, 0, 0, upper_keys, q_groups, bank_groups);
 }
 
 int b200knn_topk_ex(int mode, const void* q_hi, const void* q_lo, const void* bank_hi,

@@ -28,7 +28,9 @@ __device__ __forceinline__ float load_f32(const void* p, int dtype, int64_t i) {
   return __bfloat162float(static_cast<const __nv_bfloat16*>(p)[i]);
 }
 
-template <int ITEMS>
+// EXCL: bank columns of the query row's group (ExactParams::q_gid / bank_gid) are never admitted;
+// the filter sits next to the peeling bound, so every pass of a peeled search applies it.
+template <int ITEMS, bool EXCL>
 __global__ void __launch_bounds__(256) exact_topk_kernel(ExactParams p) {
   extern __shared__ float smem[];
   float* As = smem;              // [TD][TM]  queries, d-major
@@ -57,6 +59,8 @@ __global__ void __launch_bounds__(256) exact_topk_kernel(ExactParams p) {
     // k > 992 is served in passes ("peeling", b200knn/knn.py): pass i admits only keys strictly
     // below the last key of pass i-1.  Filtering the stream keeps the threshold logic valid.
     const uint64_t upper = (p.upper != nullptr && tid < TM && m0 + tid < p.B) ? p.upper[m0 + tid] : ~0ull;
+    int32_t my_gid = 0;
+    if constexpr (EXCL) my_gid = (tid < TM && m0 + tid < p.B) ? p.q_gid[m0 + tid] : 0;
 
     for (int64_t n0 = n_begin; n0 < n_end; n0 += TN) {
       float acc[8][8];
@@ -138,7 +142,9 @@ __global__ void __launch_bounds__(256) exact_topk_kernel(ExactParams p) {
             if (s[j] > st.tau) {
               const int64_t gn = n0 + c0 + j;
               const uint64_t key = make_key(s[j], uint32_t(gn + p.idx_offset));
-              if (gn < n_end && key < upper) my_list[c++] = key;
+              bool ok = gn < n_end && key < upper;
+              if constexpr (EXCL) ok = ok && __ldg(p.bank_gid + gn) != my_gid;
+              if (ok) my_list[c++] = key;
             }
           }
           st.cnt = c;
@@ -163,27 +169,33 @@ __global__ void __launch_bounds__(256) exact_topk_kernel(ExactParams p) {
   }
 }
 
-template <int ITEMS>
+template <int ITEMS, bool EXCL>
 cudaError_t launch_exact_t(const ExactParams& p, int grid, cudaStream_t stream) {
   const size_t smem = sizeof(float) * (TD * TM + TD * TN + TM * S_LD);
-  cudaError_t e = cudaFuncSetAttribute(exact_topk_kernel<ITEMS>,
+  cudaError_t e = cudaFuncSetAttribute(exact_topk_kernel<ITEMS, EXCL>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
   if (e != cudaSuccess) return e;
-  exact_topk_kernel<ITEMS><<<grid, 256, smem, stream>>>(p);
+  exact_topk_kernel<ITEMS, EXCL><<<grid, 256, smem, stream>>>(p);
   return cudaGetLastError();
+}
+
+template <bool EXCL>
+cudaError_t launch_exact_cap(const ExactParams& p, int grid, int cap, cudaStream_t stream) {
+  switch (cap) {
+    case 64: return launch_exact_t<2, EXCL>(p, grid, stream);
+    case 128: return launch_exact_t<4, EXCL>(p, grid, stream);
+    case 256: return launch_exact_t<8, EXCL>(p, grid, stream);
+    case 512: return launch_exact_t<16, EXCL>(p, grid, stream);
+    case 1024: return launch_exact_t<32, EXCL>(p, grid, stream);
+    default: return cudaErrorInvalidValue;
+  }
 }
 
 }  // namespace
 
 cudaError_t launch_exact(const ExactParams& p, int grid, int cap, cudaStream_t stream) {
-  switch (cap) {
-    case 64: return launch_exact_t<2>(p, grid, stream);
-    case 128: return launch_exact_t<4>(p, grid, stream);
-    case 256: return launch_exact_t<8>(p, grid, stream);
-    case 512: return launch_exact_t<16>(p, grid, stream);
-    case 1024: return launch_exact_t<32>(p, grid, stream);
-    default: return cudaErrorInvalidValue;
-  }
+  return p.bank_gid != nullptr ? launch_exact_cap<true>(p, grid, cap, stream)
+                               : launch_exact_cap<false>(p, grid, cap, stream);
 }
 
 }  // namespace b200knn

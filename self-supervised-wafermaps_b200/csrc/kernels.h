@@ -21,6 +21,10 @@ struct ExactParams {
   uint64_t* lists;
   uint64_t* out;  // (splits, B, k)
   const uint64_t* upper = nullptr;  // optional (B,): only keys strictly below upper[row] are admitted
+  // optional group exclusion (both or neither): q_gid (B,), bank_gid (N,) indexed before idx_offset;
+  // bank row n is never admitted to query row b's list when bank_gid[n] == q_gid[b]
+  const int32_t* q_gid = nullptr;
+  const int32_t* bank_gid = nullptr;
 };
 
 cudaError_t launch_exact(const ExactParams& p, int grid, int cap, cudaStream_t stream);
@@ -147,6 +151,9 @@ struct TcParams {
   int n_peers = 0, my_rank = 0;
   int64_t rows_per_owner = 0;
   bool sample = false;  // sampling pre-pass: k == 16 best SIMILARITIES per row (keys carry index 0)
+  // optional group exclusion, as ExactParams (no tau0, sample, debug output or peers with it)
+  const int32_t* q_gid = nullptr;
+  const int32_t* bank_gid = nullptr;
 };
 // returns cudaErrorNotSupported if (D, k) is outside what the kernel handles
 // `dump` (optional, (B,N) fp32) receives the raw similarity tiles (unit tests only);

@@ -110,6 +110,10 @@ struct TcKernelArgs {
   int32_t* diag;
   int flags;    // experiment switches of the debug entry point (0 in production):
                 // 1 no selection, 2 no TMEM loads, 4 no MMA issue, 8 no bank TMA loads
+  // EXCL: group ids of the query rows, (B,), and of the bank rows of this launch, (N,) indexed
+  // before idx_offset; a column whose id equals its query row's id is never admitted to its list
+  const int32_t* q_gid;
+  const int32_t* bank_gid;
 };
 
 // PAIR: two CTAs of a cluster (one TPC) run one tcgen05.mma.cta_group::2 per k-step:
@@ -127,6 +131,11 @@ struct TcKernelArgs {
 // insert — no candidate lists, no prunes, no indices.  Its 16-th value is <= the 16-th best
 // sampled similarity, which is all the main pass's admission threshold needs.  The general
 // list machinery spent 2/3 of the pre-pass warming up its lists.
+//
+// EXCL: group exclusion (product builds only, never with DEBUG or SAMPLE).  Only the hit path of
+// the epilogue changes: an excluded column can turn a miss into a false hit, never the reverse, so
+// the no-hit test stays as it is and the qualifying columns of a hit are filtered by their group
+// ids (gathered from the L2-resident id array) before they are appended.
 // One unit of work of a worker: query tile `qt` against bank rows [n_begin, n_end).
 struct WorkItem {
   int64_t qt, sp, n_begin, n_end;
@@ -165,7 +174,7 @@ __device__ __forceinline__ void for_each_item(const TcKernelArgs& a, int64_t wor
   }
 }
 
-template <int MODE, int BLOCK_N, int ITEMS, bool DEBUG, bool PAIR, bool SAMPLE>
+template <int MODE, int BLOCK_N, int ITEMS, bool DEBUG, bool PAIR, bool SAMPLE, bool EXCL>
 __global__ void __launch_bounds__(kThreads, 1)
     tc_topk_kernel(const __grid_constant__ CUtensorMap map_q_hi,
                    const __grid_constant__ CUtensorMap map_q_lo,
@@ -176,6 +185,7 @@ __global__ void __launch_bounds__(kThreads, 1)
   constexpr int kBArrays = (MODE == B200KNN_MODE_F16X2) ? 2 : 1;  // bank arrays streamed per k-block (lo, hi)
   constexpr bool kHalf = (MODE != B200KNN_MODE_TF32X3);   // 2-byte elements (kind::f16)
   static_assert(!PAIR || kBf16, "CTA pairs are implemented for the resident-query modes");
+  static_assert(!EXCL || (!DEBUG && !SAMPLE), "group exclusion is a product-build variant");
   constexpr int CAP = ITEMS * 32;
   constexpr int kCtas = PAIR ? 2 : 1;
   constexpr int kBRows = BLOCK_N / kCtas;  // bank rows of one tile this CTA loads
@@ -410,6 +420,8 @@ __global__ void __launch_bounds__(kThreads, 1)
           a.lists + ((size_t(blockIdx.x) * size_t(a.slots) + size_t(it.slot)) * kTileM + size_t(quarter) * 32) * CAP;
       uint64_t* my_list = warp_lists + size_t(lane) * CAP;
       const bool mine = owner && grow < a.B;  // this lane selects for a real query row
+      int32_t my_gid = 0;
+      if constexpr (EXCL) my_gid = mine ? a.q_gid[grow] : 0;
       RowState st;
       if (it.first || SAMPLE) {
         st.cnt = 0;
@@ -497,7 +509,20 @@ __global__ void __launch_bounds__(kThreads, 1)
               }
             }
             const uint32_t gidx0 = uint32_t(n0 + c0 + a.idx_offset);
-            if ((m & (m - 1u)) == 0u) {
+            bool one = (m & (m - 1u)) == 0u;
+            if constexpr (EXCL) {
+              // drop the qualifying columns of the row's own group; the row maximum may be one of
+              // them, so a single survivor of a filtered mask takes the general path below
+              const int32_t* g = a.bank_gid + (n0 + c0);
+              unsigned keep = m;
+              for (unsigned r = m; r != 0u; r &= r - 1u) {
+                const int j = __ffs(r) - 1;
+                if (__ldg(g + j) == my_gid) keep &= ~(1u << j);
+              }
+              one = one && keep == m;
+              m = keep;
+            }
+            if (one) {
               // the common case, exactly one candidate: it is the row maximum
               my_list[st.cnt] = make_key(mx, gidx0 + uint32_t(__ffs(m) - 1));
               st.cnt += 1;
@@ -617,7 +642,7 @@ bool make_map(CUtensorMap* m, const void* base, bool bf16, uint64_t rows, uint64
   return r == CUDA_SUCCESS;
 }
 
-template <int MODE, int BLOCK_N, int ITEMS, bool DEBUG, bool PAIR, bool SAMPLE = false>
+template <int MODE, int BLOCK_N, int ITEMS, bool DEBUG, bool PAIR, bool SAMPLE = false, bool EXCL = false>
 cudaError_t launch_t(const TcParams& p, int grid, cudaStream_t stream, float* dump, int32_t* diag,
                      int flags, const char** why) {
   constexpr bool kBf16 = (MODE == B200KNN_MODE_BF16 || MODE == B200KNN_MODE_F16X2 ||
@@ -654,6 +679,8 @@ cudaError_t launch_t(const TcParams& p, int grid, cudaStream_t stream, float* du
   a.dump = dump;
   a.diag = diag;
   a.flags = flags;
+  a.q_gid = p.q_gid;
+  a.bank_gid = p.bank_gid;
   const int b_block = kBRows * kRowBytes;
   const int stage_bytes = kBf16 ? b_block : 2 * (kABlockBytes + b_block);
   const int q_bytes = kBf16 ? a.n_kblocks * kABlockBytes : 0;
@@ -679,7 +706,7 @@ cudaError_t launch_t(const TcParams& p, int grid, cudaStream_t stream, float* du
   }
   if (kBf16) mq_lo = mq_hi;
   if (kBf16 && !kTwoB) mb_lo = mb_hi;
-  auto kern = tc_topk_kernel<MODE, BLOCK_N, ITEMS, DEBUG, PAIR, SAMPLE>;
+  auto kern = tc_topk_kernel<MODE, BLOCK_N, ITEMS, DEBUG, PAIR, SAMPLE, EXCL>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
   if (e != cudaSuccess) return e;
   // `grid` counts workers: CTAs, or CTA pairs (clusters of 2 on one TPC) when PAIR
@@ -707,6 +734,20 @@ cudaError_t launch_cap(const TcParams& p, int grid, int cap, cudaStream_t stream
       return cudaErrorNotSupported;
     }
     return launch_t<MODE, BLOCK_N, 2, false, PAIR, true>(p, grid, stream, nullptr, diag, 0, why);
+  }
+  if (p.bank_gid != nullptr) {
+    if (DEBUG || p.tau0 != nullptr || p.n_peers > 0) {
+      *why = "group exclusion runs without debug output, thresholds or a peer exchange";
+      return cudaErrorNotSupported;
+    }
+    switch (cap) {
+      case 64: return launch_t<MODE, BLOCK_N, 2, false, PAIR, false, true>(p, grid, stream, nullptr, diag, 0, why);
+      case 128: return launch_t<MODE, BLOCK_N, 4, false, PAIR, false, true>(p, grid, stream, nullptr, diag, 0, why);
+      case 256: return launch_t<MODE, BLOCK_N, 8, false, PAIR, false, true>(p, grid, stream, nullptr, diag, 0, why);
+      case 512: return launch_t<MODE, BLOCK_N, 16, false, PAIR, false, true>(p, grid, stream, nullptr, diag, 0, why);
+      case 1024: return launch_t<MODE, BLOCK_N, 32, false, PAIR, false, true>(p, grid, stream, nullptr, diag, 0, why);
+      default: *why = "unsupported k"; return cudaErrorNotSupported;
+    }
   }
   switch (cap) {
     case 64: return launch_t<MODE, BLOCK_N, 2, DEBUG, PAIR>(p, grid, stream, dump, diag, flags, why);
