@@ -33,8 +33,12 @@
 extern "C" {
 #endif
 
-#define B200KNN_VERSION 142 /* 0.1.4.2: + b200knn_topk_sample_scatter, b200knn_broadcast_f32; 0.1.4.1: + b200knn_plan_info_ex; 0.1.4: + b200knn_topk_exact_below (k > 992), b200knn_route_scatter, b200knn_rescore_scatter,
-                              b200knn_compact_rows, b200knn_scatter_rows (sync-free sharded fp32 mode); 0.1.3: + B200KNN_MODE_F16; 0.1.2: + b200knn_route_keys, b200knn_certify (sharded fp32 mode); 0.1.1: b200knn_rescore workspace */
+#define B200KNN_VERSION 150 /* 0.1.5: the b200knn_topk_* variants become options of b200knn_topk_opt; plan_info folds into
+                              b200knn_plan_info_ex; 0.1.4.2: + the peer-memory threshold exchange, b200knn_broadcast_f32;
+                              0.1.4.1: + b200knn_plan_info_ex; 0.1.4: + peeling (k > 992), b200knn_route_scatter,
+                              b200knn_rescore_scatter, b200knn_compact_rows, b200knn_scatter_rows (sync-free sharded fp32 mode);
+                              0.1.3: + B200KNN_MODE_F16; 0.1.2: + b200knn_route_keys, b200knn_certify (sharded fp32 mode);
+                              0.1.1: b200knn_rescore workspace */
 
 /* error codes */
 #define B200KNN_OK 0
@@ -112,95 +116,74 @@ int b200knn_topk(int mode,
                  void* workspace, size_t workspace_bytes, void* stream);
 
 /*
- * b200knn_topk for the tensor-core modes with two extras used by the sampling
- * pre-pass (no counterpart in the reference):
- *   bank_row_stride: visit prepared bank rows 0, s, 2s, ... (n_visit of them);
- *                    returned indices are the VISIT index (+ idx_offset)
- *   tau0           : optional (B,) initial admission thresholds: only rows with
- *                    sim > tau0[b] are considered, so fewer than k may be found
- *                    (the remaining key slots are 0); NULL = no threshold.
- * A threshold taken from the r-th best similarity of a strided sample is below
- * the true k-th similarity except with negligible probability; the host shim
- * detects the exception (empty k-th slot) and recomputes that row without tau0.
- */
-/*
- * Tensor.topk accepts any k <= N; the streaming lists hold at most 992 keys.  Larger k is served in
- * passes of <= 992 ("peeling"): b200knn_topk in MODE_EXACT restricted to keys strictly below
- * upper_keys[b] (the last key of row b from the previous pass; nullptr = no bound).  Arguments as
- * b200knn_topk.
- */
-int b200knn_topk_exact_below(const void* q, int q_dtype, int64_t q_ld, const void* bank, int bank_dtype,
-                             int bank_layout, int64_t bank_ld, int64_t B, int64_t N, int dim, int k,
-                             int64_t idx_offset, const uint64_t* upper_keys, uint64_t* out_keys,
-                             void* workspace, size_t workspace_bytes, void* stream);
-
-/*
- * Group-excluding searches (no counterpart in the reference; k-fold cross-validation and held-out
- * queries whose group also has rows in the bank): b200knn_topk, except that bank row n is never
- * admitted to query row b's list when bank_groups[n] == q_groups[b].  Order, key format and indices
- * (idx_offset included) are unchanged; a row with fewer than k eligible bank rows gets empty (0)
- * trailing slots.
- *   q_groups   : (B,) int32 group id of every query row
- *   bank_groups: (N,) int32 group id of every bank row, indexed before idx_offset
- * Both must be non-null (B200KNN_E_ARG otherwise).
- * b200knn_topk_excl      : the tensor-core modes (operands as b200knn_topk_ex; no sampling
- *                          threshold, no row stride).
- * b200knn_topk_exact_excl: MODE_EXACT, arguments as b200knn_topk_exact_below (upper_keys may be
- *                          NULL), so peeled passes for k > 992 exclude the groups too.
- */
-int b200knn_topk_excl(int mode, const void* q_hi, const void* q_lo, const void* bank_hi,
-                      const void* bank_lo, int64_t B, int64_t N, int dim, int k, int64_t idx_offset,
-                      const int32_t* q_groups, const int32_t* bank_groups, uint64_t* out_keys,
-                      void* workspace, size_t workspace_bytes, void* stream);
-int b200knn_topk_exact_excl(const void* q, int q_dtype, int64_t q_ld, const void* bank, int bank_dtype,
-                            int bank_layout, int64_t bank_ld, int64_t B, int64_t N, int dim, int k,
-                            int64_t idx_offset, const int32_t* q_groups, const int32_t* bank_groups,
-                            const uint64_t* upper_keys, uint64_t* out_keys, void* workspace,
-                            size_t workspace_bytes, void* stream);
-
-int b200knn_topk_ex(int mode, const void* q_hi, const void* q_lo,
-                    const void* bank_hi, const void* bank_lo, int64_t B,
-                    int64_t n_visit, int dim, int k, int64_t idx_offset,
-                    int64_t bank_row_stride, const float* tau0,
-                    uint64_t* out_keys, void* workspace, size_t workspace_bytes,
-                    void* stream);
-
-/*
- * Sampling pre-pass (no counterpart in the reference): for every query, the
- * B200KNN_SAMPLE_R = 16 best 32-column CHUNK MAXIMA of its similarities with prepared bank
- * rows 0, s, 2s, ... (n_visit of them), as (B,16) keys sorted descending whose index field
- * is 0 (values only — each row's running top-16 lives in registers, no candidate lists).
- * Every returned value is a sampled similarity and the 16-th is <= the 16-th best sampled
- * similarity, so it is a valid seed for b200knn_topk_ex's tau0.  Workspace: b200knn_topk_workspace_bytes(B, n_visit, dim, 16, mode).
+ * b200knn_topk with options (no counterpart in the reference).  opts == NULL, or an all-zero
+ * struct, is exactly b200knn_topk.  The options:
+ *   bank_row_stride : 0 or 1 visit every bank row; s > 1 visits prepared rows 0, s, 2s, ...
+ *                     (N of them, the "n_visit" of a sample); indices are the VISIT index
+ *                     (+ idx_offset).  Tensor-core modes.
+ *   tau0            : (B,) initial admission thresholds: only rows with sim > tau0[b] are
+ *                     considered, so fewer than k may be found (the remaining key slots are 0).
+ *                     A threshold taken from the r-th best similarity of a strided sample is
+ *                     below the true k-th similarity except with negligible probability; the
+ *                     host shim detects the exception (empty k-th slot) and recomputes that row
+ *                     without tau0.  Tensor-core modes.
+ *   upper_keys      : (B,) peeling bound: only keys strictly below upper_keys[b] (the last key of
+ *                     row b from the previous pass).  Tensor.topk accepts any k <= N and the
+ *                     streaming lists hold at most 992 keys, so larger k is served in passes of
+ *                     <= 992 ("peeling").  MODE_EXACT.
+ *   q_groups,       : (B,) and (N,) int32 group ids (bank ids indexed before idx_offset), both or
+ *   bank_groups       neither: bank row n is never admitted to query row b's list when
+ *                     bank_groups[n] == q_groups[b] (k-fold cross-validation, held-out queries whose
+ *                     group also has rows in the bank).  Order, key format and indices are
+ *                     unchanged; a row with fewer than k eligible bank rows gets empty (0) trailing
+ *                     slots.  Every mode: alone in the tensor-core modes, with or without
+ *                     upper_keys in MODE_EXACT.
+ *   sample          : non-zero = the sampling pre-pass: for every query, the B200KNN_SAMPLE_R = 16
+ *                     best 32-column CHUNK MAXIMA of its similarities with the visited rows, as
+ *                     (B,16) keys sorted descending whose index field is 0 (values only: each
+ *                     row's running top-16 lives in registers, no candidate lists).  Every value
+ *                     is a sampled similarity and the 16-th is <= the 16-th best sampled
+ *                     similarity, so it is a valid seed for tau0.  Needs k == 16 and N >= 16.
+ *                     Tensor-core modes.
+ *   host_peer_out,  : fused exchange for the bank-row-sharded mode: result rows are not returned
+ *   n_peers,          locally (out_keys must be NULL) but stored, as each query tile finishes,
+ *   my_rank,          straight into the exchange buffer of the GPU that owns that query (peer
+ *   rows_per_owner    memory over NVLink, so the all-to-all overlaps the remaining tiles' math).
+ *                     host_peer_out is a HOST array of n_peers (1..8) DEVICE pointers, each mapped
+ *                     in this process; peer g's buffer is (n_peers, rows_per_owner, k) uint64.
+ *                     Query row b's owner is b / rows_per_owner (rows_per_owner * n_peers >= B),
+ *                     and its keys go to peer_out[owner][my_rank][b - owner*rows_per_owner][0..k).
+ *                     After a cross-GPU barrier every GPU holds, for its own query rows, all
+ *                     shards' sorted lists in b200knn_merge's input layout.  Only problems planned
+ *                     without bank splits (b200knn_plan_info_ex splits == 1) are supported; others
+ *                     return B200KNN_E_UNSUPPORTED.  Tensor-core modes, with tau0 at stride 1 or
+ *                     with sample at any stride.
+ * Combinations (anything else returns B200KNN_E_ARG, checked before any work is planned):
+ *   MODE_EXACT        : upper_keys, groups, or both;
+ *   tensor-core modes : bank_row_stride with tau0; sample with bank_row_stride, optionally with
+ *                       the peer exchange; tau0 with the peer exchange at stride 1; groups alone.
+ * Workspace: b200knn_topk_workspace_bytes(B, N, dim, k, mode) bytes, N the rows visited.
  */
 #define B200KNN_SAMPLE_R 16
-int b200knn_topk_sample(int mode, const void* q_hi, const void* q_lo,
-                        const void* bank_hi, const void* bank_lo, int64_t B,
-                        int64_t n_visit, int dim, int64_t bank_row_stride,
-                        uint64_t* out_keys, void* workspace, size_t workspace_bytes,
-                        void* stream);
+typedef struct b200knn_topk_options {
+  int64_t bank_row_stride;          /* 0 or 1: every row; s > 1: rows 0, s, 2s, ... (tensor-core modes) */
+  const float* tau0;                /* (B,) admission thresholds (tensor-core modes) */
+  const uint64_t* upper_keys;       /* (B,) peeling bound: only keys strictly below (MODE_EXACT) */
+  const int32_t* q_groups;          /* (B,) and (N,) group ids: both or neither */
+  const int32_t* bank_groups;
+  int sample;                       /* values-only B200KNN_SAMPLE_R best (tensor-core modes) */
+  const void* const* host_peer_out; /* fused exchange: n_peers device pointers (HOST array) */
+  int n_peers, my_rank;
+  int64_t rows_per_owner;
+} b200knn_topk_options;
 
-/*
- * Fused similarity + top-k + exchange for the bank-row-sharded mode (no counterpart in the
- * reference): b200knn_topk_ex whose result rows are not returned locally but stored, as each
- * query tile finishes, straight into the exchange buffer of the GPU that owns that query —
- * peer memory over NVLink, so the all-to-all of candidate keys overlaps the remaining tiles'
- * math instead of following the kernel.
- *   host_peer_out : HOST array of n_peers DEVICE pointers; peer g's buffer is
- *                   (n_peers, rows_per_owner, k) uint64 and must be mapped in this process
- *                   (symmetric / IPC memory with peer access enabled);
- *   query row b   : owner = b / rows_per_owner; keys go to
- *                   peer_out[owner][my_rank][b - owner*rows_per_owner][0..k)
- * After a cross-GPU barrier every GPU holds, for its own query rows, all shards' sorted
- * lists in b200knn_merge's input layout.  Only problems planned without bank splits
- * (b200knn_plan_info splits == 1) are supported; others return B200KNN_E_UNSUPPORTED.
- */
-int b200knn_topk_scatter(int mode, const void* q_hi, const void* q_lo,
-                         const void* bank_hi, const void* bank_lo, int64_t B, int64_t N,
-                         int dim, int k, int64_t idx_offset, const float* tau0,
-                         const void* const* host_peer_out, int n_peers, int my_rank,
-                         int64_t rows_per_owner, void* workspace, size_t workspace_bytes,
-                         void* stream);
+int b200knn_topk_opt(int mode,
+                     const void* q_hi, const void* q_lo, int q_dtype, int64_t q_ld,
+                     const void* bank_hi, const void* bank_lo, int bank_dtype,
+                     int bank_layout, int64_t bank_ld,
+                     int64_t B, int64_t N, int dim, int k, int64_t idx_offset,
+                     uint64_t* out_keys, void* workspace, size_t workspace_bytes,
+                     const b200knn_topk_options* opts, void* stream);
 
 /*
  * Merge G sorted candidate lists per query into one (replaces nothing in the
@@ -267,7 +250,7 @@ int b200knn_vote(const uint64_t* keys, const int64_t* labels, int64_t B, int k,
 /*
  * b200knn_vote writing into a wider row-major buffer: pred has row stride pred_ld >= C, and
  * when status_col >= C a per-row status word is stored in that column: bit 0 = the row's
- * k-th key slot is empty (a b200knn_topk_ex threshold starved it), bit 1 = a label outside
+ * k-th key slot is empty (a tau0 threshold of b200knn_topk_opt starved it), bit 1 = a label outside
  * [0,C), bit 2 = a neighbour index outside the labels.  The sharded driver all-gathers this
  * (B_owned, C+1) buffer as it is.
  */
@@ -291,7 +274,7 @@ int b200knn_vote_multi(const uint64_t* keys, const int64_t* labels, int64_t B, i
                        int32_t* err_flag, void* stream);
 
 /* out[b] = similarity of keys[b, j] (-inf for an empty slot): the threshold a (B,r) sample
- * hands to b200knn_topk_ex (j = r-1). */
+ * hands to b200knn_topk_opt as tau0 (j = r-1). */
 int b200knn_key_sim_column(const uint64_t* keys, int64_t B, int k, int j, float* out,
                            void* stream);
 
@@ -311,7 +294,7 @@ int b200knn_key_sim_column(const uint64_t* keys, int64_t B, int k, int j, float*
  *              caller must recompute row b in MODE_EXACT; *n_uncertified counts such rows
  *              (caller zeroes it).  max_abs > 0 additionally refuses rows with ||q_b|| or M
  *              >= max_abs (operand range of a half-precision candidate pass).  A row whose
- *              k_in-th candidate slot is empty although k_in < N (a b200knn_topk_ex
+ *              k_in-th candidate slot is empty although k_in < N (a b200knn_topk_opt tau0
  *              threshold starved it) is uncertified as well.
  *   workspace: optional, b200knn_rescore_workspace_bytes(B, k_in) bytes of device memory.
  *              With it (and fp32 queries, rows_b NULL) the rows are gathered by a persistent
@@ -366,15 +349,9 @@ int b200knn_certify(const void* q, int q_dtype, int64_t q_ld, int dim, const uin
  *   runs on a fixed-capacity sub-batch without a host read.
  * b200knn_scatter_rows: dst[rows[i]*dst_ld + c] = src[i*src_ld + c], c < width, i < min(n, *count).
  */
-/* The sharded threshold exchange over peer memory: b200knn_topk_sample whose 16 values of query row b go into
- * the exchange buffer of the GPU that owns b (host_peer_out[b / rows_per_owner] + ((my_rank * rows_per_owner +
- * b % rows_per_owner) * 16); refused (B200KNN_E_UNSUPPORTED) when the sample is planned with bank splits), and
- * b200knn_broadcast_f32: dst[g][dst_offset + i] = src[i] for every peer g (the owner publishes its thresholds). */
-int b200knn_topk_sample_scatter(int mode, const void* q_hi, const void* q_lo, const void* bank_hi,
-                                const void* bank_lo, int64_t B, int64_t n_visit, int dim,
-                                int64_t bank_row_stride, const void* const* host_peer_out, int n_peers,
-                                int my_rank, int64_t rows_per_owner, void* workspace, size_t workspace_bytes,
-                                void* stream);
+/* The sharded threshold exchange over peer memory: a sample (b200knn_topk_opt) with the peer exchange stores the
+ * 16 values of query row b into the buffer of the GPU that owns b, and b200knn_broadcast_f32:
+ * dst[g][dst_offset + i] = src[i] for every peer g (the owner publishes its thresholds). */
 int b200knn_broadcast_f32(const float* src, int64_t n, const void* const* host_peer_dst, int n_peers,
                           int64_t dst_offset, void* stream);
 int b200knn_route_scatter(const uint64_t* keys, int64_t n, int k, int64_t rows_per_shard, int n_shards,
@@ -413,11 +390,9 @@ int b200knn_confusion(const int64_t* pred, const int64_t* target, int64_t n, int
 /* Device capability probe for the host shim: 1 if the current device is sm_100. */
 int b200knn_device_ok(void);
 
-/* How b200knn_topk decomposes a call (for the bench and the docs):
- * out6 = {n_qtiles, splits, split_rows, n_items, grid, list_capacity}. HOST pointer. */
-int b200knn_plan_info(int mode, int64_t B, int64_t N, int dim, int k, int64_t* host_out6);
-/* ... plus the chunk-major order of the tensor-core kernel: out9 = out6 + {chunks, chunk_rows, slots}
- * (a worker keeps `slots` query tiles open and scans the bank in `chunks` L2-sized pieces). */
+/* How b200knn_topk decomposes a call (for the bench and the docs), HOST pointer:
+ * out9 = {n_qtiles, splits, split_rows, n_items, grid, list_capacity, chunks, chunk_rows, slots}
+ * (a tensor-core worker keeps `slots` query tiles open and scans the bank in `chunks` L2-sized pieces). */
 int b200knn_plan_info_ex(int mode, int64_t B, int64_t N, int dim, int k, int64_t* host_out9);
 /* Tuning knob: bytes of bank one chunk of the chunk-major order may occupy (default 40 MiB, or
  * $B200KNN_L2_CHUNK_MB; 0 = never chunk).  Process-wide; affects planning only, never results. */

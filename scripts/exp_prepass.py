@@ -36,17 +36,17 @@ def timed(label, fn, reps=3):
 for s, r in ((62, 16),):
     n_visit = (N + s - 1) // s
     keys = timed(f"(a) strided sample  s={s} n_visit={n_visit} k={r}",
-                 lambda: K._tc_call("bf16", pq, pb, Q, n_visit, D, r, 0, s, None, dev))
+                 lambda: K._search("bf16", pq, pb, Q, n_visit, D, r, stride=s))
     timed(f"(b) contiguous rows          n_visit={n_visit} k={r}",
-          lambda: K._tc_call("bf16", pq, pb, Q, n_visit, D, r, 0, 1, None, dev))
+          lambda: K._search("bf16", pq, pb, Q, n_visit, D, r))
     timed(f"(a') strided sample, register top-16 variant",
-          lambda: K._tc_call("bf16", pq, pb, Q, n_visit, D, r, 0, s, None, dev, sample=True))
+          lambda: K._search("bf16", pq, pb, Q, n_visit, D, r, stride=s, sample=True))
     tau = K.kth_sim(keys)
     timed(f"(c) contiguous rows, tau0 = own {r}-th best (few appends)",
-          lambda: K._tc_call("bf16", pq, pb, Q, n_visit, D, r, 0, 1, tau, dev))
+          lambda: K._search("bf16", pq, pb, Q, n_visit, D, r, tau0=tau))
     timed(f"(c') strided rows, tau0 = own {r}-th best (few appends)",
-          lambda: K._tc_call("bf16", pq, pb, Q, n_visit, D, r, 0, s, tau, dev))
-keys = K._tc_call("bf16", pq, pb, Q, (N + 61) // 62, D, 16, 0, 62, None, dev)
+          lambda: K._search("bf16", pq, pb, Q, n_visit, D, r, stride=s, tau0=tau))
+keys = K._search("bf16", pq, pb, Q, (N + 61) // 62, D, 16, stride=62)
 tau = K.kth_sim(keys)
-timed("(d) main pass k=200 with prepass tau", lambda: K._tc_call("bf16", pq, pb, Q, N, D, 200, 0, 1, tau, dev))
-timed("(d') main pass k=200 without tau", lambda: K._tc_call("bf16", pq, pb, Q, N, D, 200, 0, 1, None, dev), reps=1)
+timed("(d) main pass k=200 with prepass tau", lambda: K._search("bf16", pq, pb, Q, N, D, 200, tau0=tau))
+timed("(d') main pass k=200 without tau", lambda: K._search("bf16", pq, pb, Q, N, D, 200), reps=1)

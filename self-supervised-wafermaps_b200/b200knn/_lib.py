@@ -21,6 +21,15 @@ MODE_EXACT, MODE_BF16, MODE_TF32X3, MODE_F32ROWS, MODE_BF16X3, MODE_F16X2, MODE_
 SAMPLE_R = 16  # B200KNN_SAMPLE_R
 MODES = {"exact": MODE_EXACT, "bf16": MODE_BF16, "tf32x3": MODE_TF32X3, "bf16x3": MODE_BF16X3, "f16x2": MODE_F16X2, "f16": MODE_F16}
 
+
+class TopkOptions(ctypes.Structure):
+    """b200knn_topk_options: all zero is a plain b200knn_topk."""
+    _fields_ = [("bank_row_stride", c_int64), ("tau0", c_void_p), ("upper_keys", c_void_p),
+                ("q_groups", c_void_p), ("bank_groups", c_void_p), ("sample", c_int),
+                ("host_peer_out", ctypes.POINTER(c_void_p)), ("n_peers", c_int), ("my_rank", c_int),
+                ("rows_per_owner", c_int64)]
+
+
 # every symbol include/b200knn.h declares: (restype, argtypes)
 SIGNATURES = {
     "b200knn_version": (c_int, []),
@@ -36,42 +45,13 @@ SIGNATURES = {
         [c_int, c_void_p, c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int, c_int, c_int64,
          c_int64, c_int64, c_int, c_int, c_int64, c_void_p, c_void_p, c_size_t, c_void_p],
     ),
-    "b200knn_topk_exact_below": (
+    "b200knn_topk_opt": (
         c_int,
-        [c_void_p, c_int, c_int64, c_void_p, c_int, c_int, c_int64, c_int64, c_int64, c_int, c_int, c_int64,
-         c_void_p, c_void_p, c_void_p, c_size_t, c_void_p],
-    ),
-    "b200knn_topk_excl": (
-        c_int,
-        [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_int64, c_void_p, c_void_p,
-         c_void_p, c_void_p, c_size_t, c_void_p],
-    ),
-    "b200knn_topk_exact_excl": (
-        c_int,
-        [c_void_p, c_int, c_int64, c_void_p, c_int, c_int, c_int64, c_int64, c_int64, c_int, c_int, c_int64,
-         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p],
-    ),
-    "b200knn_topk_ex": (
-        c_int,
-        [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_int64, c_int64,
-         c_void_p, c_void_p, c_void_p, c_size_t, c_void_p],
-    ),
-    "b200knn_topk_sample": (
-        c_int,
-        [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int64,
-         c_void_p, c_void_p, c_size_t, c_void_p],
-    ),
-    "b200knn_topk_sample_scatter": (
-        c_int,
-        [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int64,
-         ctypes.POINTER(c_void_p), c_int, c_int, c_int64, c_void_p, c_size_t, c_void_p],
+        [c_int, c_void_p, c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int, c_int, c_int64,
+         c_int64, c_int64, c_int, c_int, c_int64, c_void_p, c_void_p, c_size_t, ctypes.POINTER(TopkOptions),
+         c_void_p],
     ),
     "b200knn_broadcast_f32": (c_int, [c_void_p, c_int64, ctypes.POINTER(c_void_p), c_int, c_int64, c_void_p]),
-    "b200knn_topk_scatter": (
-        c_int,
-        [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_int64, c_void_p,
-         ctypes.POINTER(c_void_p), c_int, c_int, c_int64, c_void_p, c_size_t, c_void_p],
-    ),
     "b200knn_merge": (c_int, [c_void_p, c_int, c_int64, c_int, c_int, c_void_p, c_void_p]),
     "b200knn_decode_keys": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
     "b200knn_drop_self": (c_int, [c_void_p, c_int64, c_int, c_int64, c_void_p, c_void_p]),
@@ -120,7 +100,6 @@ SIGNATURES = {
         [c_void_p, c_int, c_int64, c_int, c_void_p, c_int, c_void_p, c_int, c_int64, c_int, ctypes.c_float,
          ctypes.c_float, ctypes.c_float, c_void_p, c_void_p, c_void_p, c_void_p],
     ),
-    "b200knn_plan_info": (c_int, [c_int, c_int64, c_int64, c_int, c_int, ctypes.POINTER(c_int64)]),
     "b200knn_set_l2_chunk_bytes": (c_int, [c_int64]),
     "b200knn_plan_info_ex": (c_int, [c_int, c_int64, c_int64, c_int, c_int, ctypes.POINTER(c_int64)]),
     "b200knn_debug_topk_dump": (
@@ -135,12 +114,10 @@ _lib = None
 # kernels each C entry point launches (bench.py's gpu_launches; a b200knn_topk* call whose plan
 # splits the bank launches one more, the split merge — bench.py adds those from plan_info)
 KERNELS_PER_CALL = {
-    "b200knn_prepare_rows": 1, "b200knn_topk": 1, "b200knn_topk_ex": 1, "b200knn_topk_sample": 1, "b200knn_topk_scatter": 1,
+    "b200knn_prepare_rows": 1, "b200knn_topk": 1, "b200knn_topk_opt": 1,
     "b200knn_merge": 1, "b200knn_decode_keys": 1, "b200knn_drop_self": 1, "b200knn_drop_group": 1, "b200knn_vote": 1, "b200knn_vote_ex": 1, "b200knn_vote_multi": 1,
     "b200knn_key_sim_column": 1, "b200knn_normalize_rows": 1, "b200knn_confusion": 1, "b200knn_row_sqnorms": 1, "b200knn_rescore": 2, "b200knn_route_keys": 1, "b200knn_certify": 1,
-    "b200knn_row_norm_max": 1, "b200knn_debug_topk_dump": 1, "b200knn_topk_exact_below": 1,
-    "b200knn_topk_excl": 1, "b200knn_topk_exact_excl": 1,
-    "b200knn_topk_sample_scatter": 1, "b200knn_broadcast_f32": 1,
+    "b200knn_row_norm_max": 1, "b200knn_debug_topk_dump": 1, "b200knn_broadcast_f32": 1,
     "b200knn_route_scatter": 1, "b200knn_rescore_scatter": 2, "b200knn_compact_rows": 1, "b200knn_scatter_rows": 1,
 }
 launch_counter = {"kernels": 0}

@@ -497,34 +497,52 @@ def prepass_stride(n_rows: int, k: int, batch: Optional[int] = None) -> int:
     return s if n_rows // s >= PREPASS["min_sample_rows"] else 0
 
 
-def _tc_call(mode, pq, pb, B, n_visit, D, k, idx_offset, stride, tau0, dev, timed=False, sample=False,
-             out=None, exclude=None):
+def _search(mode, q, bank, B, n_visit, D, k, idx_offset=0, *, stride=1, tau0=None, upper=None, groups=None,
+            sample=False, peers=None, out=None, timed=False) -> Optional[torch.Tensor]:
+    """One b200knn_topk_opt call: the (B, k) keys of queries q among n_visit bank rows.
+    q, bank: the caller tensors of ``_exact_operands`` in mode "exact", PreparedRows otherwise.
+    Options (include/b200knn.h): row stride, (B,) thresholds tau0, (B,) peeling bound `upper`,
+    groups = (query ids, bank ids, ...), the values-only sample, and peers = (device pointers,
+    rank, rows_per_owner), which stores the keys into the peers' buffers and returns None."""
     lib = _lib.load()
-    if out is not None:
+    if mode == "exact":
+        bank, layout, ld = bank
+        args = (q.data_ptr(), None, _DTYPES[q.dtype], q.stride(0), bank.data_ptr(), None, _DTYPES[bank.dtype],
+                layout, ld)
+        dev = q.device
+    else:
+        args = (q.hi.data_ptr(), _ptr(q.lo), 0, 0, bank.hi.data_ptr(), _ptr(bank.lo), 0, 0, 0)
+        dev = q.hi.device
+    opts = _lib.TopkOptions(bank_row_stride=stride, tau0=_ptr(tau0), upper_keys=_ptr(upper), sample=sample)
+    if groups is not None:
+        opts.q_groups, opts.bank_groups = groups[0].data_ptr(), groups[1].data_ptr()
+    keys = None
+    if peers is not None:
+        ptrs, opts.my_rank, opts.rows_per_owner = peers
+        opts.host_peer_out, opts.n_peers = _ptr_array(ptrs), len(ptrs)
+    elif out is not None:
         assert out.shape == (B, k) and out.dtype == torch.int64 and out.is_contiguous()
-    keys = out if out is not None else torch.empty((B, k), dtype=torch.int64, device=dev)
+        keys = out
+    else:
+        keys = torch.empty((B, k), dtype=torch.int64, device=dev)
     ws_bytes = lib.b200knn_topk_workspace_bytes(B, n_visit, D, k, _lib.MODES[mode])
     if ws_bytes == 0:
         raise RuntimeError(f"b200knn: unsupported problem (B={B}, N={n_visit}, D={D}, k={k})")
     ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
-    if sample:  # values-only sampling variant (k == 16, indices are not produced)
-        _lib.check(lib.b200knn_topk_sample(_lib.MODES[mode], pq.hi.data_ptr(), _ptr(pq.lo), pb.hi.data_ptr(),
-                                           _ptr(pb.lo), B, n_visit, D, stride, keys.data_ptr(), ws.data_ptr(),
-                                           ws_bytes, _stream()), "topk_sample")
-        return keys
-    if exclude is not None:
-        with _Timed("topk", timed):
-            rc = lib.b200knn_topk_excl(_lib.MODES[mode], pq.hi.data_ptr(), _ptr(pq.lo), pb.hi.data_ptr(), _ptr(pb.lo),
-                                       B, n_visit, D, k, idx_offset, exclude[0].data_ptr(), exclude[1].data_ptr(),
-                                       keys.data_ptr(), ws.data_ptr(), ws_bytes, _stream())
-        _lib.check(rc, "topk_excl")
-        return keys
     with _Timed("topk", timed):
-        rc = lib.b200knn_topk_ex(_lib.MODES[mode], pq.hi.data_ptr(), _ptr(pq.lo), pb.hi.data_ptr(), _ptr(pb.lo),
-                                 B, n_visit, D, k, idx_offset, stride, _ptr(tau0), keys.data_ptr(),
-                                 ws.data_ptr(), ws_bytes, _stream())
+        rc = lib.b200knn_topk_opt(_lib.MODES[mode], *args, B, n_visit, D, k, idx_offset, _ptr(keys), ws.data_ptr(),
+                                  ws_bytes, opts, _stream())
     _lib.check(rc, "topk")
     return keys
+
+
+def _exact_operands(feature: torch.Tensor, feature_bank: torch.Tensor):
+    """(q, (bank, layout, ld)): the caller tensors as MODE_EXACT reads them, copied only when needed."""
+    q = feature if feature.dtype in _DTYPES else feature.float()
+    if q.stride(1) != 1:
+        q = q.contiguous()
+    bank = feature_bank if feature_bank.dtype in _DTYPES else feature_bank.float()
+    return q, _layout_of(bank, vectors_are_columns=True)
 
 
 def kth_sim(keys: torch.Tensor) -> torch.Tensor:
@@ -577,8 +595,8 @@ def sample_keys(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, mode:
     with torch.cuda.device(feature.device):
         pb = bank_cache.get(feature_bank, mode)
         pq = query_cache.get(feature, mode)
-        return _tc_call(mode, pq, pb, B, n_visit, D, r, 0, s, None, feature.device,
-                        sample=(r == _lib.SAMPLE_R and PREPASS["register_sample"]))
+        return _search(mode, pq, pb, B, n_visit, D, r, stride=s,
+                       sample=(r == _lib.SAMPLE_R and PREPASS["register_sample"]))
 
 
 def sample_scatter_supported(B: int, n_rows: int, D: int, k: int, mode: str, n_rows_for_decision: int) -> bool:
@@ -599,22 +617,16 @@ def sample_scatter(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, mo
                    peer_ptrs, rank: int, rows_per_owner: int) -> None:
     """sample_keys whose (B, 16) sample of query row b is stored straight into the exchange buffer of
     the GPU that owns b (the sharded threshold exchange over NVLink peer memory)."""
-    lib = _lib.load()
     N = feature_bank.shape[1]
     B, D = feature.shape
     s = prepass_stride(n_rows_for_decision, k, B)
     mode = effective_mode(mode, D)
     n_visit = (N + s - 1) // s
-    dev = feature.device
-    with torch.cuda.device(dev):
+    with torch.cuda.device(feature.device):
         pb = bank_cache.get(feature_bank, mode)
         pq = query_cache.get(feature, mode)
-        ws_bytes = lib.b200knn_topk_workspace_bytes(B, n_visit, D, PREPASS["r"], _lib.MODES[mode])
-        ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
-        _lib.check(lib.b200knn_topk_sample_scatter(_lib.MODES[mode], pq.hi.data_ptr(), _ptr(pq.lo), pb.hi.data_ptr(),
-                                                   _ptr(pb.lo), B, n_visit, D, s, _ptr_array(peer_ptrs), len(peer_ptrs),
-                                                   rank, rows_per_owner, ws.data_ptr(), ws_bytes, _stream()),
-                   "topk_sample_scatter")
+        _search(mode, pq, pb, B, n_visit, D, PREPASS["r"], stride=s, sample=True,
+                peers=(peer_ptrs, rank, rows_per_owner))
 
 
 def broadcast_f32(src: torch.Tensor, peer_ptrs, dst_offset: int) -> None:
@@ -663,7 +675,7 @@ def topk_keys(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, mode: O
     bank row n is left out of query row b's search when bank_gids[n] == query_gids[b], in every mode
     and path (no sampling pre-pass then).  Keys keep the full bank's indices; k must not exceed
     N minus the largest number of bank rows sharing one query row's id."""
-    lib = _lib.load()
+    _lib.load()
     mode = mode or _default_mode
     if mode not in _lib.MODES and mode not in RESCORED_MODES:
         raise ValueError(f"unknown mode {mode!r}")
@@ -678,7 +690,7 @@ def topk_keys(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, mode: O
         # Tensor.topk takes any k <= N; the streaming lists hold MAX_K keys.  Larger k is served by
         # the exact kernel in passes of <= MAX_K (a completeness path, whatever the mode).
         _check_feature_bank(feature, feature_bank)
-        return _topk_keys_peeled(feature, feature_bank, int(k), idx_offset, exclude)
+        return _topk_keys_exact(feature, feature_bank, int(k), idx_offset, exclude)
     if mode in RESCORED_MODES:
         return _topk_keys_rescored(feature, feature_bank, k, mode, idx_offset, exclude=exclude)
     _check_feature_bank(feature, feature_bank)
@@ -693,53 +705,31 @@ def topk_keys(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, mode: O
         if B == 0:
             return torch.empty((B, k), dtype=torch.int64, device=dev)
         if mode == "exact":
-            keys = torch.empty((B, k), dtype=torch.int64, device=dev)
-            ws_bytes = lib.b200knn_topk_workspace_bytes(B, N, D, k, _lib.MODE_EXACT)
-            if ws_bytes == 0:
-                raise RuntimeError(f"b200knn: unsupported problem (B={B}, N={N}, D={D}, k={k})")
-            ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
-            q = feature if feature.dtype in _DTYPES else feature.float()
-            if q.stride(1) != 1:
-                q = q.contiguous()
-            bank = feature_bank if feature_bank.dtype in _DTYPES else feature_bank.float()
-            bank, layout, ld = _layout_of(bank, vectors_are_columns=True)
-            with _Timed("topk"):
-                if exclude is not None:
-                    rc = lib.b200knn_topk_exact_excl(q.data_ptr(), _DTYPES[q.dtype], q.stride(0), bank.data_ptr(),
-                                                     _DTYPES[bank.dtype], layout, ld, B, N, D, k, idx_offset,
-                                                     exclude[0].data_ptr(), exclude[1].data_ptr(), None,
-                                                     keys.data_ptr(), ws.data_ptr(), ws_bytes, _stream())
-                else:
-                    rc = lib.b200knn_topk(_lib.MODE_EXACT, q.data_ptr(), None, _DTYPES[q.dtype], q.stride(0),
-                                          bank.data_ptr(), None, _DTYPES[bank.dtype], layout, ld,
-                                          B, N, D, k, idx_offset, keys.data_ptr(), ws.data_ptr(), ws_bytes,
-                                          _stream())
-            _lib.check(rc, "topk")
-            return keys
+            return _topk_keys_exact(feature, feature_bank, k, idx_offset, exclude)
         pb = bank_cache.get(feature_bank, mode)
         pq = query_cache.get(feature, mode)
         if exclude is not None:
             # no sampling pre-pass: a threshold sampled from the whole bank may come from the row's
             # own group and would starve the row
-            return _tc_call(mode, pq, pb, B, N, D, k, idx_offset, 1, None, dev, timed=True, exclude=exclude)
+            return _search(mode, pq, pb, B, N, D, k, idx_offset, groups=exclude, timed=True)
         if tau0 is not None:  # `out`: write the keys straight into a caller buffer (sharded exchange)
-            return _tc_call(mode, pq, pb, B, N, D, k, idx_offset, 1, tau0.contiguous(), dev, timed=True, out=out)
+            return _search(mode, pq, pb, B, N, D, k, idx_offset, tau0=tau0.contiguous(), out=out, timed=True)
         sk = sample_keys(feature, feature_bank, k, mode)
         if sk is None:
-            return _tc_call(mode, pq, pb, B, N, D, k, idx_offset, 1, None, dev, timed=True)
-        keys = _tc_call(mode, pq, pb, B, N, D, k, idx_offset, 1, kth_sim(sk), dev, timed=True)
+            return _search(mode, pq, pb, B, N, D, k, idx_offset, timed=True)
+        keys = _search(mode, pq, pb, B, N, D, k, idx_offset, tau0=kth_sim(sk), timed=True)
         if not repair:
             return keys
-        return _repair_rows(keys, lambda rows: _tc_call(mode, _rows_of(pq, rows), pb, rows.numel(), N, D, k,
-                                                        idx_offset, 1, None, dev))
+        return _repair_rows(keys, lambda rows: _search(mode, _rows_of(pq, rows), pb, rows.numel(), N, D, k,
+                                                       idx_offset))
 
 
-def _topk_keys_peeled(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, idx_offset: int,
-                      exclude=None) -> torch.Tensor:
-    """Exact keys for k > MAX_K: pass i selects the best min(MAX_K, remaining) keys strictly below
-    the last key of pass i-1 (b200knn_topk_exact_below, or b200knn_topk_exact_excl with
-    ``topk_keys``' checked exclusion); ceil(k / MAX_K) scans of the bank."""
-    lib = _lib.load()
+def _topk_keys_exact(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, idx_offset: int,
+                     exclude=None) -> torch.Tensor:
+    """MODE_EXACT keys, with ``topk_keys``' checked exclusion.  Tensor.topk takes any k <= N and the
+    streaming lists hold MAX_K keys: pass i selects the best min(MAX_K, remaining) keys strictly
+    below the last key of pass i-1, so k <= MAX_K is one pass without a bound and larger k takes
+    ceil(k / MAX_K) scans of the bank."""
     B, D = feature.shape
     N = feature_bank.shape[1]
     if k > N:
@@ -748,32 +738,15 @@ def _topk_keys_peeled(feature: torch.Tensor, feature_bank: torch.Tensor, k: int,
     keys = torch.empty((B, k), dtype=torch.int64, device=dev)
     if B == 0:
         return keys
-    q = feature if feature.dtype in _DTYPES else feature.float()
-    if q.stride(1) != 1:
-        q = q.contiguous()
-    bank = feature_bank if feature_bank.dtype in _DTYPES else feature_bank.float()
-    bank, layout, ld = _layout_of(bank, vectors_are_columns=True)
+    q, bank = _exact_operands(feature, feature_bank)
     upper = None
     done = 0
     with torch.cuda.device(dev):
         while done < k:
             kp = min(MAX_K, k - done)
-            part = torch.empty((B, kp), dtype=torch.int64, device=dev)
-            ws_bytes = lib.b200knn_topk_workspace_bytes(B, N, D, kp, _lib.MODE_EXACT)
-            if ws_bytes == 0:
-                raise RuntimeError(f"b200knn: unsupported problem (B={B}, N={N}, D={D}, k={kp})")
-            ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
-            if exclude is not None:
-                _lib.check(lib.b200knn_topk_exact_excl(q.data_ptr(), _DTYPES[q.dtype], q.stride(0), bank.data_ptr(),
-                                                       _DTYPES[bank.dtype], layout, ld, B, N, D, kp, idx_offset,
-                                                       exclude[0].data_ptr(), exclude[1].data_ptr(), _ptr(upper),
-                                                       part.data_ptr(), ws.data_ptr(), ws_bytes, _stream()),
-                           "topk_exact_excl")
-            else:
-                _lib.check(lib.b200knn_topk_exact_below(q.data_ptr(), _DTYPES[q.dtype], q.stride(0), bank.data_ptr(),
-                                                        _DTYPES[bank.dtype], layout, ld, B, N, D, kp, idx_offset,
-                                                        _ptr(upper), part.data_ptr(), ws.data_ptr(), ws_bytes,
-                                                        _stream()), "topk_exact_below")
+            if kp == k:  # one pass: straight into keys, recorded as the "topk" event
+                return _search("exact", q, bank, B, N, D, k, idx_offset, groups=exclude, out=keys, timed=True)
+            part = _search("exact", q, bank, B, N, D, kp, idx_offset, upper=upper, groups=exclude)
             keys[:, done:done + kp] = part
             upper = part[:, -1].contiguous()
             done += kp
@@ -782,37 +755,25 @@ def _topk_keys_peeled(feature: torch.Tensor, feature_bank: torch.Tensor, k: int,
 
 def topk_scatter(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, mode: str, idx_offset: int,
                  tau0: Optional[torch.Tensor], peer_ptrs, rank: int, rows_per_owner: int) -> bool:
-    """Fused top-k + exchange (b200knn_topk_scatter): this shard's keys of query row b are stored
+    """Fused top-k + exchange (b200knn_topk_opt with peers): this shard's keys of query row b are stored
     into peer_ptrs[b // rows_per_owner] (device pointers of every rank's (G, rows_per_owner, k)
     exchange buffer, mapped in this process).  Returns False when the problem is planned with
     bank splits (caller falls back to the NCCL exchange)."""
-    lib = _lib.load()
     if mode not in TC_MODES:
         return False
     _check_feature_bank(feature, feature_bank)
     B, D = feature.shape
     mode = effective_mode(mode, D)
     N = feature_bank.shape[1]
-    G = len(peer_ptrs)
-    if B == 0 or k > N or G > 8:
+    if B == 0 or k <= 0 or k > N or len(peer_ptrs) > 8:
         return False
     if plan_info(B, N, D, k, mode)["splits"] != 1:
         return False
-    dev = feature.device
-    with torch.cuda.device(dev):
+    with torch.cuda.device(feature.device):
         pb = bank_cache.get(feature_bank, mode)
         pq = query_cache.get(feature, mode)
-        ws_bytes = lib.b200knn_topk_workspace_bytes(B, N, D, k, _lib.MODES[mode])
-        if ws_bytes == 0:
-            return False
-        ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
-        ptrs = (ctypes.c_void_p * G)(*[int(p) for p in peer_ptrs])
-        with _Timed("topk"):
-            rc = lib.b200knn_topk_scatter(_lib.MODES[mode], pq.hi.data_ptr(), _ptr(pq.lo), pb.hi.data_ptr(),
-                                          _ptr(pb.lo), B, N, D, k, idx_offset,
-                                          _ptr(None if tau0 is None else tau0.contiguous()), ptrs, G, rank,
-                                          rows_per_owner, ws.data_ptr(), ws_bytes, _stream())
-        _lib.check(rc, "topk_scatter")
+        _search(mode, pq, pb, B, N, D, k, idx_offset, tau0=None if tau0 is None else tau0.contiguous(),
+                peers=(peer_ptrs, rank, rows_per_owner), timed=True)
     return True
 
 
@@ -831,7 +792,7 @@ def recompute_rows(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, mo
     with torch.cuda.device(feature.device):
         pb = bank_cache.get(feature_bank, mode)
         pq = prepare_rows(sub, mode, vectors_are_columns=False)
-        return _tc_call(mode, pq, pb, B, feature_bank.shape[1], D, k, idx_offset, 1, None, feature.device)
+        return _search(mode, pq, pb, B, feature_bank.shape[1], D, k, idx_offset)
 
 
 def _rows_of(pq: "PreparedRows", rows: torch.Tensor) -> "PreparedRows":

@@ -65,6 +65,61 @@ bool plan_for(int mode, int64_t B, int64_t N, int dim, int k, b200knn::TopkPlan*
   return true;
 }
 
+// The operands and shape of one search, named as b200knn_topk_opt names them.
+struct TopkOperands {
+  const void* q_hi;
+  const void* q_lo;
+  int q_dtype;
+  int64_t q_ld;
+  const void* bank_hi;
+  const void* bank_lo;
+  int bank_dtype, bank_layout;
+  int64_t bank_ld;
+  uint64_t* out_keys;
+  void* workspace;
+  size_t workspace_bytes;
+  void* stream;
+};
+struct TopkShape {
+  int64_t B, N;
+  int dim, k;
+  int64_t idx_offset;
+};
+
+// Which options of b200knn_topk_opt go together (the table in include/b200knn.h).  Runs before
+// any planning or launch, so every refusal here needs no GPU.
+int check_options(int mode, const TopkShape& s, const uint64_t* out_keys, const b200knn_topk_options& o) {
+  const bool groups = o.q_groups != nullptr || o.bank_groups != nullptr;
+  const bool peers = o.n_peers != 0 || o.host_peer_out != nullptr;
+  const bool strided = o.bank_row_stride > 1;
+  if (groups && (o.q_groups == nullptr || o.bank_groups == nullptr))
+    return fail(B200KNN_E_ARG, "topk: null group ids (q_groups and bank_groups go together)");
+  if (o.bank_row_stride < 0) return fail(B200KNN_E_ARG, "topk: bank_row_stride must be >= 0");
+  if (o.sample && (s.k != B200KNN_SAMPLE_R || s.N < B200KNN_SAMPLE_R))
+    return fail(B200KNN_E_ARG, "topk: sample needs k == 16 and at least 16 rows to visit");
+  if (peers) {
+    if (o.host_peer_out == nullptr || o.n_peers < 1 || o.n_peers > 8 || o.my_rank < 0 || o.my_rank >= o.n_peers)
+      return fail(B200KNN_E_ARG, "topk: 1..8 peers and a rank among them");
+    if (o.rows_per_owner <= 0 || o.rows_per_owner * o.n_peers < s.B)
+      return fail(B200KNN_E_ARG, "topk: rows_per_owner * n_peers must cover B");
+    for (int g = 0; g < o.n_peers; ++g)
+      if (o.host_peer_out[g] == nullptr) return fail(B200KNN_E_ARG, "topk: null peer buffer");
+    if (out_keys != nullptr) return fail(B200KNN_E_ARG, "topk: the peer exchange stores the keys; out_keys must be NULL");
+  }
+  if (mode == B200KNN_MODE_EXACT) {
+    if (strided || o.tau0 || o.sample || peers)
+      return fail(B200KNN_E_ARG, "topk: MODE_EXACT takes no bank_row_stride, tau0, sample or peers");
+    return B200KNN_OK;
+  }
+  if (o.upper_keys) return fail(B200KNN_E_ARG, "topk: upper_keys needs MODE_EXACT");
+  if (groups && (strided || o.tau0 || o.sample || peers))
+    return fail(B200KNN_E_ARG, "topk: group ids take no bank_row_stride, tau0, sample or peers");
+  if (o.sample && o.tau0) return fail(B200KNN_E_ARG, "topk: sample takes no tau0");
+  if (peers && !o.sample && strided)
+    return fail(B200KNN_E_ARG, "topk: the peer exchange of a search visits every row (bank_row_stride 1)");
+  return B200KNN_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -102,51 +157,49 @@ size_t b200knn_topk_workspace_bytes(int64_t B, int64_t N, int dim, int k, int mo
   return plan.total_bytes + 256;
 }
 
-static int topk_impl(int mode, const void* q_hi, const void* q_lo, int q_dtype, int64_t q_ld,
-                     const void* bank_hi, const void* bank_lo, int bank_dtype, int bank_layout,
-                     int64_t bank_ld, int64_t B, int64_t N, int dim, int k, int64_t idx_offset,
-                     uint64_t* out_keys, void* workspace, size_t workspace_bytes, void* stream,
-                     float* dump, int32_t* diag, int flags, int64_t bank_row_stride = 1,
-                     const float* tau0 = nullptr, bool sample = false,
-                     const void* const* host_peer_out = nullptr, int n_peers = 0, int my_rank = 0,
-                     int64_t rows_per_owner = 0, const uint64_t* upper = nullptr,
-                     const int32_t* q_gid = nullptr, const int32_t* bank_gid = nullptr) {
+static int topk_impl(int mode, const TopkOperands& x, const TopkShape& s, const b200knn_topk_options& o,
+                     float* dump, int32_t* diag, int flags) {
+  const int64_t B = s.B, N = s.N;
+  const int dim = s.dim, k = s.k;
+  uint64_t* out_keys = x.out_keys;
+  int rc = check_options(mode, s, out_keys, o);
+  if (rc != B200KNN_OK) return rc;
   if (B < 0 || N <= 0 || dim <= 0) return fail(B200KNN_E_ARG, "topk: bad shape");
   if (k <= 0 || k > N) return fail(B200KNN_E_ARG, "topk: selected index k out of range");
-  if (N + idx_offset >= 0xFFFFFFFFll || idx_offset < 0)
+  if (N + s.idx_offset >= 0xFFFFFFFFll || s.idx_offset < 0)
     return fail(B200KNN_E_ARG, "topk: bank index does not fit 32 bits");
   if (B == 0) return B200KNN_OK;
-  if (!q_hi || !bank_hi || (!out_keys && n_peers == 0) || !workspace)
+  if (!x.q_hi || !x.bank_hi || (!out_keys && o.n_peers == 0) || !x.workspace)
     return fail(B200KNN_E_ARG, "topk: null pointer");
   b200knn::TopkPlan plan;
   if (!plan_for(mode, B, N, dim, k, &plan)) return fail(B200KNN_E_UNSUPPORTED, "topk: k too large (max 992)");
-  if (n_peers > 0 && plan.splits > 1)
-    return fail(B200KNN_E_UNSUPPORTED, "topk_scatter: this problem is planned with bank splits; use topk_ex");
-  uintptr_t ws = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255);
-  const size_t slack = ws - reinterpret_cast<uintptr_t>(workspace);
-  if (workspace_bytes < plan.total_bytes + slack) return fail(B200KNN_E_WORKSPACE, "topk: workspace too small");
+  if (o.n_peers > 0 && plan.splits > 1)
+    return fail(B200KNN_E_UNSUPPORTED, "topk: the peer exchange needs a problem planned without bank splits");
+  uintptr_t ws = (reinterpret_cast<uintptr_t>(x.workspace) + 255) & ~uintptr_t(255);
+  const size_t slack = ws - reinterpret_cast<uintptr_t>(x.workspace);
+  if (x.workspace_bytes < plan.total_bytes + slack) return fail(B200KNN_E_WORKSPACE, "topk: workspace too small");
   uint64_t* lists = reinterpret_cast<uint64_t*>(ws);
   float* st_tau = plan.chunks > 1 ? reinterpret_cast<float*>(ws + plan.lists_bytes) : nullptr;
   uint32_t* st_cnt = plan.chunks > 1 ? reinterpret_cast<uint32_t*>(st_tau + B) : nullptr;
   uint64_t* partial =
       plan.splits > 1 ? reinterpret_cast<uint64_t*>(ws + plan.lists_bytes + plan.state_bytes) : out_keys;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  cudaStream_t st = static_cast<cudaStream_t>(x.stream);
   cudaError_t e;
   if (mode == B200KNN_MODE_EXACT) {
-    if (q_dtype < 0 || q_dtype > 2 || bank_dtype < 0 || bank_dtype > 2)
+    if (x.q_dtype < 0 || x.q_dtype > 2 || x.bank_dtype < 0 || x.bank_dtype > 2)
       return fail(B200KNN_E_ARG, "topk: unknown dtype");
     b200knn::ExactParams p;
-    p.q = q_hi;
-    p.q_dtype = q_dtype;
-    p.q_ld = q_ld;
-    p.bank = bank_hi;
-    p.bank_dtype = bank_dtype;
-    if (bank_layout == B200KNN_LAYOUT_DN) {
-      p.bank_sd = bank_ld;
+    p.q = x.q_hi;
+    p.q_dtype = x.q_dtype;
+    p.q_ld = x.q_ld;
+    p.bank = x.bank_hi;
+    p.bank_dtype = x.bank_dtype;
+    if (x.bank_layout == B200KNN_LAYOUT_DN) {
+      p.bank_sd = x.bank_ld;
       p.bank_sn = 1;
-    } else if (bank_layout == B200KNN_LAYOUT_ND) {
+    } else if (x.bank_layout == B200KNN_LAYOUT_ND) {
       p.bank_sd = 1;
-      p.bank_sn = bank_ld;
+      p.bank_sn = x.bank_ld;
     } else {
       return fail(B200KNN_E_ARG, "topk: unknown bank layout");
     }
@@ -154,32 +207,32 @@ static int topk_impl(int mode, const void* q_hi, const void* q_lo, int q_dtype, 
     p.N = N;
     p.D = dim;
     p.k = k;
-    p.idx_offset = idx_offset;
+    p.idx_offset = s.idx_offset;
     p.n_qtiles = plan.n_qtiles;
     p.n_items = plan.n_items;
     p.split_rows = plan.split_rows;
     p.lists = lists;
     p.out = partial;
-    p.upper = upper;
-    p.q_gid = q_gid;
-    p.bank_gid = bank_gid;
+    p.upper = o.upper_keys;
+    p.q_gid = o.q_groups;
+    p.bank_gid = o.bank_groups;
     e = b200knn::launch_exact(p, plan.grid, plan.cap, st);
     if (e != cudaSuccess) return fail_cuda("topk(exact)", e);
   } else if (is_tc_mode(mode)) {
-    if (mode == B200KNN_MODE_F16X2 ? !bank_lo
-                                   : (mode != B200KNN_MODE_BF16 && mode != B200KNN_MODE_F16 && (!q_lo || !bank_lo)))
+    if (mode == B200KNN_MODE_F16X2 ? !x.bank_lo
+                                   : (mode != B200KNN_MODE_BF16 && mode != B200KNN_MODE_F16 && (!x.q_lo || !x.bank_lo)))
       return fail(B200KNN_E_ARG, "topk: split modes need the lo operands");
     b200knn::TcParams p;
     p.mode = mode;
-    p.q_hi = q_hi;
-    p.q_lo = q_lo;
-    p.bank_hi = bank_hi;
-    p.bank_lo = bank_lo;
+    p.q_hi = x.q_hi;
+    p.q_lo = x.q_lo;
+    p.bank_hi = x.bank_hi;
+    p.bank_lo = x.bank_lo;
     p.B = B;
     p.N = N;
     p.D = dim;
     p.k = k;
-    p.idx_offset = idx_offset;
+    p.idx_offset = s.idx_offset;
     p.n_qtiles = plan.n_qtiles;
     p.n_items = plan.n_items;
     p.split_rows = plan.split_rows;
@@ -190,16 +243,16 @@ static int topk_impl(int mode, const void* q_hi, const void* q_lo, int q_dtype, 
     p.st_cnt = st_cnt;
     p.lists = lists;
     p.out = partial;
-    p.bank_row_stride = bank_row_stride;
-    p.tau0 = tau0;
-    p.sample = sample;
-    p.n_peers = n_peers;
-    p.my_rank = my_rank;
-    p.rows_per_owner = rows_per_owner;
-    for (int g = 0; g < n_peers; ++g)
-      p.peer_out[g] = static_cast<uint64_t*>(const_cast<void*>(host_peer_out[g]));
-    p.q_gid = q_gid;
-    p.bank_gid = bank_gid;
+    p.bank_row_stride = o.bank_row_stride > 1 ? o.bank_row_stride : 1;
+    p.tau0 = o.tau0;
+    p.sample = o.sample != 0;
+    p.n_peers = o.n_peers;
+    p.my_rank = o.my_rank;
+    p.rows_per_owner = o.rows_per_owner;
+    for (int g = 0; g < o.n_peers; ++g)
+      p.peer_out[g] = static_cast<uint64_t*>(const_cast<void*>(o.host_peer_out[g]));
+    p.q_gid = o.q_groups;
+    p.bank_gid = o.bank_groups;
     const char* why = "";
     e = b200knn::launch_tc(p, plan.grid, plan.cap, st, dump, diag, flags, &why);
     if (e == cudaErrorNotSupported) return fail(B200KNN_E_UNSUPPORTED, "topk(tc): %s", why);
@@ -217,86 +270,24 @@ static int topk_impl(int mode, const void* q_hi, const void* q_lo, int q_dtype, 
   return B200KNN_OK;
 }
 
+int b200knn_topk_opt(int mode, const void* q_hi, const void* q_lo, int q_dtype, int64_t q_ld,
+                     const void* bank_hi, const void* bank_lo, int bank_dtype, int bank_layout,
+                     int64_t bank_ld, int64_t B, int64_t N, int dim, int k, int64_t idx_offset,
+                     uint64_t* out_keys, void* workspace, size_t workspace_bytes,
+                     const b200knn_topk_options* opts, void* stream) {
+  const b200knn_topk_options none = {};
+  return topk_impl(mode,
+                   {q_hi, q_lo, q_dtype, q_ld, bank_hi, bank_lo, bank_dtype, bank_layout, bank_ld, out_keys,
+                    workspace, workspace_bytes, stream},
+                   {B, N, dim, k, idx_offset}, opts ? *opts : none, nullptr, nullptr, 0);
+}
+
 int b200knn_topk(int mode, const void* q_hi, const void* q_lo, int q_dtype, int64_t q_ld,
                  const void* bank_hi, const void* bank_lo, int bank_dtype, int bank_layout,
                  int64_t bank_ld, int64_t B, int64_t N, int dim, int k, int64_t idx_offset,
                  uint64_t* out_keys, void* workspace, size_t workspace_bytes, void* stream) {
-  return topk_impl(mode, q_hi, q_lo, q_dtype, q_ld, bank_hi, bank_lo, bank_dtype, bank_layout,
-                   bank_ld, B, N, dim, k, idx_offset, out_keys, workspace, workspace_bytes, stream,
-                   nullptr, nullptr, 0);
-}
-
-int b200knn_topk_exact_below(const void* q, int q_dtype, int64_t q_ld, const void* bank, int bank_dtype,
-                             int bank_layout, int64_t bank_ld, int64_t B, int64_t N, int dim, int k,
-                             int64_t idx_offset, const uint64_t* upper_keys, uint64_t* out_keys,
-                             void* workspace, size_t workspace_bytes, void* stream) {
-  return topk_impl(B200KNN_MODE_EXACT, q, nullptr, q_dtype, q_ld, bank, nullptr, bank_dtype, bank_layout,
-                   bank_ld, B, N, dim, k, idx_offset, out_keys, workspace, workspace_bytes, stream, nullptr,
-                   nullptr, 0, 1, nullptr, false, nullptr, 0, 0, 0, upper_keys);
-}
-
-int b200knn_topk_excl(int mode, const void* q_hi, const void* q_lo, const void* bank_hi, const void* bank_lo,
-                      int64_t B, int64_t N, int dim, int k, int64_t idx_offset, const int32_t* q_groups,
-                      const int32_t* bank_groups, uint64_t* out_keys, void* workspace, size_t workspace_bytes,
-                      void* stream) {
-  if (!is_tc_mode(mode)) return fail(B200KNN_E_ARG, "topk_excl: tensor-core modes only");
-  if (!q_groups || !bank_groups) return fail(B200KNN_E_ARG, "topk_excl: null group ids");
-  return topk_impl(mode, q_hi, q_lo, 0, 0, bank_hi, bank_lo, 0, 0, 0, B, N, dim, k, idx_offset, out_keys,
-                   workspace, workspace_bytes, stream, nullptr, nullptr, 0, 1, nullptr, false, nullptr, 0, 0, 0,
-                   nullptr, q_groups, bank_groups);
-}
-
-int b200knn_topk_exact_excl(const void* q, int q_dtype, int64_t q_ld, const void* bank, int bank_dtype,
-                            int bank_layout, int64_t bank_ld, int64_t B, int64_t N, int dim, int k,
-                            int64_t idx_offset, const int32_t* q_groups, const int32_t* bank_groups,
-                            const uint64_t* upper_keys, uint64_t* out_keys, void* workspace,
-                            size_t workspace_bytes, void* stream) {
-  if (!q_groups || !bank_groups) return fail(B200KNN_E_ARG, "topk_exact_excl: null group ids");
-  return topk_impl(B200KNN_MODE_EXACT, q, nullptr, q_dtype, q_ld, bank, nullptr, bank_dtype, bank_layout,
-                   bank_ld, B, N, dim, k, idx_offset, out_keys, workspace, workspace_bytes, stream, nullptr,
-                   nullptr, 0, 1, nullptr, false, nullptr, 0, 0, 0, upper_keys, q_groups, bank_groups);
-}
-
-int b200knn_topk_ex(int mode, const void* q_hi, const void* q_lo, const void* bank_hi,
-                    const void* bank_lo, int64_t B, int64_t n_visit, int dim, int k, int64_t idx_offset,
-                    int64_t bank_row_stride, const float* tau0, uint64_t* out_keys, void* workspace,
-                    size_t workspace_bytes, void* stream) {
-  if (!is_tc_mode(mode)) return fail(B200KNN_E_ARG, "topk_ex: tensor-core modes only");
-  if (bank_row_stride < 1) return fail(B200KNN_E_ARG, "topk_ex: bank_row_stride must be >= 1");
-  return topk_impl(mode, q_hi, q_lo, 0, 0, bank_hi, bank_lo, 0, 0, 0, B, n_visit, dim, k, idx_offset,
-                   out_keys, workspace, workspace_bytes, stream, nullptr, nullptr, 0, bank_row_stride,
-                   tau0);
-}
-
-int b200knn_topk_sample(int mode, const void* q_hi, const void* q_lo, const void* bank_hi,
-                        const void* bank_lo, int64_t B, int64_t n_visit, int dim,
-                        int64_t bank_row_stride, uint64_t* out_keys, void* workspace,
-                        size_t workspace_bytes, void* stream) {
-  if (!is_tc_mode(mode)) return fail(B200KNN_E_ARG, "topk_sample: tensor-core modes only");
-  if (bank_row_stride < 1) return fail(B200KNN_E_ARG, "topk_sample: bank_row_stride must be >= 1");
-  if (n_visit < B200KNN_SAMPLE_R) return fail(B200KNN_E_ARG, "topk_sample: fewer than 16 rows to sample");
-  return topk_impl(mode, q_hi, q_lo, 0, 0, bank_hi, bank_lo, 0, 0, 0, B, n_visit, dim, B200KNN_SAMPLE_R, 0,
-                   out_keys, workspace, workspace_bytes, stream, nullptr, nullptr, 0, bank_row_stride,
-                   nullptr, true);
-}
-
-int b200knn_topk_sample_scatter(int mode, const void* q_hi, const void* q_lo, const void* bank_hi,
-                                const void* bank_lo, int64_t B, int64_t n_visit, int dim,
-                                int64_t bank_row_stride, const void* const* host_peer_out, int n_peers,
-                                int my_rank, int64_t rows_per_owner, void* workspace, size_t workspace_bytes,
-                                void* stream) {
-  if (!is_tc_mode(mode)) return fail(B200KNN_E_ARG, "topk_sample_scatter: tensor-core modes only");
-  if (bank_row_stride < 1) return fail(B200KNN_E_ARG, "topk_sample_scatter: bank_row_stride must be >= 1");
-  if (n_visit < B200KNN_SAMPLE_R) return fail(B200KNN_E_ARG, "topk_sample_scatter: fewer than 16 rows to sample");
-  if (!host_peer_out || n_peers < 1 || n_peers > 8 || my_rank < 0 || my_rank >= n_peers)
-    return fail(B200KNN_E_ARG, "topk_sample_scatter: 1..8 peers and a rank among them");
-  if (rows_per_owner <= 0 || rows_per_owner * n_peers < B)
-    return fail(B200KNN_E_ARG, "topk_sample_scatter: rows_per_owner * n_peers must cover B");
-  for (int g = 0; g < n_peers; ++g)
-    if (!host_peer_out[g]) return fail(B200KNN_E_ARG, "topk_sample_scatter: null peer buffer");
-  return topk_impl(mode, q_hi, q_lo, 0, 0, bank_hi, bank_lo, 0, 0, 0, B, n_visit, dim, B200KNN_SAMPLE_R, 0, nullptr,
-                   workspace, workspace_bytes, stream, nullptr, nullptr, 0, bank_row_stride, nullptr, true,
-                   host_peer_out, n_peers, my_rank, rows_per_owner);
+  return b200knn_topk_opt(mode, q_hi, q_lo, q_dtype, q_ld, bank_hi, bank_lo, bank_dtype, bank_layout, bank_ld, B,
+                          N, dim, k, idx_offset, out_keys, workspace, workspace_bytes, nullptr, stream);
 }
 
 int b200knn_broadcast_f32(const float* src, int64_t n, const void* const* host_peer_dst, int n_peers,
@@ -312,22 +303,6 @@ int b200knn_broadcast_f32(const float* src, int64_t n, const void* const* host_p
   return e == cudaSuccess ? B200KNN_OK : fail_cuda("broadcast_f32", e);
 }
 
-int b200knn_topk_scatter(int mode, const void* q_hi, const void* q_lo, const void* bank_hi,
-                         const void* bank_lo, int64_t B, int64_t N, int dim, int k, int64_t idx_offset,
-                         const float* tau0, const void* const* host_peer_out, int n_peers, int my_rank,
-                         int64_t rows_per_owner, void* workspace, size_t workspace_bytes, void* stream) {
-  if (!is_tc_mode(mode)) return fail(B200KNN_E_ARG, "topk_scatter: tensor-core modes only");
-  if (!host_peer_out || n_peers < 1 || n_peers > 8 || my_rank < 0 || my_rank >= n_peers)
-    return fail(B200KNN_E_ARG, "topk_scatter: 1..8 peers and a rank among them");
-  if (rows_per_owner <= 0 || rows_per_owner * n_peers < B)
-    return fail(B200KNN_E_ARG, "topk_scatter: rows_per_owner * n_peers must cover B");
-  for (int g = 0; g < n_peers; ++g)
-    if (!host_peer_out[g]) return fail(B200KNN_E_ARG, "topk_scatter: null peer buffer");
-  return topk_impl(mode, q_hi, q_lo, 0, 0, bank_hi, bank_lo, 0, 0, 0, B, N, dim, k, idx_offset, nullptr,
-                   workspace, workspace_bytes, stream, nullptr, nullptr, 0, 1, tau0, false,
-                   host_peer_out, n_peers, my_rank, rows_per_owner);
-}
-
 // Test hook (not part of the product path): same as b200knn_topk for the tensor-core
 // modes, additionally dumping the raw (B,N) fp32 similarity tiles and the pipeline
 // diagnostic word.  Used by tests/ to validate the MMA path against a plain GEMM.
@@ -335,21 +310,8 @@ int b200knn_debug_topk_dump(int mode, const void* q_hi, const void* q_lo, const 
                             const void* bank_lo, int64_t B, int64_t N, int dim, int k,
                             uint64_t* out_keys, void* workspace, size_t workspace_bytes,
                             float* dump, int32_t* diag, int flags, void* stream) {
-  return topk_impl(mode, q_hi, q_lo, 0, 0, bank_hi, bank_lo, 0, 0, 0, B, N, dim, k, 0, out_keys,
-                   workspace, workspace_bytes, stream, dump, diag, flags);
-}
-
-// Plan introspection for the host shim / bench (how the work was split).
-int b200knn_plan_info(int mode, int64_t B, int64_t N, int dim, int k, int64_t* out6) {
-  b200knn::TopkPlan plan;
-  if (!out6 || !plan_for(mode, B, N, dim, k, &plan)) return fail(B200KNN_E_ARG, "plan_info: bad argument");
-  out6[0] = plan.n_qtiles;
-  out6[1] = plan.splits;
-  out6[2] = plan.split_rows;
-  out6[3] = plan.n_items;
-  out6[4] = plan.grid;
-  out6[5] = plan.cap;
-  return B200KNN_OK;
+  return topk_impl(mode, {q_hi, q_lo, 0, 0, bank_hi, bank_lo, 0, 0, 0, out_keys, workspace, workspace_bytes, stream},
+                   {B, N, dim, k, 0}, b200knn_topk_options{}, dump, diag, flags);
 }
 
 int b200knn_set_l2_chunk_bytes(int64_t bytes) {
@@ -358,10 +320,16 @@ int b200knn_set_l2_chunk_bytes(int64_t bytes) {
   return B200KNN_OK;
 }
 
+// Plan introspection for the host shim / bench (how the work was split).
 int b200knn_plan_info_ex(int mode, int64_t B, int64_t N, int dim, int k, int64_t* out9) {
   b200knn::TopkPlan plan;
   if (!out9 || !plan_for(mode, B, N, dim, k, &plan)) return fail(B200KNN_E_ARG, "plan_info_ex: bad argument");
-  if (b200knn_plan_info(mode, B, N, dim, k, out9) != B200KNN_OK) return B200KNN_E_ARG;
+  out9[0] = plan.n_qtiles;
+  out9[1] = plan.splits;
+  out9[2] = plan.split_rows;
+  out9[3] = plan.n_items;
+  out9[4] = plan.grid;
+  out9[5] = plan.cap;
   out9[6] = plan.chunks;
   out9[7] = plan.chunk_rows;
   out9[8] = plan.slots;

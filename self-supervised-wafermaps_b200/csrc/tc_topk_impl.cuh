@@ -728,18 +728,9 @@ cudaError_t launch_t(const TcParams& p, int grid, cudaStream_t stream, float* du
 template <int MODE, int BLOCK_N, bool DEBUG, bool PAIR>
 cudaError_t launch_cap(const TcParams& p, int grid, int cap, cudaStream_t stream, float* dump,
                        int32_t* diag, int flags, const char** why) {
-  if (p.sample) {
-    if (DEBUG || p.k != kSampleR || p.tau0 != nullptr) {
-      *why = "the sampling variant keeps exactly 16 values per row";
-      return cudaErrorNotSupported;
-    }
-    return launch_t<MODE, BLOCK_N, 2, false, PAIR, true>(p, grid, stream, nullptr, diag, 0, why);
-  }
+  // which options combine is checked before planning (api.cu); the debug hook passes none
+  if (p.sample) return launch_t<MODE, BLOCK_N, 2, false, PAIR, true>(p, grid, stream, nullptr, diag, 0, why);
   if (p.bank_gid != nullptr) {
-    if (DEBUG || p.tau0 != nullptr || p.n_peers > 0) {
-      *why = "group exclusion runs without debug output, thresholds or a peer exchange";
-      return cudaErrorNotSupported;
-    }
     switch (cap) {
       case 64: return launch_t<MODE, BLOCK_N, 2, false, PAIR, false, true>(p, grid, stream, nullptr, diag, 0, why);
       case 128: return launch_t<MODE, BLOCK_N, 4, false, PAIR, false, true>(p, grid, stream, nullptr, diag, 0, why);

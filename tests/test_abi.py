@@ -27,9 +27,9 @@ def test_library_exports_every_declared_symbol():
         assert hasattr(lib, name), name
 
 
-def test_version_and_error_string():
+def test_abi_version_and_error_string():
     lib = _lib.load()
-    assert lib.b200knn_version() == 142
+    assert lib.b200knn_version() == 150
     assert isinstance(lib.b200knn_last_error(), bytes)
 
 
@@ -45,6 +45,54 @@ def test_argument_validation_without_gpu():
     rc = lib.b200knn_prepare_rows(1, 7, 0, 4, 8, 4, 1, 1, None, None)  # bad dtype
     assert rc == -1
     assert lib.b200knn_topk_workspace_bytes(64, 1000, 512, 2000, 0) == 0  # k too large
+
+
+PEERS = dict(peers=[1, 1], n_peers=2, my_rank=0, rows_per_owner=2)  # a valid exchange for B = 4
+BF16, EXACT = _lib.MODE_BF16, _lib.MODE_EXACT
+
+
+@pytest.mark.parametrize("mode,opts,message", [
+    (EXACT, dict(bank_row_stride=2), "MODE_EXACT takes no"),
+    (EXACT, dict(tau0=1), "MODE_EXACT takes no"),
+    (EXACT, dict(sample=1), "MODE_EXACT takes no"),
+    (EXACT, dict(PEERS), "MODE_EXACT takes no"),
+    (BF16, dict(upper_keys=1), "upper_keys needs MODE_EXACT"),
+    (BF16, dict(q_groups=1, bank_groups=1, bank_row_stride=2), "group ids take no"),
+    (BF16, dict(q_groups=1, bank_groups=1, tau0=1), "group ids take no"),
+    (BF16, dict(q_groups=1, bank_groups=1, sample=1), "group ids take no"),
+    (BF16, dict(q_groups=1, bank_groups=1, **PEERS), "group ids take no"),
+    (BF16, dict(sample=1, tau0=1), "sample takes no tau0"),
+    (BF16, dict(bank_row_stride=2, **PEERS), "visits every row"),
+    (BF16, dict(q_groups=1), "null group ids"),
+    (EXACT, dict(bank_groups=1), "null group ids"),
+    (BF16, dict(bank_row_stride=-1), "bank_row_stride must be >= 0"),
+    (BF16, dict(sample=1, k=15), "sample needs k == 16"),
+    (BF16, dict(sample=1, N=15), "sample needs k == 16 and at least 16 rows"),
+    (BF16, dict(PEERS, n_peers=9, peers=[1] * 9), "1..8 peers"),
+    (BF16, dict(PEERS, n_peers=0), "1..8 peers"),
+    (BF16, dict(PEERS, peers=None), "1..8 peers"),
+    (BF16, dict(PEERS, my_rank=2), "1..8 peers"),
+    (BF16, dict(PEERS, my_rank=-1), "1..8 peers"),
+    (BF16, dict(PEERS, rows_per_owner=1), "must cover B"),
+    (BF16, dict(PEERS, peers=[1, None]), "null peer buffer"),
+    (BF16, dict(PEERS, out_keys=1), "out_keys must be NULL"),
+    (BF16, dict(out_keys=None), "null pointer"),
+])
+def test_topk_options_refused_without_gpu(mode, opts, message):
+    """Every combination of b200knn_topk_opt's options that no search implements is refused before
+    any planning, including sample or a row stride together with group ids."""
+    lib = _lib.load()
+    opts = dict(opts)
+    k, N, out_keys = opts.pop("k", 16), opts.pop("N", 100), opts.pop("out_keys", None if "peers" in opts else 1)
+    peers = opts.pop("peers", None)
+    o = _lib.TopkOptions(**opts)
+    if peers is not None:
+        o.host_peer_out = (ctypes.c_void_p * len(peers))(*peers)
+    # (mode, q_hi, q_lo, q_dtype, q_ld, bank_hi, bank_lo, bank_dtype, bank_layout, bank_ld, B, N, dim, k,
+    #  idx_offset, out_keys, workspace, workspace_bytes, opts, stream)
+    rc = lib.b200knn_topk_opt(mode, 1, 1, 0, 64, 1, 1, 0, 1, 64, 4, N, 64, k, 0, out_keys, 1, 1 << 20, o, None)
+    assert rc == -1
+    assert message.encode() in lib.b200knn_last_error()
 
 
 def test_plan_is_deterministic_and_covers_bank():

@@ -1,7 +1,7 @@
 """GPU, >= 2 devices: the bank-row-sharded mode over NCCL + NVLink peer memory must reproduce the
 single-GPU result BIT FOR BIT on every rank (SURVEY.md §8e invariant) — exact, fp32 (bit-exact,
 fused route_scatter / rescore_scatter exchange and the NCCL fallback) and bf16 (fused
-b200knn_topk_scatter and NCCL all-to-all), including a batch large enough for the fused exchange,
+b200knn_topk_opt's peer exchange and NCCL all-to-all), including a batch large enough for the fused exchange,
 forced second-level rows and the host-driven fallback.  Skipped on a single-GPU box."""
 import os
 import socket

@@ -249,8 +249,8 @@ def test_prepass_threshold_does_not_change_results(mode):
 
 @pytest.mark.parametrize("mode", ["bf16", "tf32x3"])
 @pytest.mark.parametrize("B,N,stride", [(200, 300000, 62), (513, 40000, 8), (64, 811457, 62), (3, 4096, 1)])
-def test_register_sample_is_a_valid_threshold(mode, B, N, stride):
-    """b200knn_topk_sample keeps, per row, the 16 best 32-column chunk maxima in registers.  Every
+def test_sample_option_is_a_valid_threshold(mode, B, N, stride):
+    """The sample option of b200knn_topk_opt keeps, per row, the 16 best 32-column chunk maxima in registers.  Every
     value it returns must be one of the row's sampled similarities (bit for bit), the best one is
     the row maximum, the list is sorted, and its 16-th value is <= the true 16-th best sampled
     similarity (so it is a valid admission threshold) without being much weaker."""
@@ -262,8 +262,8 @@ def test_register_sample_is_a_valid_threshold(mode, B, N, stride):
     pq = K.prepare_rows(q, mode, vectors_are_columns=False)
     n_visit = (N + stride - 1) // stride
     kk = min(64, n_visit)
-    lists = K._tc_call(mode, pq, pb, B, n_visit, D, kk, 0, stride, None, q.device)
-    regs = K._tc_call(mode, pq, pb, B, n_visit, D, 16, 0, stride, None, q.device, sample=True)
+    lists = K._search(mode, pq, pb, B, n_visit, D, kk, stride=stride)
+    regs = K._search(mode, pq, pb, B, n_visit, D, 16, stride=stride, sample=True)
     s_list, _ = b200knn.decode_keys(lists)
     s_reg, i_reg = b200knn.decode_keys(regs)
     assert bool((i_reg == 0).all())

@@ -1,6 +1,6 @@
 """CPU: group exclusion inside the neighbour search (topk_keys(exclude=...), knn_predict_multi /
-knn_topk(query_groups=, bank_groups=)).  The C ABI's argument checks of the two group-excluding
-entry points, the Python argument errors and the k bound (raised before any search, so they need no
+knn_topk(query_groups=, bank_groups=)).  The C ABI's argument checks of the group-excluding
+options, the Python argument errors and the k bound (raised before any search, so they need no
 GPU), and the rule that picks which leave-one-group-out searches skip the group inside the search."""
 import pytest
 import torch
@@ -10,26 +10,22 @@ from b200knn import _lib
 from b200knn import knn as K
 
 
-def test_excl_abi_refuses_null_group_ids_without_gpu():
+def test_topk_opt_refuses_null_group_ids_without_gpu():
     lib = _lib.load()
-    # b200knn_topk_excl(mode, q_hi, q_lo, bank_hi, bank_lo, B, N, dim, k, idx_offset, q_groups, bank_groups,
-    #                   out_keys, workspace, workspace_bytes, stream)
-    for qg, bg in ((None, 1), (1, None), (None, None)):
-        assert lib.b200knn_topk_excl(_lib.MODE_BF16, 1, None, 1, None, 4, 100, 64, 5, 0, qg, bg, 1, 1, 1 << 20,
-                                     None) == -1
-        assert b"null group ids" in lib.b200knn_last_error()
-        # b200knn_topk_exact_excl(q, q_dtype, q_ld, bank, bank_dtype, bank_layout, bank_ld, B, N, dim, k,
-        #                         idx_offset, q_groups, bank_groups, upper_keys, out_keys, ws, ws_bytes, stream)
-        assert lib.b200knn_topk_exact_excl(1, 0, 64, 1, 0, 1, 64, 4, 100, 64, 5, 0, qg, bg, None, 1, 1, 1 << 20,
-                                           None) == -1
-        assert b"null group ids" in lib.b200knn_last_error()
-    assert lib.b200knn_topk_excl(_lib.MODE_EXACT, 1, None, 1, None, 4, 100, 64, 5, 0, 1, 1, 1, 1, 1 << 20,
-                                 None) == -1
-    assert b"tensor-core modes only" in lib.b200knn_last_error()
-    # the shape checks of b200knn_topk apply as they are
-    assert lib.b200knn_topk_exact_excl(1, 0, 64, 1, 0, 1, 64, 4, 100, 64, 101, 0, 1, 1, None, 1, 1, 1 << 20,
-                                       None) == -1
-    assert b"k out of range" in lib.b200knn_last_error()
+
+    def topk_opt(mode, k, qg, bg):
+        # (mode, q_hi, q_lo, q_dtype, q_ld, bank_hi, bank_lo, bank_dtype, bank_layout, bank_ld, B, N, dim, k,
+        #  idx_offset, out_keys, workspace, workspace_bytes, opts, stream)
+        return lib.b200knn_topk_opt(mode, 1, None, 0, 64, 1, None, 0, 1, 64, 4, 100, 64, k, 0, 1, 1, 1 << 20,
+                                    _lib.TopkOptions(q_groups=qg, bank_groups=bg), None)
+
+    for mode in (_lib.MODE_BF16, _lib.MODE_EXACT):
+        for qg, bg in ((None, 1), (1, None)):
+            assert topk_opt(mode, 5, qg, bg) == -1
+            assert b"null group ids" in lib.b200knn_last_error()
+        # the shape checks of b200knn_topk apply as they are
+        assert topk_opt(mode, 101, 1, 1) == -1
+        assert b"k out of range" in lib.b200knn_last_error()
 
 
 def _case(B=4, N=50):
