@@ -81,9 +81,14 @@ const char* b200knn_last_error(void);
  * n_vec vectors of dimension dim, leading dimension ld in ELEMENTS) into the
  * K-major row layout the tensor-core kernels stream with TMA:
  *   mode BF16  : dst_hi = (n_vec, dim) bf16 (round-to-nearest-even); dst_lo unused
- *   mode TF32X3: dst_hi = (n_vec, dim) f32 holding tf32-truncated values,
+ *   mode TF32X3: dst_hi = (n_vec, dim) f32 holding x rounded to tf32 (10 mantissa bits), to nearest
+ *                with ties away from zero (cvt.rna),
  *                dst_lo = (n_vec, dim) f32 holding  x - hi  (exact)
  *   mode BF16X3: dst_hi = (n_vec, dim) bf16 = rn(x), dst_lo = (n_vec, dim) bf16 = rn(x - hi)
+ *   mode F16 / F16X2: dst_hi = (n_vec, dim) fp16 = rn(sat(x)), sat clamping to +-65504; dst_lo
+ *                (optional) = rn(sat(x - hi))
+ *   mode F32ROWS: dst_hi = (n_vec, dim) f32 = x
+ * rn = round to nearest, ties to even; dim is padded to a multiple of 64 with +0 columns.
  */
 int b200knn_prepare_rows(const void* src, int src_dtype, int src_layout,
                          int64_t n_vec, int dim, int64_t ld, int mode,
@@ -189,8 +194,11 @@ int b200knn_topk_opt(int mode,
  * Merge G sorted candidate lists per query into one (replaces nothing in the
  * reference; it is the exchange step of the bank-row-sharded mode, applied to
  * the buffer an all-gather of per-shard b200knn_topk outputs produces).
- *   keys_in : (G, B, k_in) uint64, each (g,b,:) sorted descending
- *   keys_out: (B, k_out) uint64 sorted descending, k_out <= G*k_in
+ *   keys_in : (G, B, k_in) uint64, each (g,b,:) a zero-terminated set: its non-empty keys first,
+ *             in any order (sorted descending is one such order), then only empty (0) keys.  The
+ *             first empty key ends a list; keys may repeat within and across lists.
+ *   keys_out: (B, k_out) uint64 sorted descending, the best k_out keys of the union (repeats
+ *             counted), zero-filled, k_out <= G*k_in
  */
 int b200knn_merge(const uint64_t* keys_in, int G, int64_t B, int k_in, int k_out,
                   uint64_t* keys_out, void* stream);

@@ -211,3 +211,34 @@ def test_north_star_shape_properties():
     lab = torch.randint(0, 9, (N,), device=DEV)
     pred = b200knn.vote(keys, lab, 9, 0.1)
     assert sorted(pred[0].tolist()) == list(range(9))
+
+
+def test_exact_at_north_star_size_against_seq_oracle():
+    """The large-bank tests take mode "exact" as their reference at N = 811,457 (test_gpu_tc.py's
+    test_large_bank_against_exact_mode draws the same bank and queries); here it meets the
+    sequential-fma oracle at that size, for 16 of those queries."""
+    N, D, k, B = 811457, 512, 200, 256
+    g = torch.Generator(device=DEV).manual_seed(811)
+    bank = torch.nn.functional.normalize(torch.randn(N, D, generator=g, device=DEV), dim=1).t().contiguous()
+    q = torch.nn.functional.normalize(torch.randn(B, D, generator=g, device=DEV), dim=1)[:16].contiguous()
+    sims, idx = b200knn.knn_topk(q, bank, k, mode="exact")
+    ss, si = O.topk_seqfma(q.cpu().numpy(), bank.cpu().numpy(), k)
+    assert np.array_equal(idx.cpu().numpy(), si)
+    assert np.array_equal(sims.cpu().numpy().view(np.uint32), ss.view(np.uint32))
+
+
+@pytest.mark.parametrize("k", [49, 112])
+@pytest.mark.parametrize("B,N,D", [(64, 30011, 200), (300, 5003, 128)])
+def test_exact_list_capacity_256_against_seq_oracle(B, N, D, k):
+    from b200knn import knn as K
+
+    plan = K.plan_info(B, N, D, k, "exact")
+    assert plan["list_capacity"] == 256 and plan["splits"] > 1, plan
+    g = torch.Generator(device=DEV).manual_seed(B + k)
+    bank = torch.randn(D, N, generator=g, device=DEV)
+    bank[:, N // 2:N // 2 + 40] = bank[:, :40]  # exact duplicates: ties broken by the lower index
+    q = torch.randn(B, D, generator=g, device=DEV)
+    sims, idx = b200knn.knn_topk(q, bank, k, mode="exact")
+    ss, si = O.topk_seqfma(q.cpu().numpy(), bank.cpu().numpy(), k)
+    assert np.array_equal(idx.cpu().numpy(), si)
+    assert np.array_equal(sims.cpu().numpy().view(np.uint32), ss.view(np.uint32))
