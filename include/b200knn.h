@@ -322,6 +322,28 @@ int b200knn_rescore(const void* q, int q_dtype, int64_t q_ld, const float* rows_
 size_t b200knn_rescore_workspace_bytes(int64_t B, int k_in);
 
 /*
+ * b200knn_rescore_vote: knn_predict's class ranking from the approximate candidates cand_keys
+ * (B, k_in), k_in < N, re-scoring only the candidates near rank k (fp32 queries, one fp32 row
+ * array; DESIGN.md §4.1c).  With E the bound of b200knn_rescore:
+ *   band_info (B, 4) int32 out: (p, r, bits of E, 0), p = the leading candidates certainly in the
+ *             exact top k, candidates p+1..r re-scored; p = -1: the row was not attempted
+ *   band_keys (B, k_in) out: those candidates, front-filled, zero tail
+ *   pred      (B, C) int64: the exact mode's class ranking where uncertified[b] == 0; rows with
+ *             uncertified[b] == 1 are left unset for the caller to recompute
+ *   status    int32[2], caller-zeroed: status[0] = 1 / 2 label / neighbour index out of range
+ *             (b200knn_vote's flag) on certified neighbour sets; status[1] += uncertified rows
+ *   workspace b200knn_rescore_workspace_bytes(B, k_in) bytes; 1 <= C <= 256, t != 0.
+ */
+#define B200KNN_RESCORE_VOTE_MAX_CLASSES 256
+int b200knn_rescore_vote(const float* q, int64_t q_ld, const float* rows, int64_t N, int dim,
+                         const uint64_t* cand_keys, int64_t B, int k_in, int k, float err_coef,
+                         float err_abs, float max_abs, const float* bank_max_norm,
+                         const int64_t* labels, int64_t n_labels, int C, double t,
+                         uint64_t* band_keys, int32_t* band_info, int64_t* pred,
+                         int32_t* uncertified, int32_t* status, void* workspace,
+                         size_t workspace_bytes, void* stream);
+
+/*
  * Sharded fp32 mode (no counterpart in the reference, which is single-device): the owner of a
  * query merges every shard's approximate candidates, has each candidate re-scored by the shard
  * that holds its bank row, merges the exact keys that come back and certifies the result.

@@ -821,7 +821,6 @@ def _rescored_level(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, l
     """One cascade level, nothing synchronises: (keys (B,k), uncertified flags (B,) int32, count int32[1]).
     n_bad: optional zeroed int32[1] the count is accumulated into (the caller's status word).
     exclude: ``topk_keys``' checked (query ids, bank ids, m) for these rows."""
-    lib = _lib.load()
     B, D = feature.shape
     cfg = level_config(level, D)
     N = feature_bank.shape[1]
@@ -833,10 +832,20 @@ def _rescored_level(feature: torch.Tensor, feature_bank: torch.Tensor, k: int, l
         # re-scoring kernel would read an empty k_in-th slot as uncertified).  The certificate's
         # max row norm of the whole bank still bounds the reduced bank's.
         k_in = min(k_in, N - exclude[2])
-    dev = feature.device
     # no repair pass on the candidates: a row its sampled threshold starved has an empty k_in-th
     # slot, which the re-scoring kernel reports as uncertified
     cand = topk_keys(feature, feature_bank, k_in, cfg["cand"], idx_offset, repair=False, exclude=exclude)
+    return _rescore_candidates(feature, feature_bank, cand, k, cfg, idx_offset, n_bad)
+
+
+def _rescore_candidates(feature: torch.Tensor, feature_bank: torch.Tensor, cand: torch.Tensor, k: int, cfg: dict,
+                        idx_offset: int, n_bad: Optional[torch.Tensor] = None):
+    """The re-scoring and certificate of a level on its candidates cand (B, k_in): ``_rescored_level``'s result."""
+    lib = _lib.load()
+    B, D = feature.shape
+    N = feature_bank.shape[1]
+    k_in = cand.shape[1]
+    dev = feature.device
     pb = bank_cache.get(feature_bank, cfg["cand"])
     rows_a, rows_b = pb.rescore_rows()
     max_norm = pb.max_norm()
@@ -1341,6 +1350,93 @@ def _vote_step(keys, feature_labels, num_classes, knn_t, flag):
     return vote(keys, feature_labels, num_classes, knn_t, check_labels=False, return_flag=True, flag=flag)[0]
 
 
+# knn_predict returns the class ranking only, so a rescored-mode call re-scores only the candidates
+# near rank k and certifies the ranking from intervals on the others (b200knn_rescore_vote,
+# DESIGN §4.1c).  Rows it cannot certify are re-scored in full and voted as before.  The switch
+# exists for A/B measurements (scripts/bench_vote_certificate.py) and tests; results are the same.
+CERTIFIED_VOTE = {"enabled": os.environ.get("B200KNN_CERTIFIED_VOTE", "1") == "1"}
+CERTIFIED_VOTE_MAX_CLASSES = 256  # B200KNN_RESCORE_VOTE_MAX_CLASSES
+
+
+def _certified_vote_applies(feature, feature_bank, num_classes, knn_k, knn_t, mode, exclude) -> bool:
+    """Whether a knn_predict call takes the certified vote: a rescored mode with one fp32 row array,
+    a single temperature, no group exclusion, and k_in < N at every margin (k_in <= max(k, MAX_K))."""
+    return (CERTIFIED_VOTE["enabled"] and mode in RESCORED_MODES and mode != "fp32_tf32"
+            and not isinstance(knn_t, tuple) and float(knn_t) != 0.0 and exclude is None
+            and int(num_classes) <= CERTIFIED_VOTE_MAX_CLASSES
+            and feature_bank.shape[1] > max(int(knn_k), MAX_K))
+
+
+def _predict_certified(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t, mode, track, boost, status):
+    """The certified vote of a rescored-mode call, nothing synchronises: (pred (B,C), flags (B,) int32, fix).
+    status[1] counts the rows it leaves uncertified; fix(rows, n) returns their exact keys: their full
+    candidate lists re-scored under the first level's certificate, then the rest of the cascade."""
+    lib = _lib.load()
+    _check_feature_bank(feature, feature_bank)
+    B, D = feature.shape
+    N = feature_bank.shape[1]
+    k, C = int(knn_k), int(num_classes)
+    dev = feature.device
+    levels = _cascade_levels(feature_bank, mode, track, boost)
+    cfg = level_config(levels[0], D)
+    k_in = min(N, k + cfg["margin"], max(k, MAX_K))
+    cand = topk_keys(feature, feature_bank, k_in, cfg["cand"], repair=False)
+    pb = bank_cache.get(feature_bank, cfg["cand"])
+    rows, _ = pb.rescore_rows()
+    max_norm = pb.max_norm()
+    q = feature if feature.dtype == torch.float32 else feature.float()
+    if q.stride(1) != 1:
+        q = q.contiguous()
+    labels = (feature_labels if feature_labels.dtype == torch.int64 else feature_labels.long()).contiguous().view(-1)
+    pred = torch.empty((B, C), dtype=torch.int64, device=dev)
+    with torch.cuda.device(dev):
+        flags = torch.empty((B,), dtype=torch.int32, device=dev)
+        band = torch.empty((B, k_in), dtype=torch.int64, device=dev)
+        info = torch.empty((B, 4), dtype=torch.int32, device=dev)
+        ws_bytes = int(lib.b200knn_rescore_workspace_bytes(B, k_in))
+        ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+        with _Timed("rescore"):
+            rc = lib.b200knn_rescore_vote(q.data_ptr(), q.stride(0), rows.data_ptr(), N, D, cand.data_ptr(), B, k_in, k,
+                                          float(cfg["err_coef"]),
+                                          float(cfg.get("err_abs", 0.0)) * math.sqrt(padded_dim(D)),
+                                          float(cfg.get("max_abs", 0.0)), max_norm.data_ptr(), labels.data_ptr(),
+                                          labels.numel(), C, float(knn_t), band.data_ptr(), info.data_ptr(),
+                                          pred.data_ptr(), flags.data_ptr(), status.data_ptr(), ws.data_ptr(),
+                                          ws_bytes, _stream())
+        _lib.check(rc, "rescore_vote")
+
+    def fix(rows_bad, n_rows_bad):
+        last_rescore_stats["band_info"] = info  # (B, 4): p, r per row (band_stats)
+        if rows_bad is None:
+            _note_first_level(feature_bank, mode, levels, B, 0, track)
+            last_rescore_stats["vote_fallback"] = 0
+            return None
+        sub = feature[rows_bad].contiguous()
+        keys, left_flags, n_left = _rescore_candidates(sub, feature_bank, cand[rows_bad].contiguous(), k, cfg, 0)
+        n_left = int(n_left.item())
+        _note_first_level(feature_bank, mode, levels, B, n_left, track)
+        last_rescore_stats["vote_fallback"] = n_rows_bad
+        if n_left:
+            left = left_flags.nonzero(as_tuple=False).view(-1)
+            keys[left] = _cascade_fix(sub, feature_bank, k, levels[1:], left, 0)
+        return keys
+
+    return pred, flags, fix
+
+
+def band_stats() -> dict:
+    """Band sizes (candidates re-scored per row) of the last certified-vote call: mean, max, and the
+    rows it left to the full re-scoring.  Synchronises; for measurements."""
+    info = last_rescore_stats.get("band_info")
+    if info is None:
+        return {}
+    served = info[:, 0] >= 0
+    size = (info[:, 1] - info[:, 0])[served].double()
+    return {"rows": int(info.shape[0]), "mean": float(size.mean()) if size.numel() else 0.0,
+            "max": int(size.max()) if size.numel() else 0, "sure_mean": float(info[served, 0].double().mean())
+            if size.numel() else 0.0, "fallback_rows": int(last_rescore_stats.get("vote_fallback", 0))}
+
+
 def _predict_enqueue(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t, mode, track=True, boost=1,
                      exclude=None):
     """Everything of one tensor-core-mode call, enqueued without a host synchronisation (so it can
@@ -1350,6 +1446,10 @@ def _predict_enqueue(feature, feature_bank, feature_labels, num_classes, knn_k, 
     knn_t: a temperature, or a (ks, ts) grid (``_vote_step``; pred is then (B, n_k*n_t*C))."""
     # one zeroed status word per call: [vote flag, rows to recompute] — the kernels write into it
     status = torch.zeros((2,), dtype=torch.int32, device=feature.device)
+    if _certified_vote_applies(feature, feature_bank, num_classes, knn_k, knn_t, mode, exclude):
+        pred, bad_rows, fix = _predict_certified(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t,
+                                                 mode, track, boost, status)
+        return pred, status, bad_rows, fix
     if mode in RESCORED_MODES:
         keys, bad_rows, _, fix = _topk_keys_rescored(feature, feature_bank, knn_k, mode, defer=True,
                                                      track=track, boost=boost, n_bad=status[1:2], exclude=exclude)
@@ -1411,7 +1511,7 @@ def _graph_key(feature, feature_bank, labels, num_classes, knn_k, knn_t, mode):
     return (_graph_boost(feature_bank, mode), feature_bank.data_ptr(), feature_bank._version, tuple(feature_bank.shape), tuple(feature_bank.stride()),
             feature_bank.dtype, feature_bank.device.index, labels.data_ptr(), labels._version,
             tuple(feature.shape), feature.dtype, int(num_classes), int(knn_k),
-            knn_t if isinstance(knn_t, tuple) else float(knn_t), mode)
+            knn_t if isinstance(knn_t, tuple) else float(knn_t), mode, CERTIFIED_VOTE["enabled"])
 
 
 def _graph_for(feature, feature_bank, labels, num_classes, knn_k, knn_t, mode):

@@ -410,6 +410,44 @@ int b200knn_rescore(const void* q, int q_dtype, int64_t q_ld, const float* rows_
   return e == cudaSuccess ? B200KNN_OK : fail_cuda("rescore", e);
 }
 
+int b200knn_rescore_vote(const float* q, int64_t q_ld, const float* rows, int64_t N, int dim,
+                         const uint64_t* cand_keys, int64_t B, int k_in, int k, float err_coef, float err_abs,
+                         float max_abs, const float* bank_max_norm, const int64_t* labels, int64_t n_labels,
+                         int C, double t, uint64_t* band_keys, int32_t* band_info, int64_t* pred,
+                         int32_t* uncertified, int32_t* status, void* workspace, size_t workspace_bytes,
+                         void* stream) {
+  if (!q || !rows || !cand_keys || !bank_max_norm || !labels || !band_keys || !band_info || !pred ||
+      !uncertified || !status || !workspace)
+    return fail(B200KNN_E_ARG, "rescore_vote: null pointer");
+  if (B < 0 || dim <= 0 || k <= 0 || k_in < k || k_in > 1024 || int64_t(k_in) >= N)
+    return fail(B200KNN_E_ARG, "rescore_vote: bad shape (need 0 < k <= k_in <= 1024, k_in < N)");
+  if (C < 1 || C > B200KNN_RESCORE_VOTE_MAX_CLASSES || !(t != 0.0))
+    return fail(B200KNN_E_ARG, "rescore_vote: need 1 <= C <= 256 and t != 0");
+  if (reinterpret_cast<uintptr_t>(rows) % 16 != 0) return fail(B200KNN_E_ARG, "rescore_vote: rows must be 16-byte aligned");
+  if (workspace_bytes < b200knn::rescore_workspace_bytes(B, k_in))
+    return fail(B200KNN_E_WORKSPACE, "rescore_vote: workspace too small");
+  b200knn::RescoreParams p = {};
+  p.q = q;
+  p.q_dtype = B200KNN_F32;
+  p.q_ld = q_ld;
+  p.rows_a = rows;
+  p.dim = dim;
+  p.dim_pad = (dim + 63) / 64 * 64;
+  p.cand = cand_keys;
+  p.B = B;
+  p.k_in = k_in;
+  p.k_out = k;
+  p.err_coef = err_coef;
+  p.err_abs = err_abs;
+  p.max_abs = max_abs;
+  p.bank_max_norm = bank_max_norm;
+  p.uncertified = uncertified;
+  p.n_uncertified = status + 1;
+  cudaError_t e = b200knn::launch_rescore_vote(p, band_keys, band_info, labels, n_labels, C, t, pred, status,
+                                               workspace, static_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? B200KNN_OK : fail_cuda("rescore_vote", e);
+}
+
 int b200knn_certify(const void* q, int q_dtype, int64_t q_ld, int dim, const uint64_t* exact_keys, int k,
                     const uint64_t* approx_keys, int k_in, int64_t B, int all_rows, float err_coef,
                     float err_abs, float max_abs, const float* bank_max_norm, int32_t* uncertified,

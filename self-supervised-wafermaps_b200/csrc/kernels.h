@@ -109,6 +109,12 @@ struct RescoreParams {
 cudaError_t launch_rescore(const RescoreParams& p, void* workspace, size_t workspace_bytes,
                            cudaStream_t stream);
 size_t rescore_workspace_bytes(int64_t B, int k_in);
+// knn_predict's certified class vote (band compaction, dot kernel over the band, rescore_vote_kernel):
+// p.cand = approximate candidates (B, k_in), p.k_out = k, p.uncertified / p.n_uncertified = rows it
+// leaves to the caller; band (B, k_in) and info (B, 4) are outputs, workspace rescore_workspace_bytes
+cudaError_t launch_rescore_vote(const RescoreParams& p, uint64_t* band, int32_t* info, const int64_t* labels,
+                                int64_t n_labels, int C, double t, int64_t* pred, int32_t* status,
+                                void* workspace, cudaStream_t stream);
 // the certificate alone: p.out = merged exact keys (read), p.cand = merged approximate candidates
 cudaError_t launch_certify(const RescoreParams& p, cudaStream_t stream);
 // split (n, k) key lists by owning shard: out (G, n, k), each shard's keys compacted to the front

@@ -572,6 +572,179 @@ int dot_stages() {
   return v;
 }
 
+// ------------------------------------------------------------------ certified class vote (DESIGN §4.1c)
+// knn_predict needs the class ranking, not the neighbour keys.  Per query (warp), with the
+// approximate candidates a_1 >= ... >= a_m (m = k_in) and the row's certificate bound E:
+//   S    = {i <= k : a_i > a_{k+1} + 2E}  (p = |S|): certainly in the exact top k (a_{k+1} := a_m
+//          when k = m; every row outside the list has s <= a_m + E);
+//   band = c_{p+1} .. c_r,  r = #{i : a_i + E >= a_k - E}: the only candidates re-scored.
+// band_kernel writes the band front-filled (zero tail) into `band` (B, k_in), the list format the
+// dot kernel reads, and info[b] = (p, r, E bits, 0); p = -1 marks a row it cannot serve (starved
+// list, operand range, non-finite E), whose band is empty.
+__global__ void __launch_bounds__(128)
+    band_kernel(RescoreParams p, uint64_t* __restrict__ band, int4* __restrict__ info) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int64_t b = int64_t(blockIdx.x) * 4 + warp;
+  if (b >= p.B) return;
+  const uint64_t* cand = p.cand + b * p.k_in;
+  const float* qrow = static_cast<const float*>(p.q) + b * p.q_ld;
+  float qq = 0.0f;  // the select kernel's ||q||, so that E is the certificate's E
+  for (int d = lane; d < p.dim; d += 32) qq = fmaf(qrow[d], qrow[d], qq);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) qq += __shfl_xor_sync(kFull, qq, o);
+  const float qn = sqrtf(qq) * 1.001f, m = *p.bank_max_norm;
+  const float e = p.err_coef * qn * m + p.err_abs * (qn + m);
+  const bool ok = cand[p.k_in - 1] != 0ull && isfinite(e) &&
+                  !(p.max_abs > 0.0f && !(qn < p.max_abs && m < p.max_abs));
+  int n_s = -1, r = 0;
+  if (ok) {
+    const double E = e;
+    const double ak = key_sim(cand[p.k_out - 1]);
+    const double ak1 = key_sim(cand[p.k_out < p.k_in ? p.k_out : p.k_in - 1]);
+    n_s = 0;
+    for (int j0 = 0; j0 < p.k_in; j0 += 32) {
+      const int j = j0 + lane;
+      const double a = j < p.k_in ? double(key_sim(cand[j])) : -INFINITY;
+      n_s += __popc(__ballot_sync(kFull, j < p.k_out && a > ak1 + 2.0 * E));
+      r += __popc(__ballot_sync(kFull, a + E >= ak - E));
+    }
+  }
+  uint64_t* o = band + b * p.k_in;
+  for (int j = lane; j < p.k_in; j += 32) o[j] = (ok && j < r - n_s) ? cand[n_s + j] : 0ull;
+  if (lane == 0) info[b] = make_int4(n_s, r, __float_as_int(e), 0);
+}
+
+// The exact keys of the band (tmp, from the dot kernel over `band`) -> the class ranking, when it
+// is certified; otherwise uncertified[b] = 1 and *n_uncertified counts the row (pred row unset).
+//  set:     the (k-p)-th exact band key must beat a_{r+1} + E (a_m + E when r = m): then S and the
+//           best k - p of the band are the exact top k (today's certificate, applied to the band);
+//  ranking: S members vote with the interval [exp((a-E)/t), exp((a+E)/t)] (ends swapped for
+//           t < 0), the chosen band members with vote_kernel's exact exp(double(s)/t); intervals
+//           are padded for the fp64 rounding of division, exp and summation (any order), and the
+//           ranking is certified when the intervals of the present classes are pairwise disjoint
+//           and each has a positive, finite lower / upper end.  Absent classes score exactly 0
+//           and follow in class order, as in vote_kernel.  A certified ranking is vote_kernel's
+//           ranking of the exact top k, element for element.
+// Label / index errors of a row whose set is certified go to status[0] as in vote_kernel.
+template <int ITEMS>
+__global__ void __launch_bounds__(128)
+    rescore_vote_kernel(RescoreParams p, const uint64_t* __restrict__ tmp, int n_groups,
+                        const int4* __restrict__ info, const int64_t* __restrict__ labels, int64_t n_labels,
+                        int C, double t, int64_t* __restrict__ pred, int32_t* __restrict__ status) {
+  extern __shared__ __align__(16) unsigned char cv_smem[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  double* lo = reinterpret_cast<double*>(cv_smem) + size_t(warp) * 2 * C;
+  double* hi = lo + C;
+  int* cnt = reinterpret_cast<int*>(reinterpret_cast<double*>(cv_smem) + size_t(4) * 2 * C) + warp * C;
+  const int64_t b = int64_t(blockIdx.x) * 4 + warp;
+  if (b >= p.B) return;
+  const int4 in = info[b];
+  const int n_s = in.x, r = in.y;
+  const float e = __int_as_float(in.z);
+  const int k = p.k_out;
+  const uint64_t* cand = p.cand + b * p.k_in;
+  auto fail = [&]() {
+    if (lane == 0) {
+      p.uncertified[b] = 1;
+      atomicAdd(p.n_uncertified, 1);
+    }
+  };
+  if (n_s < 0) return fail();
+  const int nb = r - n_s, need = k - n_s;
+  uint64_t v[ITEMS];
+  int groups = 0;
+#pragma unroll
+  for (int i = 0; i < ITEMS; ++i) {
+    const int c = i * 32 + lane;
+    const bool has = c < nb;
+    v[i] = has ? tmp[b * n_groups * 32 + c] : 0ull;
+    if (__any_sync(kFull, has)) groups = i + 1;
+  }
+  sort_groups<ITEMS>(v, groups, lane);
+  if (need > 0) {
+    uint64_t kth = 0;
+#pragma unroll
+    for (int i = 0; i < ITEMS; ++i) kth = (i * 32 + lane == need - 1) ? v[i] : kth;
+    kth = __shfl_sync(kFull, kth, (need - 1) & 31);
+    const double bound = double(key_sim(cand[r < p.k_in ? r : p.k_in - 1])) + double(e);
+    if (kth == 0ull || !(double(key_sim(kth)) > bound)) return fail();
+  }
+
+  for (int c = lane; c < C; c += 32) {
+    lo[c] = 0.0;
+    hi[c] = 0.0;
+    cnt[c] = 0;
+  }
+  __syncwarp();
+  auto add = [&](uint64_t key, double wl, double wh) {
+    const int64_t li = key_idx(key) - p.idx_offset;
+    if (li >= 0 && li < n_labels) {
+      const int64_t c = labels[li];
+      if (c >= 0 && c < C) {
+        atomicAdd(&lo[c], wl);
+        atomicAdd(&hi[c], wh);
+        atomicAdd(&cnt[c], 1);
+      } else {
+        atomicExch(status, 1);
+      }
+    } else {
+      atomicExch(status, 2);
+    }
+  };
+  for (int i = lane; i < n_s; i += 32) {
+    const uint64_t key = cand[i];
+    const double a = key_sim(key);
+    const double x1 = (a - double(e)) / t, x2 = (a + double(e)) / t;
+    const double pad = (fabs(x1) + fabs(x2)) * 0x1p-48;  // rounding of a -+ E, of the division
+    add(key, exp(fmin(x1, x2) - pad) * (1.0 - 0x1p-48), exp(fmax(x1, x2) + pad) * (1.0 + 0x1p-48));
+  }
+#pragma unroll
+  for (int i = 0; i < ITEMS; ++i) {
+    if (i * 32 + lane < need) {
+      const double w = exp(double(key_sim(v[i])) / t);  // vote_kernel's weight
+      add(v[i], w, w);
+    }
+  }
+  __syncwarp();
+  const double widen = double(k + 8) * 0x1p-48;  // fp64 sums of <= k positive terms, any order
+  bool good = true;
+  int n_present = 0;
+  for (int c = 0; c < C; ++c) n_present += cnt[c] != 0;
+  for (int c = lane; c < C; c += 32) {
+    if (cnt[c] == 0) continue;
+    const double l = lo[c] * (1.0 - widen), h = hi[c] * (1.0 + widen);
+    if (!(l >= 2.2250738585072014e-308) || !(h < INFINITY)) good = false;
+    for (int o = 0; o < C; ++o) {
+      if (o == c || cnt[o] == 0) continue;
+      if (!(l > hi[o] * (1.0 + widen) || lo[o] * (1.0 - widen) > h)) good = false;
+    }
+  }
+  if (!__all_sync(kFull, good)) return fail();
+  int64_t* out = pred + b * C;
+  for (int c = lane; c < C; c += 32) {
+    int rank = 0;
+    if (cnt[c] != 0) {
+      const double h = hi[c] * (1.0 + widen);
+      for (int o = 0; o < C; ++o) rank += (cnt[o] != 0 && lo[o] * (1.0 - widen) > h) ? 1 : 0;
+    } else {
+      rank = n_present;
+      for (int o = 0; o < c; ++o) rank += cnt[o] == 0 ? 1 : 0;
+    }
+    out[rank] = c;
+  }
+  if (lane == 0) p.uncertified[b] = 0;
+}
+
+template <int ITEMS>
+cudaError_t launch_rescore_vote_t(const RescoreParams& p, const uint64_t* tmp, int n_groups, const int4* info,
+                                  const int64_t* labels, int64_t n_labels, int C, double t, int64_t* pred,
+                                  int32_t* status, cudaStream_t stream) {
+  const size_t smem = size_t(4) * C * (2 * sizeof(double) + sizeof(int));
+  rescore_vote_kernel<ITEMS><<<unsigned((p.B + 3) / 4), 128, smem, stream>>>(p, tmp, n_groups, info, labels,
+                                                                             n_labels, C, t, pred, status);
+  return cudaGetLastError();
+}
+
 template <int CHUNK, int STAGES, int R>
 cudaError_t launch_dot_t(const RescoreParams& p, uint64_t* tmp, cudaStream_t stream) {
   constexpr int kSmem = 232448 - 1024;
@@ -592,6 +765,24 @@ cudaError_t launch_dot_t(const RescoreParams& p, uint64_t* tmp, cudaStream_t str
   kern<<<unsigned(blocks), warps * 32, smem, stream>>>(p, tmp, n_groups, n_units, q_vec16);
   return cudaGetLastError();
 }
+
+// the exact keys of p.cand's candidates into tmp (B, ws_slots(k_in)); the first empty 32-slot unit of
+// a list ends its query
+cudaError_t launch_dot(const RescoreParams& p, uint64_t* tmp, cudaStream_t stream) {
+  const int ch = dot_chunk(), stg = dot_stages();
+  // default: 64 columns x 32 candidates per stage, 11 warps per SM.  Measured at the north-star step
+  // (74.5 GB of candidate rows, power-capped clocks): 128 columns / 6 warps 14.95 ms, 64 columns / 11 warps
+  // 13.96 ms, 3-4 stages with fewer warps 19.6-26.2 ms, two fma chains per lane over 64 candidates x 64
+  // columns (B200KNN_RESCORE_ROWS=2) 23.1 ms: the kernel is bound by the rate of its per-row bulk copies and
+  // by how many warps keep them in flight, not by the dependent-fma latency.
+  // small calls (the reference-shaped B = 64) are latency-bound chains of steps: fewer, larger steps
+  const bool small_call = p.B * int64_t(ws_slots(p.k_in) / 32) < 148 * 12 * 8;
+  if (dot_rows() == 2) return launch_dot_t<64, 2, 2>(p, tmp, stream);
+  if ((ch == 128 || small_call) && stg == 2) return launch_dot_t<128, 2, 1>(p, tmp, stream);
+  if (ch == 128) return launch_dot_t<128, 3, 1>(p, tmp, stream);
+  if (stg == 3) return launch_dot_t<64, 3, 1>(p, tmp, stream);
+  return launch_dot_t<64, 2, 1>(p, tmp, stream);
+}
 }  // namespace
 
 size_t rescore_workspace_bytes(int64_t B, int k_in) { return size_t(B) * size_t(ws_slots(k_in)) * sizeof(uint64_t); }
@@ -606,20 +797,7 @@ cudaError_t launch_rescore(const RescoreParams& p, void* workspace, size_t works
   if (p.n_peers > 0 && !pipelined) return cudaErrorInvalidValue;  // the scatter lives in the pipelined variant
   if (pipelined) {
     uint64_t* tmp = static_cast<uint64_t*>(workspace);
-    cudaError_t e;
-    const int ch = dot_chunk(), stg = dot_stages();
-    // default: 64 columns x 32 candidates per stage, 11 warps per SM.  Measured at the north-star step
-    // (74.5 GB of candidate rows, power-capped clocks): 128 columns / 6 warps 14.95 ms, 64 columns / 11 warps
-    // 13.96 ms, 3-4 stages with fewer warps 19.6-26.2 ms, two fma chains per lane over 64 candidates x 64
-    // columns (B200KNN_RESCORE_ROWS=2) 23.1 ms: the kernel is bound by the rate of its per-row bulk copies and
-    // by how many warps keep them in flight, not by the dependent-fma latency.
-    // small calls (the reference-shaped B = 64) are latency-bound chains of steps: fewer, larger steps
-    const bool small_call = p.B * int64_t(ws_slots(p.k_in) / 32) < 148 * 12 * 8;
-    if (dot_rows() == 2) e = launch_dot_t<64, 2, 2>(p, tmp, stream);
-    else if ((ch == 128 || small_call) && stg == 2) e = launch_dot_t<128, 2, 1>(p, tmp, stream);
-    else if (ch == 128) e = launch_dot_t<128, 3, 1>(p, tmp, stream);
-    else if (stg == 3) e = launch_dot_t<64, 3, 1>(p, tmp, stream);
-    else e = launch_dot_t<64, 2, 1>(p, tmp, stream);
+    const cudaError_t e = launch_dot(p, tmp, stream);
     if (e != cudaSuccess) return e;
     const int g32 = ws_slots(p.k_in) / 32;  // 32-slot groups per query in the workspace (always even)
     if (g32 <= 2) return launch_select_t<2>(p, tmp, g32, stream);
@@ -634,6 +812,28 @@ cudaError_t launch_rescore(const RescoreParams& p, void* workspace, size_t works
   if (items <= 8) return launch_rescore_t<8>(p, stream);
   if (items <= 16) return launch_rescore_t<16>(p, stream);
   if (items <= 32) return launch_rescore_t<32>(p, stream);
+  return cudaErrorInvalidValue;
+}
+
+cudaError_t launch_rescore_vote(const RescoreParams& p, uint64_t* band, int32_t* info, const int64_t* labels,
+                                int64_t n_labels, int C, double t, int64_t* pred, int32_t* status,
+                                void* workspace, cudaStream_t stream) {
+  if (p.B == 0) return cudaSuccess;
+  int4* inf = reinterpret_cast<int4*>(info);
+  band_kernel<<<unsigned((p.B + 3) / 4), 128, 0, stream>>>(p, band, inf);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return e;
+  RescoreParams pb = p;
+  pb.cand = band;
+  uint64_t* tmp = static_cast<uint64_t*>(workspace);
+  e = launch_dot(pb, tmp, stream);
+  if (e != cudaSuccess) return e;
+  const int g32 = ws_slots(p.k_in) / 32;
+  if (g32 <= 2) return launch_rescore_vote_t<2>(p, tmp, g32, inf, labels, n_labels, C, t, pred, status, stream);
+  if (g32 <= 4) return launch_rescore_vote_t<4>(p, tmp, g32, inf, labels, n_labels, C, t, pred, status, stream);
+  if (g32 <= 8) return launch_rescore_vote_t<8>(p, tmp, g32, inf, labels, n_labels, C, t, pred, status, stream);
+  if (g32 <= 16) return launch_rescore_vote_t<16>(p, tmp, g32, inf, labels, n_labels, C, t, pred, status, stream);
+  if (g32 <= 32) return launch_rescore_vote_t<32>(p, tmp, g32, inf, labels, n_labels, C, t, pred, status, stream);
   return cudaErrorInvalidValue;
 }
 
