@@ -309,9 +309,14 @@ int b200knn_key_sim_column(const uint64_t* keys, int64_t B, int k, int j, float*
  *              TMA-pipelined kernel (cp.async.bulk per candidate row) and ranked by a second
  *              one; without it a single block-per-query kernel does both.  Same results.
  * b200knn_row_norm_max writes max_n ||row_n|| (x1.001) to *out_dev.
+ * b200knn_row_f16_residual_max: rows (n, dim_pad) fp32; out_dev[0] = R = max_n ||x_n - f16(x_n)||,
+ *   out_dev[1] = max_n ||f16(x_n)||, f16(x) = rn(sat(x)) as b200knn_prepare_rows makes the fp16
+ *   operand; fp64 accumulation, rounded up (+inf for a bank holding a NaN).  The measured
+ *   residuals of b200knn_rescore_vote's bound.
  */
 int b200knn_row_norm_max(const float* rows_a, const float* rows_b, int64_t n,
                          int dim_pad, float* out_dev, void* stream);
+int b200knn_row_f16_residual_max(const float* rows, int64_t n, int dim_pad, float* out_dev, void* stream);
 int b200knn_rescore(const void* q, int q_dtype, int64_t q_ld, const float* rows_a,
                     const float* rows_b, int64_t N, int dim,
                     const uint64_t* cand_keys, int64_t B, int k_in, int k_out,
@@ -324,7 +329,11 @@ size_t b200knn_rescore_workspace_bytes(int64_t B, int k_in);
 /*
  * b200knn_rescore_vote: knn_predict's class ranking from the approximate candidates cand_keys
  * (B, k_in), k_in < N, re-scoring only the candidates near rank k (fp32 queries, one fp32 row
- * array; DESIGN.md §4.1c).  With E the bound of b200knn_rescore:
+ * array; DESIGN.md §4.1c).  E is the bound of b200knn_rescore when bank_resid is NULL.  With
+ * bank_resid = b200knn_row_f16_residual_max's [R, M~] of an fp16 candidate pass's bank it is
+ *     E = err_coef ||q_b|| M + err_abs (||q_b|| + M)
+ *       + ||f16(q_b)|| R + rho_b M~ + rho_b R + acc_coef ||f16(q_b)|| M~,   rho_b = ||q_b - f16(q_b)||
+ * (the caller then passes err_coef = the exact chain's gamma_D and err_abs = 0).
  *   band_info (B, 4) int32 out: (p, r, bits of E, 0), p = the leading candidates certainly in the
  *             exact top k, candidates p+1..r re-scored; p = -1: the row was not attempted
  *   band_keys (B, k_in) out: those candidates, front-filled, zero tail
@@ -338,6 +347,7 @@ size_t b200knn_rescore_workspace_bytes(int64_t B, int k_in);
 int b200knn_rescore_vote(const float* q, int64_t q_ld, const float* rows, int64_t N, int dim,
                          const uint64_t* cand_keys, int64_t B, int k_in, int k, float err_coef,
                          float err_abs, float max_abs, const float* bank_max_norm,
+                         const float* bank_resid, float acc_coef,
                          const int64_t* labels, int64_t n_labels, int C, double t,
                          uint64_t* band_keys, int32_t* band_info, int64_t* pred,
                          int32_t* uncertified, int32_t* status, void* workspace,

@@ -77,6 +77,7 @@ SIGNATURES = {
     "b200knn_row_sqnorms": (c_int, [c_void_p, c_int, c_int64, c_int, c_int64, c_void_p, c_void_p]),
     "b200knn_confusion": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p]),
     "b200knn_row_norm_max": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
+    "b200knn_row_f16_residual_max": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     "b200knn_rescore": (
         c_int,
         [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_int64, c_int, c_int,
@@ -87,8 +88,8 @@ SIGNATURES = {
     "b200knn_rescore_vote": (
         c_int,
         [c_void_p, c_int64, c_void_p, c_int64, c_int, c_void_p, c_int64, c_int, c_int, ctypes.c_float,
-         ctypes.c_float, ctypes.c_float, c_void_p, c_void_p, c_int64, c_int, c_double, c_void_p, c_void_p,
-         c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p],
+         ctypes.c_float, ctypes.c_float, c_void_p, c_void_p, ctypes.c_float, c_void_p, c_int64, c_int, c_double,
+         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p],
     ),
     "b200knn_route_keys": (c_int, [c_void_p, c_int64, c_int, c_int64, c_int, c_void_p, c_void_p]),
     "b200knn_route_scatter": (
@@ -123,7 +124,7 @@ KERNELS_PER_CALL = {
     "b200knn_prepare_rows": 1, "b200knn_topk": 1, "b200knn_topk_opt": 1,
     "b200knn_merge": 1, "b200knn_decode_keys": 1, "b200knn_drop_self": 1, "b200knn_drop_group": 1, "b200knn_vote": 1, "b200knn_vote_ex": 1, "b200knn_vote_multi": 1,
     "b200knn_key_sim_column": 1, "b200knn_normalize_rows": 1, "b200knn_confusion": 1, "b200knn_row_sqnorms": 1, "b200knn_rescore": 2, "b200knn_rescore_vote": 3, "b200knn_route_keys": 1, "b200knn_certify": 1,
-    "b200knn_row_norm_max": 1, "b200knn_debug_topk_dump": 1, "b200knn_broadcast_f32": 1,
+    "b200knn_row_norm_max": 1, "b200knn_row_f16_residual_max": 1, "b200knn_debug_topk_dump": 1, "b200knn_broadcast_f32": 1,
     "b200knn_route_scatter": 1, "b200knn_rescore_scatter": 2, "b200knn_compact_rows": 1, "b200knn_scatter_rows": 1,
 }
 launch_counter = {"kernels": 0}

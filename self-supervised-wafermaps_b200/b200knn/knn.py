@@ -96,10 +96,18 @@ class _Timed:
 # Unlike round 1's flat 2e-5 this grows with D and holds for same-sign products (the reference's
 # live embeddings are non-negative: timm ResNet-18 pooled post-ReLU, knn.py:322), where truncation
 # errors do not cancel: 6.9e-5 (f16) ... 2.3e-4 (tf32x3) at D = 512.
+#
+# residual_bound — knn_predict's certified vote (b200knn_rescore_vote) replaces op_coef's worst case by
+# the rounding residuals the operands really have (DESIGN §4.1c, §5): per query
+#   E = ||f16(q)|| R + rho M~ + rho R + acc_c D_pad 2^-23 ||f16(q)|| M~ + gamma_D ||q|| M,
+# R = max ||x - f16(x)||, M~ = max ||f16(x)|| over the bank (PreparedRows.f16_residuals), rho =
+# ||q - f16(q)||, gamma_D = D 2^-24 / (1 - D 2^-24) for the exact side's own fma chain.  Real rows use
+# about half of the 2^-11 a rounding may cost, so E halves and fewer candidates are re-scored.  The
+# full re-scoring of the rows the vote leaves, topk_keys and the sharded path keep op_coef.
 ACC_ULP = 2.0 ** -23
 LEVELS = {
     "fp32_f16": dict(cand="f16", margin=40, op_coef=1.001 * 2.0 ** -10, acc_c=1.125,
-                     err_abs=1.01 * 2.0 ** -25, max_abs=6.0e4),
+                     err_abs=1.01 * 2.0 ** -25, max_abs=6.0e4, residual_bound=True),
     "fp32_f16x2": dict(cand="f16x2", margin=40, op_coef=1.001 * (2.0 ** -11 + 2.0 ** -22), acc_c=2.25,
                        err_abs=1.01 * 2.0 ** -25, max_abs=6.0e4),
     "fp32_bf16": dict(cand="bf16", margin=128, op_coef=1.02 * 2.0 ** -7, acc_c=1.125),
@@ -231,12 +239,13 @@ def effective_mode(mode: str, dim: int) -> str:
 class PreparedRows:
     """K-major rows in the layout the tensor-core kernel streams with TMA."""
 
-    __slots__ = ("mode", "n", "dim", "hi", "lo", "_f32", "_max_norm", "_src", "_delegate")
+    __slots__ = ("mode", "n", "dim", "hi", "lo", "_f32", "_max_norm", "_f16_resid", "_src", "_delegate")
 
     def __init__(self, mode: str, n: int, dim: int, hi: torch.Tensor, lo: Optional[torch.Tensor]):
         self.mode, self.n, self.dim, self.hi, self.lo = mode, n, dim, hi, lo
         self._f32 = None       # (n, dim_pad) fp32 shadow rows for the exact re-scoring (bf16 candidates)
         self._max_norm = None  # device scalar: max row norm (certificate)
+        self._f16_resid = None  # device [R, M~]: fp16 residual statistics (certified vote)
         self._src = None       # (tensor, vectors_are_columns) to build the shadow lazily
         self._delegate = None  # another preparation of the same bank that owns the shadow rows / norm
 
@@ -265,6 +274,23 @@ class PreparedRows:
                                                             out.data_ptr(), _stream()), "row_norm_max")
             self._max_norm = out
         return self._max_norm
+
+    def f16_residuals(self) -> torch.Tensor:
+        """Device float32[2]: max ||x - f16(x)|| and max ||f16(x)|| over the rows, f16 the rounding of
+        the fp16 candidate pass.  Computed once and kept as long as the preparation: captured call
+        graphs read it by pointer."""
+        if self._delegate is not None:
+            return self._delegate.f16_residuals()
+        if self._f16_resid is None:
+            a, b = self.rescore_rows()
+            if b is not None:
+                raise RuntimeError("f16_residuals needs one fp32 row array")
+            out = torch.zeros((2,), dtype=torch.float32, device=a.device)
+            with torch.cuda.device(a.device):
+                _lib.check(_lib.load().b200knn_row_f16_residual_max(a.data_ptr(), self.n, a.shape[1], out.data_ptr(),
+                                                                    _stream()), "row_f16_residual_max")
+            self._f16_resid = out
+        return self._f16_resid
 
 
 # (D,N) bank views backed by zero-padded (N, D_pad) fp32 rows (b200knn.bank.FeatureBank)
@@ -1384,6 +1410,15 @@ def _predict_certified(feature, feature_bank, feature_labels, num_classes, knn_k
     pb = bank_cache.get(feature_bank, cfg["cand"])
     rows, _ = pb.rescore_rows()
     max_norm = pb.max_norm()
+    if cfg.get("residual_bound"):
+        resid = pb.f16_residuals()
+        u = D * 2.0 ** -24
+        err_coef, err_abs = u / (1.0 - u), 0.0
+        acc_coef = 1.01 * cfg["acc_c"] * padded_dim(D) * ACC_ULP
+    else:
+        resid = None
+        err_coef, err_abs = cfg["err_coef"], cfg.get("err_abs", 0.0) * math.sqrt(padded_dim(D))
+        acc_coef = 0.0
     q = feature if feature.dtype == torch.float32 else feature.float()
     if q.stride(1) != 1:
         q = q.contiguous()
@@ -1397,9 +1432,8 @@ def _predict_certified(feature, feature_bank, feature_labels, num_classes, knn_k
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
         with _Timed("rescore"):
             rc = lib.b200knn_rescore_vote(q.data_ptr(), q.stride(0), rows.data_ptr(), N, D, cand.data_ptr(), B, k_in, k,
-                                          float(cfg["err_coef"]),
-                                          float(cfg.get("err_abs", 0.0)) * math.sqrt(padded_dim(D)),
-                                          float(cfg.get("max_abs", 0.0)), max_norm.data_ptr(), labels.data_ptr(),
+                                          float(err_coef), float(err_abs), float(cfg.get("max_abs", 0.0)),
+                                          max_norm.data_ptr(), _ptr(resid), float(acc_coef), labels.data_ptr(),
                                           labels.numel(), C, float(knn_t), band.data_ptr(), info.data_ptr(),
                                           pred.data_ptr(), flags.data_ptr(), status.data_ptr(), ws.data_ptr(),
                                           ws_bytes, _stream())

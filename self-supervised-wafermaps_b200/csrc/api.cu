@@ -375,6 +375,12 @@ int b200knn_row_norm_max(const float* rows_a, const float* rows_b, int64_t n, in
   return e == cudaSuccess ? B200KNN_OK : fail_cuda("row_norm_max", e);
 }
 
+int b200knn_row_f16_residual_max(const float* rows, int64_t n, int dim_pad, float* out_dev, void* stream) {
+  if (!rows || !out_dev || n < 0 || dim_pad <= 0) return fail(B200KNN_E_ARG, "row_f16_residual_max: bad argument");
+  cudaError_t e = b200knn::launch_row_f16_residual_max(rows, n, dim_pad, out_dev, static_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? B200KNN_OK : fail_cuda("row_f16_residual_max", e);
+}
+
 int b200knn_rescore(const void* q, int q_dtype, int64_t q_ld, const float* rows_a, const float* rows_b,
                     int64_t N, int dim, const uint64_t* cand_keys, int64_t B, int k_in, int k_out,
                     int64_t idx_offset, float err_coef, float err_abs, float max_abs,
@@ -412,7 +418,8 @@ int b200knn_rescore(const void* q, int q_dtype, int64_t q_ld, const float* rows_
 
 int b200knn_rescore_vote(const float* q, int64_t q_ld, const float* rows, int64_t N, int dim,
                          const uint64_t* cand_keys, int64_t B, int k_in, int k, float err_coef, float err_abs,
-                         float max_abs, const float* bank_max_norm, const int64_t* labels, int64_t n_labels,
+                         float max_abs, const float* bank_max_norm, const float* bank_resid, float acc_coef,
+                         const int64_t* labels, int64_t n_labels,
                          int C, double t, uint64_t* band_keys, int32_t* band_info, int64_t* pred,
                          int32_t* uncertified, int32_t* status, void* workspace, size_t workspace_bytes,
                          void* stream) {
@@ -441,6 +448,8 @@ int b200knn_rescore_vote(const float* q, int64_t q_ld, const float* rows, int64_
   p.err_abs = err_abs;
   p.max_abs = max_abs;
   p.bank_max_norm = bank_max_norm;
+  p.bank_resid = bank_resid;
+  p.acc_coef = acc_coef;
   p.uncertified = uncertified;
   p.n_uncertified = status + 1;
   cudaError_t e = b200knn::launch_rescore_vote(p, band_keys, band_info, labels, n_labels, C, t, pred, status,

@@ -8,6 +8,7 @@
 // knn_predict (call site: src/ssl_wafermap/models/knn.py:91-98).
 #pragma once
 #include <cstdint>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
 namespace b200knn {
@@ -32,6 +33,13 @@ __device__ __forceinline__ float key_sim(uint64_t key) {
 }
 __device__ __forceinline__ int64_t key_idx(uint64_t key) {
   return key == 0 ? int64_t(-1) : int64_t(0xFFFFFFFFu - uint32_t(key & 0xFFFFFFFFu));
+}
+
+// The fp16 operand of x in the F16 / F16X2 modes: rn(sat(x)), sat clamping to +-65504 so that no
+// inf/NaN ever enters the contraction.  The bank and query preparation and the certificate's
+// residual norms (rescore.cu) all round through this one function.
+__device__ __forceinline__ __half f16_operand(float x) {
+  return __float2half_rn(fminf(fmaxf(x, -65504.0f), 65504.0f));
 }
 
 // Bitonic sort, descending, of ITEMS*32 keys held as v[r] on lane l <-> element

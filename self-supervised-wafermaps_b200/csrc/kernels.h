@@ -95,6 +95,9 @@ struct RescoreParams {
   float err_abs;
   float max_abs;               // > 0: rows with ||q|| or M >= max_abs are uncertified (operand range)
   const float* bank_max_norm;  // device scalar
+  // band_kernel only: the fp16 operand bound of rescore.cu's cert_bound; nullptr: none
+  const float* bank_resid = nullptr;  // device [R, M~]: max ||x - f16(x)||, max ||f16(x)|| over the bank
+  float acc_coef = 0.0f;              // tensor-core accumulation term, relative to ||f16(q)|| M~
   uint64_t* out;               // (B, k_out)
   int32_t* uncertified;        // (B,)
   int32_t* n_uncertified;      // device counter (caller zeroes)
@@ -132,6 +135,8 @@ cudaError_t launch_scatter_rows(int64_t* dst, int64_t dst_ld, const int64_t* src
                                 cudaStream_t stream);
 cudaError_t launch_row_norm_max(const float* a, const float* b, int64_t n, int dim_pad, float* out,
                                 cudaStream_t stream);
+// out[0] = max_n ||x_n - f16(x_n)||, out[1] = max_n ||f16(x_n)|| (fp64, rounded up)
+cudaError_t launch_row_f16_residual_max(const float* a, int64_t n, int dim_pad, float* out, cudaStream_t stream);
 
 // tensor-core path (tc_topk.cu)
 struct TcParams {

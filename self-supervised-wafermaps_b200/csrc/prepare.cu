@@ -21,6 +21,7 @@
 #include <cuda_fp16.h>
 
 #include "../../include/b200knn.h"
+#include "common.cuh"
 #include "kernels.h"
 
 namespace b200knn {
@@ -42,11 +43,9 @@ __device__ __forceinline__ void emit(int mode, float x, void* hi, void* lo, int6
     static_cast<__nv_bfloat16*>(hi)[o] = h;
     static_cast<__nv_bfloat16*>(lo)[o] = __float2bfloat16_rn(x - __bfloat162float(h));
   } else if (mode == B200KNN_MODE_F16X2 || mode == B200KNN_MODE_F16) {
-    const float sx = fminf(fmaxf(x, -65504.0f), 65504.0f);
-    const __half h = __float2half_rn(sx);
+    const __half h = f16_operand(x);
     static_cast<__half*>(hi)[o] = h;
-    if (lo != nullptr)
-      static_cast<__half*>(lo)[o] = __float2half_rn(fminf(fmaxf(x - __half2float(h), -65504.0f), 65504.0f));
+    if (lo != nullptr) static_cast<__half*>(lo)[o] = f16_operand(x - __half2float(h));
   } else {
     uint32_t u;
     asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(u) : "f"(x));

@@ -42,6 +42,25 @@
 namespace b200knn {
 namespace {
 
+// The bound E >= |approx - exact| of one query against every bank row (DESIGN §4.1c, §5).
+// qn = ||q||, qtn = ||f16(q)||, rho = ||q - f16(q)||, each rounded up / inflated by the caller.
+//   E = err_coef ||q|| M + err_abs (||q|| + M)              the level's model (b200knn.knn LEVELS), M = *bank_max_norm
+//     + qtn R + rho M~ + rho R + acc_coef qtn M~            with the bank's measured fp16 residuals [R, M~] (bank_resid)
+//     + dim_pad 2^-149                                       underflow of the exact fma chain
+// A level without residuals (bank_resid == nullptr) gets its worst-case model alone; with them the
+// caller passes err_coef = gamma_D (the exact chain's own rounding) and err_abs = 0.  The last term
+// changes no E above 2^-100 and covers the fp32 evaluation of a tiny E; the inflated norms cover
+// it above.
+__device__ __forceinline__ float cert_bound(const RescoreParams& p, float qn, float qtn, float rho) {
+  const float m = *p.bank_max_norm;
+  float e = p.err_coef * qn * m + p.err_abs * (qn + m);
+  if (p.bank_resid != nullptr) {
+    const float r = p.bank_resid[0], mt = p.bank_resid[1];
+    e += qtn * r + rho * mt + rho * r + p.acc_coef * qtn * mt;
+  }
+  return e + float(p.dim_pad) * 0x1p-149f;
+}
+
 // Certificate of one row (see the header): kth = exact key at rank k_out, last = approximate key
 // at rank k_in, qn = ||q|| (inflated by the caller for its rounding).
 __device__ __forceinline__ int certified(const RescoreParams& p, uint64_t kth, uint64_t last, float qn) {
@@ -52,7 +71,7 @@ __device__ __forceinline__ int certified(const RescoreParams& p, uint64_t kth, u
   }
   const float m = *p.bank_max_norm;
   if (p.max_abs > 0.0f && !(qn < p.max_abs && m < p.max_abs)) return 0;  // operand range of the candidate pass
-  const float e = p.err_coef * qn * m + p.err_abs * (qn + m);
+  const float e = cert_bound(p, qn, 0.0f, 0.0f);
   return (kth != 0) && (key_sim(kth) > key_sim(last) + e);
 }
 
@@ -527,6 +546,39 @@ __global__ void __launch_bounds__(256)
   if (lane == 0) atomicMax(reinterpret_cast<int*>(out), __float_as_int(sqrtf(best) * 1.001f));
 }
 
+// out[0] = max over rows of ||x - f16(x)||, out[1] = of ||f16(x)|| (f16_operand, the bank's fp16
+// operand).  fp64 sums of exact squares, padded for their rounding and rounded up to fp32; a row
+// holding a NaN makes both +inf, which refuses the bound.  Non-negative floats order as ints.
+__global__ void __launch_bounds__(256)
+    row_f16_residual_max_kernel(const float* __restrict__ a, int64_t n, int dim_pad, float* __restrict__ out) {
+  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  const int n_warps = (gridDim.x * blockDim.x) >> 5;
+  double best_r = 0.0, best_t = 0.0;
+  for (int64_t row = warp; row < n; row += n_warps) {
+    double rr = 0.0, tt = 0.0;
+    for (int d = lane; d < dim_pad; d += 32) {
+      const float x = a[row * dim_pad + d];
+      const double t = __half2float(f16_operand(x)), r = double(x) - t;
+      rr = fma(r, r, rr);
+      tt = fma(t, t, tt);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      rr += __shfl_xor_sync(kFull, rr, o);
+      tt += __shfl_xor_sync(kFull, tt, o);
+    }
+    const bool bad = isnan(rr) || isnan(tt);
+    best_r = bad ? INFINITY : fmax(best_r, rr);
+    best_t = bad ? INFINITY : fmax(best_t, tt);
+  }
+  if (lane == 0) {
+    const double pad = 1.0 + 0x1p-36;  // > 1 + dim_pad 2^-53 for dim_pad < 2^17
+    atomicMax(reinterpret_cast<int*>(out), __float_as_int(__double2float_ru(__dsqrt_ru(__dmul_ru(best_r, pad)))));
+    atomicMax(reinterpret_cast<int*>(out + 1),
+              __float_as_int(__double2float_ru(__dsqrt_ru(__dmul_ru(best_t, pad)))));
+  }
+}
+
 template <int ITEMS>
 cudaError_t launch_rescore_t(const RescoreParams& p, cudaStream_t stream) {
   const size_t smem = sizeof(float) * (size_t(p.dim_pad) + kWarps * 32 * kTileLd) +
@@ -588,12 +640,33 @@ __global__ void __launch_bounds__(128)
   if (b >= p.B) return;
   const uint64_t* cand = p.cand + b * p.k_in;
   const float* qrow = static_cast<const float*>(p.q) + b * p.q_ld;
+  const bool resid = p.bank_resid != nullptr;
   float qq = 0.0f;  // the select kernel's ||q||, so that E is the certificate's E
-  for (int d = lane; d < p.dim; d += 32) qq = fmaf(qrow[d], qrow[d], qq);
+  // ||f16(q)||^2 and ||q - f16(q)||^2 in fp64: the squares are exact and cannot underflow
+  double tt = 0.0, rr = 0.0;
+  for (int d = lane; d < p.dim; d += 32) {
+    const float v = qrow[d];
+    qq = fmaf(v, v, qq);
+    if (resid) {
+      const double t = __half2float(f16_operand(v)), r = double(v) - t;  // exact below the max_abs range
+      tt = fma(t, t, tt);
+      rr = fma(r, r, rr);
+    }
+  }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) qq += __shfl_xor_sync(kFull, qq, o);
+  float qtn = 0.0f, rho = 0.0f;
+  if (resid) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      tt += __shfl_xor_sync(kFull, tt, o);
+      rr += __shfl_xor_sync(kFull, rr, o);
+    }
+    qtn = __double2float_ru(sqrt(tt)) * 1.001f;
+    rho = __double2float_ru(sqrt(rr)) * 1.001f;
+  }
   const float qn = sqrtf(qq) * 1.001f, m = *p.bank_max_norm;
-  const float e = p.err_coef * qn * m + p.err_abs * (qn + m);
+  const float e = cert_bound(p, qn, qtn, rho);
   const bool ok = cand[p.k_in - 1] != 0ull && isfinite(e) &&
                   !(p.max_abs > 0.0f && !(qn < p.max_abs && m < p.max_abs));
   int n_s = -1, r = 0;
@@ -857,6 +930,15 @@ cudaError_t launch_row_norm_max(const float* a, const float* b, int64_t n, int d
   if (n == 0) return cudaSuccess;
   const int blocks = int(n < 148 * 8 * 8 ? (n + 7) / 8 : 148 * 8);
   row_norm_max_kernel<<<blocks, 256, 0, stream>>>(a, b, n, dim_pad, out);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_row_f16_residual_max(const float* a, int64_t n, int dim_pad, float* out, cudaStream_t stream) {
+  cudaError_t e = cudaMemsetAsync(out, 0, 2 * sizeof(float), stream);
+  if (e != cudaSuccess) return e;
+  if (n == 0) return cudaSuccess;
+  const int blocks = int(n < 148 * 8 * 8 ? (n + 7) / 8 : 148 * 8);
+  row_f16_residual_max_kernel<<<blocks, 256, 0, stream>>>(a, n, dim_pad, out);
   return cudaGetLastError();
 }
 
