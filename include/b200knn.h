@@ -281,6 +281,23 @@ int b200knn_vote_multi(const uint64_t* keys, const int64_t* labels, int64_t B, i
                        const double* ts, int n_t, int64_t* pred, int64_t pred_ld, int status_col,
                        int32_t* err_flag, void* stream);
 
+/*
+ * Multi-label vote over the same grid: bank row n carries the label set label_bits[n - label_offset]
+ * (bit l set: label l, 1 <= L <= 64; a row with no bit set carries no label).  For row b, k = ks[i]
+ * and t = ts[j] (finite, > 0), scores[b*scores_ld + (i*n_t + j)*L + l] = S_l / W, where
+ *   w_r = exp((double(s_r) - double(s_0)) / t)  (s_r: similarity of key r, s_0 of the row's first key),
+ *   W = sum_{r<k} w_r,  S_l = sum_{r<k, bit l of key r's row} w_r,
+ * both fp64 and added in rank order ((w_0 + w_1) + w_2) + ...  Every score lies in [0, 1]; it is
+ * exactly 0 for a label no neighbour carries and exactly 1 for one every neighbour carries; W >= 1,
+ * so no t overflows.  Empty keys add nothing; a key whose index is outside the labels adds nothing
+ * and sets *err_flag = 2 (a row without a neighbour scores 0).  ks, n_k and n_t as
+ * b200knn_vote_multi; scores_ld >= n_k*n_t*L.  Any k_max (chunks of 1024 keys).
+ */
+int b200knn_vote_multilabel(const uint64_t* keys, const uint64_t* label_bits, int64_t B, int k_max,
+                            int64_t n_labels, int64_t label_offset, int L, const int* ks, int n_k,
+                            const double* ts, int n_t, double* scores, int64_t scores_ld,
+                            int32_t* err_flag, void* stream);
+
 /* out[b] = similarity of keys[b, j] (-inf for an empty slot): the threshold a (B,r) sample
  * hands to b200knn_topk_opt as tau0 (j = r-1). */
 int b200knn_key_sim_column(const uint64_t* keys, int64_t B, int k, int j, float* out,

@@ -72,6 +72,11 @@ SIGNATURES = {
         [c_void_p, c_void_p, c_int64, c_int, c_int64, c_int64, c_int, ctypes.POINTER(c_int), c_int,
          ctypes.POINTER(c_double), c_int, c_void_p, c_int64, c_int, c_void_p, c_void_p],
     ),
+    "b200knn_vote_multilabel": (
+        c_int,
+        [c_void_p, c_void_p, c_int64, c_int, c_int64, c_int64, c_int, ctypes.POINTER(c_int), c_int,
+         ctypes.POINTER(c_double), c_int, c_void_p, c_int64, c_void_p, c_void_p],
+    ),
     "b200knn_key_sim_column": (c_int, [c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p]),
     "b200knn_normalize_rows": (c_int, [c_void_p, c_int, c_int64, c_int, c_int64, ctypes.c_float, c_void_p, c_void_p]),
     "b200knn_row_sqnorms": (c_int, [c_void_p, c_int, c_int64, c_int, c_int64, c_void_p, c_void_p]),
@@ -123,6 +128,7 @@ _lib = None
 KERNELS_PER_CALL = {
     "b200knn_prepare_rows": 1, "b200knn_topk": 1, "b200knn_topk_opt": 1,
     "b200knn_merge": 1, "b200knn_decode_keys": 1, "b200knn_drop_self": 1, "b200knn_drop_group": 1, "b200knn_vote": 1, "b200knn_vote_ex": 1, "b200knn_vote_multi": 1,
+    "b200knn_vote_multilabel": 1,
     "b200knn_key_sim_column": 1, "b200knn_normalize_rows": 1, "b200knn_confusion": 1, "b200knn_row_sqnorms": 1, "b200knn_rescore": 2, "b200knn_rescore_vote": 3, "b200knn_route_keys": 1, "b200knn_certify": 1,
     "b200knn_row_norm_max": 1, "b200knn_row_f16_residual_max": 1, "b200knn_debug_topk_dump": 1, "b200knn_broadcast_f32": 1,
     "b200knn_route_scatter": 1, "b200knn_rescore_scatter": 2, "b200knn_compact_rows": 1, "b200knn_scatter_rows": 1,

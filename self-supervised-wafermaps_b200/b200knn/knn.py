@@ -1336,6 +1336,79 @@ def vote_multi_packed(keys: torch.Tensor, feature_labels: torch.Tensor, num_clas
     return out
 
 
+MAX_LABELS = 64  # label sets are 64-bit masks (include/b200knn.h b200knn_vote_multilabel)
+
+
+def pack_label_bits(label_matrix: torch.Tensor) -> torch.Tensor:
+    """(N, L) 0/1 label matrix (bool or integer dtype, 1 <= L <= 64) -> (N,) int64 bitmasks, bit l set
+    when row n carries label l.  Bit 63 is the sign bit: the int64 view of the uint64 mask the vote
+    kernel reads."""
+    _check_label_matrix(label_matrix)
+    return _label_bits(label_matrix)
+
+
+def _label_bits(m: torch.Tensor) -> torch.Tensor:
+    weight = torch.tensor([1 << b if b < 63 else -(1 << 63) for b in range(m.shape[1])], dtype=torch.int64,
+                          device=m.device)
+    # distinct powers of two: the sum is the bitwise or, and bit 63's -2^63 cannot overflow it
+    return (m.to(torch.int64) * weight).sum(1)
+
+
+def _check_label_matrix(m: torch.Tensor, n_rows: Optional[int] = None) -> None:
+    if not isinstance(m, torch.Tensor):
+        raise TypeError(f"label_matrix must be a torch.Tensor, got {type(m).__name__}")
+    if m.dim() != 2:
+        raise ValueError(f"label_matrix must be (N, L), got shape {tuple(m.shape)}")
+    if m.dtype.is_floating_point or m.dtype.is_complex:
+        raise ValueError(f"label_matrix must be bool or integer 0/1 entries, got {m.dtype}")
+    if n_rows is not None and m.shape[0] != n_rows:
+        raise ValueError(f"label_matrix has {m.shape[0]} rows for a bank of {n_rows}")
+    if not 1 <= m.shape[1] <= MAX_LABELS:
+        raise ValueError(f"label_matrix must have 1 to {MAX_LABELS} labels, got {m.shape[1]}")
+    if m.dtype != torch.bool and bool(((m != 0) & (m != 1)).any()):
+        raise ValueError("label_matrix entries must be 0 or 1")
+
+
+class _MultiLabelVote:
+    """knn_t of a multi-label call: per-label scores over the (ks, ts) grid, ks ascending, from
+    (N,) label bitmasks (``vote_multilabel``).  Not a tuple: a tuple knn_t is the class-ranking grid."""
+
+    __slots__ = ("ks", "ts")
+
+    def __init__(self, ks, ts):
+        self.ks, self.ts = tuple(ks), tuple(ts)
+
+
+def vote_multilabel(keys: torch.Tensor, label_bits: torch.Tensor, n_labels: int, knn_ks, knn_ts,
+                    check_labels: bool = True, flag: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """keys (B, k_max) sorted + label_bits (N,) int64 (``pack_label_bits``) -> (B, n_k*n_t*L) fp64: block
+    (i, j) of a row holds, for every label l < n_labels, S_l / W over the row's first knn_ks[i] keys at
+    knn_t = knn_ts[j] (b200knn_vote_multilabel, include/b200knn.h).  knn_ks strictly increasing with
+    knn_ks[-1] == k_max; knn_ts finite and > 0.  flag: as ``vote_multi`` (2: neighbour index outside
+    the labels)."""
+    _require_cuda("label_bits", label_bits)
+    if label_bits.dtype != torch.int64:
+        raise TypeError(f"label_bits must be int64 bitmasks, got {label_bits.dtype}")
+    B, k = keys.shape
+    L = int(n_labels)
+    scores = torch.empty((B, len(knn_ks) * len(knn_ts) * L), dtype=torch.float64, device=keys.device)
+    if B:
+        if flag is None:
+            flag = torch.zeros((1,), dtype=torch.int32, device=keys.device)
+        bits = label_bits.contiguous().view(-1)
+        ks = (ctypes.c_int * len(knn_ks))(*[int(x) for x in knn_ks])
+        ts = (ctypes.c_double * len(knn_ts))(*[float(x) for x in knn_ts])
+        keys = keys.contiguous()
+        with torch.cuda.device(keys.device):
+            _lib.check(_lib.load().b200knn_vote_multilabel(keys.data_ptr(), bits.data_ptr(), B, k, bits.numel(), 0,
+                                                           L, ks, len(knn_ks), ts, len(knn_ts), scores.data_ptr(),
+                                                           scores.stride(0), flag.data_ptr(), _stream()),
+                       "vote_multilabel")
+        if check_labels:
+            _raise_vote_flag(int(flag.item()), L)
+    return scores
+
+
 def _raise_vote_flag(f: int, C: int) -> None:
     if f == 1:
         # the reference raises here from zeros(...).scatter(...) (lightly knn_predict)
@@ -1370,7 +1443,10 @@ def check_grid(knn_ks, knn_ts):
 def _vote_step(keys, feature_labels, num_classes, knn_t, flag):
     """The vote of a call, label status into the device int32[1] `flag`: knn_t a temperature ->
     (B, C) rankings (``vote``); knn_t a (ks, ts) grid, ks ascending and ks[-1] == keys.shape[1] ->
-    (B, n_k*n_t*C) rankings (``vote_multi``)."""
+    (B, n_k*n_t*C) rankings (``vote_multi``); knn_t a ``_MultiLabelVote`` (feature_labels the (N,)
+    bitmasks, num_classes the label count L) -> (B, n_k*n_t*L) fp64 scores (``vote_multilabel``)."""
+    if isinstance(knn_t, _MultiLabelVote):
+        return vote_multilabel(keys, feature_labels, num_classes, knn_t.ks, knn_t.ts, check_labels=False, flag=flag)
     if isinstance(knn_t, tuple):
         return vote_multi(keys, feature_labels, num_classes, knn_t[0], knn_t[1], check_labels=False, flag=flag)
     return vote(keys, feature_labels, num_classes, knn_t, check_labels=False, return_flag=True, flag=flag)[0]
@@ -1388,7 +1464,7 @@ def _certified_vote_applies(feature, feature_bank, num_classes, knn_k, knn_t, mo
     """Whether a knn_predict call takes the certified vote: a rescored mode with one fp32 row array,
     a single temperature, no group exclusion, and k_in < N at every margin (k_in <= max(k, MAX_K))."""
     return (CERTIFIED_VOTE["enabled"] and mode in RESCORED_MODES and mode != "fp32_tf32"
-            and not isinstance(knn_t, tuple) and float(knn_t) != 0.0 and exclude is None
+            and not isinstance(knn_t, (tuple, _MultiLabelVote)) and float(knn_t) != 0.0 and exclude is None
             and int(num_classes) <= CERTIFIED_VOTE_MAX_CLASSES
             and feature_bank.shape[1] > max(int(knn_k), MAX_K))
 
@@ -1606,6 +1682,8 @@ def knn_predict(feature: torch.Tensor, feature_bank: torch.Tensor, feature_label
 
 def _vote_checked(keys, feature_labels, num_classes, knn_t):
     """``_vote_step`` raising the label errors itself (one host synchronisation)."""
+    if isinstance(knn_t, _MultiLabelVote):
+        return vote_multilabel(keys, feature_labels, num_classes, knn_t.ks, knn_t.ts)
     if isinstance(knn_t, tuple):
         return vote_multi(keys, feature_labels, num_classes, knn_t[0], knn_t[1])
     return vote(keys, feature_labels, num_classes, knn_t)
@@ -1620,7 +1698,9 @@ def _predict(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t, m
         _check_feature_bank(feature, feature_bank)
         raise RuntimeError(
             f"feature_labels has {feature_labels.numel()} entries for a bank of {feature_bank.shape[1]}")
-    check_vote_classes(num_classes, knn_k, grid=isinstance(knn_t, tuple))
+    multilabel = isinstance(knn_t, _MultiLabelVote)  # per-label scores: no class-count bound, no graph
+    if not multilabel:
+        check_vote_classes(num_classes, knn_k, grid=isinstance(knn_t, tuple))
     if mode == "exact" or int(knn_k) > MAX_K:
         return _vote_checked(topk_keys(feature, feature_bank, knn_k, mode, exclude=exclude), feature_labels,
                              num_classes, knn_t)
@@ -1634,7 +1714,7 @@ def _predict(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t, m
     # Tensor-core modes: everything is enqueued first and ONE host synchronisation reads the
     # status word (vote flag; rows to recompute: rows a sampled threshold starved, or rows whose
     # exact re-scoring could not be certified).
-    if GRAPHS["enabled"] and exclude is None and feature.shape[0] <= GRAPH_MAX_BATCH \
+    if GRAPHS["enabled"] and exclude is None and not multilabel and feature.shape[0] <= GRAPH_MAX_BATCH \
             and feature_labels.dtype == torch.int64 \
             and feature_labels.is_contiguous() and not torch.cuda.is_current_stream_capturing():
         with torch.cuda.device(feature.device):
@@ -1685,6 +1765,38 @@ def knn_predict_multi(feature: torch.Tensor, feature_bank: torch.Tensor, feature
     parts = [_predict(feature, feature_bank, feature_labels, num_classes, part[-1], (part, tuple(ts)), mode,
                       exclude) for part in searches]
     return grid_view(torch.cat(parts, dim=1) if len(parts) > 1 else parts[0], order, len(ts), num_classes)
+
+
+def knn_predict_multilabel(feature: torch.Tensor, feature_bank: torch.Tensor, label_matrix: torch.Tensor,
+                           knn_ks=(200,), knn_ts=(0.1,)) -> torch.Tensor:
+    """Multi-label kNN scores for every (knn_k, knn_t) of a grid from ONE neighbour search at
+    k_max = max(knn_ks), as ``knn_predict_multi``: (len(knn_ks), len(knn_ts), B, L) float64, where
+    [i, j, b, l] is the exp(sim/t)-weighted share of query b's knn_ks[i] nearest bank rows that carry
+    label l, in [0, 1]:  sum_{r<k, row r has l} w_r / sum_{r<k} w_r,  w_r = exp((s_r - s_0) / t), s_0
+    the nearest similarity; fp64, added in rank order (b200knn_vote_multilabel, include/b200knn.h).
+    A row without labels (a normal wafer) still weighs in W.
+
+    label_matrix: (N, L) 0/1 targets, bool or any integer dtype, 1 <= L <= 64, on the bank's device
+    (the torchmetrics / scikit-learn multi-label format).  The neighbour lists are those of
+    ``knn_predict`` in the default mode; knn_ts must be finite and > 0.  Single-label banks get
+    class probabilities from ``F.one_hot(labels, C)``."""
+    ks, ts, order = check_grid(knn_ks, knn_ts)
+    if not all(t > 0.0 and math.isfinite(t) for t in ts):
+        raise ValueError(f"knn_ts must be finite and > 0 for per-label scores, got {ts}")
+    n_bank = feature_bank.shape[1] if feature_bank.dim() == 2 else None
+    _check_label_matrix(label_matrix, n_bank)
+    if n_bank is not None and max(ks) > n_bank:
+        raise RuntimeError("selected index k out of range")
+    _check_feature_bank(feature, feature_bank)
+    _require_cuda("label_matrix", label_matrix)
+    if label_matrix.device != feature_bank.device:
+        raise RuntimeError("Expected all tensors to be on the same device, but found "
+                           f"{label_matrix.device} and {feature_bank.device}")
+    mode = _default_mode
+    bits, L = _label_bits(label_matrix), label_matrix.shape[1]
+    parts = [_predict(feature, feature_bank, bits, L, part[-1], _MultiLabelVote(part, ts), mode)
+             for part in grid_parts(tuple(ks[i] for i in order), mode)]
+    return grid_view(torch.cat(parts, dim=1) if len(parts) > 1 else parts[0], order, len(ts), L)
 
 
 def grid_parts(ks_ascending: tuple, mode: str) -> list:

@@ -67,3 +67,67 @@ def knn_metrics(pred: torch.Tensor, target: torch.Tensor, num_classes: int) -> D
     """``on_validation_epoch_end`` of the reference (``knn.py:104-129``) for predictions
     ``pred_labels[:, 0]`` and their targets."""
     return metrics_from_counts(confusion_counts(pred, target, num_classes))
+
+
+def multilabel_metrics_from_scores(scores: torch.Tensor, target: torch.Tensor,
+                                   threshold: float = 0.5) -> Dict[str, torch.Tensor]:
+    """Multi-label metrics of per-label scores (Q, L) against 0/1 targets (Q, L), on any device, with
+    no host synchronisation.  A label is predicted when its score is > threshold.
+
+      counts          (L, 4) int64: per label tp, fp, fn, tn
+      f1_macro        mean over labels of 2 tp / (2 tp + fp + fn), 0/0 := 0, labels absent from both
+                      the predictions and the targets left out (metrics_from_counts' convention)
+      f1_micro        2 TP / (2 TP + FP + FN) over all labels, 0/0 := 0
+      subset_accuracy share of rows whose predicted label set equals the target set
+      hamming_loss    share of (row, label) cells predicted wrongly
+      auc             (L,) fp64 ROC AUC per label: the Mann-Whitney statistic with average ranks for
+                      ties; NaN for a label whose targets do not contain both values
+      auc_macro       mean of auc over the labels where it is defined (NaN if there are none)
+    The scalars are 0-dim fp64 tensors."""
+    if scores.dim() != 2 or scores.shape != target.shape:
+        raise RuntimeError(f"scores {tuple(scores.shape)} and target {tuple(target.shape)} must be the same (Q, L)")
+    s = scores.double()
+    pos = target != 0
+    pred = s > threshold
+    tp = (pred & pos).sum(0)
+    fp = (pred & ~pos).sum(0)
+    fn = (~pred & pos).sum(0)
+    tn = (~pred & ~pos).sum(0)
+    counts = torch.stack([tp, fp, fn, tn], dim=1)
+    tp_d, fp_d, fn_d = tp.double(), fp.double(), fn.double()
+    denom = 2 * tp_d + fp_d + fn_d
+    present = denom > 0
+    f1 = torch.where(present, 2 * tp_d / denom.clamp(min=1), torch.zeros_like(tp_d))
+    micro_denom = denom.sum()
+    cells = max(s.numel(), 1)
+    # average ranks (1-based) within each label's column: (#below + #below-or-equal + 1) / 2
+    cols = s.t().contiguous()
+    srt = cols.sort(dim=1).values
+    rank = (torch.searchsorted(srt, cols, right=False) + torch.searchsorted(srt, cols, right=True) + 1).double() / 2
+    n_pos = pos.sum(0).double()
+    n_neg = s.shape[0] - n_pos
+    rank_sum = (rank * pos.t()).sum(1)
+    defined = (n_pos > 0) & (n_neg > 0)
+    auc = torch.where(defined, (rank_sum - n_pos * (n_pos + 1) / 2) / (n_pos * n_neg).clamp(min=1),
+                      torch.full_like(rank_sum, float("nan")))
+    return {
+        "counts": counts,
+        "f1_macro": (f1 * present).sum() / present.sum().clamp(min=1),
+        "f1_micro": torch.where(micro_denom > 0, 2 * tp_d.sum() / micro_denom.clamp(min=1), micro_denom * 0),
+        "subset_accuracy": (pred == pos).all(1).double().sum() / max(s.shape[0], 1),
+        "hamming_loss": (pred != pos).double().sum() / cells,
+        "auc": auc,
+        "auc_macro": auc.nanmean() if auc.numel() else torch.tensor(float("nan"), dtype=torch.float64,
+                                                                      device=s.device),
+    }
+
+
+def knn_multilabel_metrics(scores: torch.Tensor, target: torch.Tensor, threshold: float = 0.5) -> Dict[str, torch.Tensor]:
+    """``multilabel_metrics_from_scores`` on the device for ``knn_predict_multilabel``'s scores [i, j]
+    (Q, L) and the queries' 0/1 label matrix (Q, L), bool or integer (a non-zero entry is a positive):
+    per-label counts, macro / micro F1, subset accuracy, Hamming loss and per-label / macro ROC AUC."""
+    K._require_cuda("scores", scores)
+    K._require_cuda("target", target)
+    if target.dtype.is_floating_point or target.dtype.is_complex:
+        raise RuntimeError(f"target must be bool or integer 0/1 entries, got {target.dtype}")
+    return multilabel_metrics_from_scores(scores, target.to(scores.device), threshold)

@@ -1,6 +1,7 @@
 // api.cu — the extern "C" boundary declared in include/b200knn.h.
 // Argument validation, work planning, workspace carving, kernel dispatch.
 // No device allocation, no implicit synchronisation, no exceptions.
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -621,6 +622,36 @@ int b200knn_vote_multi(const uint64_t* keys, const int64_t* labels, int64_t B, i
   if (e == cudaErrorInvalidValue)
     return fail(B200KNN_E_UNSUPPORTED, "vote_multi: num_classes too large for shared memory");
   return e == cudaSuccess ? B200KNN_OK : fail_cuda("vote_multi", e);
+}
+
+int b200knn_vote_multilabel(const uint64_t* keys, const uint64_t* label_bits, int64_t B, int k_max,
+                            int64_t n_labels, int64_t label_offset, int L, const int* ks, int n_k,
+                            const double* ts, int n_t, double* scores, int64_t scores_ld, int32_t* err_flag,
+                            void* stream) {
+  if (!keys || !label_bits || !scores || !err_flag || !ks || !ts || B < 0 || k_max <= 0 || n_labels <= 0)
+    return fail(B200KNN_E_ARG, "vote_multilabel: bad argument");
+  if (L < 1 || L > 64) return fail(B200KNN_E_ARG, "vote_multilabel: need 1 <= L <= 64 labels");
+  if (n_k < 1 || n_k > b200knn::kVoteMaxKs || n_t < 1 || n_t > b200knn::kVoteMaxTs)
+    return fail(B200KNN_E_ARG, "vote_multilabel: need 1 <= n_k <= 16 and 1 <= n_t <= 8");
+  b200knn::VoteGrid grid{};
+  grid.n_k = n_k;
+  grid.n_t = n_t;
+  for (int i = 0; i < n_k; ++i) {
+    if (ks[i] <= 0 || (i > 0 && ks[i] <= ks[i - 1]))
+      return fail(B200KNN_E_ARG, "vote_multilabel: ks must be positive and strictly increasing");
+    grid.ks[i] = ks[i];
+  }
+  if (ks[n_k - 1] != k_max) return fail(B200KNN_E_ARG, "vote_multilabel: ks[n_k-1] must equal k_max");
+  for (int j = 0; j < n_t; ++j) {
+    if (!(ts[j] > 0.0) || !std::isfinite(ts[j]))
+      return fail(B200KNN_E_ARG, "vote_multilabel: temperature must be finite and > 0");
+    grid.ts[j] = ts[j];
+  }
+  if (scores_ld < int64_t(n_k) * n_t * L)
+    return fail(B200KNN_E_ARG, "vote_multilabel: scores_ld does not describe a (B, >=n_k*n_t*L) output");
+  cudaError_t e = b200knn::launch_vote_multilabel(keys, label_bits, B, n_labels, label_offset, L, grid, scores,
+                                                  scores_ld, err_flag, static_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? B200KNN_OK : fail_cuda("vote_multilabel", e);
 }
 
 int b200knn_vote(const uint64_t* keys, const int64_t* labels, int64_t B, int k, int64_t n_labels,

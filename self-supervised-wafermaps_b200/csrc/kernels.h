@@ -63,6 +63,11 @@ struct VoteGrid {
 cudaError_t launch_vote_multi(const uint64_t* keys, const int64_t* labels, int64_t B, int64_t n_labels,
                               int64_t label_offset, int C, const VoteGrid& grid, int64_t* pred, int64_t pred_ld,
                               int status_col, int32_t* err_flag, cudaStream_t stream);
+// per-label scores (B, >= n_k*n_t*L) fp64 of bank rows carrying label sets label_bits (N,) (bit l:
+// label l, 1 <= L <= 64) for every (ks[i], ts[j]), ts > 0; shared memory 4 warps x 20 min(k_max, kVoteChunk) B
+cudaError_t launch_vote_multilabel(const uint64_t* keys, const uint64_t* label_bits, int64_t B, int64_t n_labels,
+                                   int64_t label_offset, int L, const VoteGrid& grid, double* scores,
+                                   int64_t scores_ld, int32_t* err_flag, cudaStream_t stream);
 // out[b] = similarity of keys[b, j] (-inf for an empty slot)
 cudaError_t launch_key_sim_column(const uint64_t* keys, int64_t B, int k, int j, float* out,
                                   cudaStream_t stream);

@@ -225,6 +225,91 @@ __global__ void __launch_bounds__(kVoteWarps * 32)
   }
 }
 
+// Shared memory per warp of vote_multilabel_kernel for chunks of kc keys: w[kc] f64 | bits[kc] u64 | sim[kc] f32
+__host__ __device__ inline size_t multilabel_warp_bytes(int kc) { return (size_t(kc) * 20 + 7) / 8 * 8; }
+
+// Per-label scores for a grid of (k, t) from one top-k_max list per row, each bank row carrying a
+// set of up to 64 labels as a bitmask: block (i, j) of a row holds, for every label l,
+// S_l / W with w_r = exp((double(s_r) - double(s_0)) / t), W = sum_{r < ks[i]} w_r and S_l the
+// same sum over the ranks whose row carries l.  Both sums run in rank order r = 0, 1, ..., so a
+// score does not depend on the launch geometry, is exactly 0 for a label no neighbour carries and
+// exactly 1 for one every neighbour carries.  The shift by s_0 keeps every exponent <= 0, so W >= 1
+// (w_0 = 1) and no temperature can overflow it.  Per t the warp evaluates the exps across its lanes,
+// then every lane adds them in rank order: lane l owns labels l and l + 32, and every lane keeps
+// the same W, so no lane waits on another.  Empty keys and keys whose index is outside the labels
+// (err_flag = 2) add nothing.  CHUNKED as vote_multi_kernel: the row is walked in chunks once per t.
+template <bool CHUNKED>
+__global__ void __launch_bounds__(kVoteWarps * 32)
+    vote_multilabel_kernel(const uint64_t* __restrict__ keys, const uint64_t* __restrict__ label_bits, int64_t B,
+                           int64_t n_labels, int64_t label_offset, int L, VoteGrid grid,
+                           double* __restrict__ scores, int64_t scores_ld, int32_t* __restrict__ err_flag) {
+  extern __shared__ unsigned char vote_smem[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int k = grid.ks[grid.n_k - 1], n_t = grid.n_t;
+  const int kc = k < kVoteChunk ? k : kVoteChunk;
+  unsigned char* base = vote_smem + size_t(warp) * multilabel_warp_bytes(kc);
+  double* w = reinterpret_cast<double*>(base);
+  uint64_t* bits = reinterpret_cast<uint64_t*>(w + kc);
+  float* sim = reinterpret_cast<float*>(bits + kc);
+
+  const int64_t row = int64_t(blockIdx.x) * kVoteWarps + warp;
+  if (row >= B) return;
+  const uint64_t* rk = keys + row * k;
+  const double s0 = double(key_sim(rk[0]));
+  const float none = __int_as_float(0xff800000);  // -inf: the key adds nothing
+  auto load = [&](int j0, int n) {  // keys [j0, j0 + n) of the row -> bits / sim
+    for (int i = lane; i < n; i += 32) {
+      const uint64_t key = rk[j0 + i];
+      uint64_t b = 0;
+      float s = none;
+      if (key != 0) {
+        const int64_t li = key_idx(key) - label_offset;
+        if (li >= 0 && li < n_labels) {
+          b = label_bits[li];
+          s = key_sim(key);
+        } else {
+          atomicExch(err_flag, 2);
+        }
+      }
+      bits[i] = b;
+      sim[i] = s;
+    }
+  };
+  double* out = scores + row * scores_ld;
+  for (int ti = 0; ti < n_t; ++ti) {
+    const double t = grid.ts[ti];
+    double W = 0.0, a0 = 0.0, a1 = 0.0;  // W, S_lane, S_{lane+32}
+    int s = 0;                           // the next segment ends at ks[s]
+    for (int j0 = 0; j0 < k; j0 += kc) {
+      const int n = k - j0 < kc ? k - j0 : kc;
+      if (CHUNKED || ti == 0) {
+        __syncwarp();  // every lane is done with the previous chunk
+        load(j0, n);
+      }
+      __syncwarp();  // bits / sim written; every lane is done with the previous pass's w
+      for (int i = lane; i < n; i += 32) w[i] = sim[i] == none ? 0.0 : exp((double(sim[i]) - s0) / t);
+      __syncwarp();
+      for (int a = 0; a < n;) {  // the segments of this chunk; a boundary may fall anywhere in it
+        const int e = grid.ks[s] - j0 < n ? grid.ks[s] - j0 : n;
+        for (int i = a; i < e; ++i) {
+          const double wi = w[i];
+          const uint64_t b = bits[i];
+          W += wi;
+          a0 += (b >> lane) & 1 ? wi : 0.0;
+          a1 += (b >> (lane + 32)) & 1 ? wi : 0.0;
+        }
+        a = e;
+        if (j0 + e == grid.ks[s]) {
+          double* o = out + (int64_t(s) * n_t + ti) * L;
+          if (lane < L) o[lane] = W > 0.0 ? a0 / W : 0.0;  // W == 0: the row has no neighbour
+          if (lane + 32 < L) o[lane + 32] = W > 0.0 ? a1 / W : 0.0;
+          ++s;
+        }
+      }
+    }
+  }
+}
+
 // counts[t * C + p] += 1 for every (target t, prediction p): the confusion matrix the
 // reference builds with torchmetrics after each validation epoch
 // (src/ssl_wafermap/models/knn.py:104-129).  Up to kConfusionSmemClasses classes: block-private
@@ -299,6 +384,23 @@ cudaError_t launch_vote_multi(const uint64_t* keys, const int64_t* labels, int64
   const int64_t blocks = (B + kVoteWarps - 1) / kVoteWarps;
   kernel<<<unsigned(blocks), kVoteWarps * 32, smem, stream>>>(
       keys, labels, B, n_labels, label_offset, C, grid, pred, pred_ld, status_col, err_flag);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_vote_multilabel(const uint64_t* keys, const uint64_t* label_bits, int64_t B, int64_t n_labels,
+                                   int64_t label_offset, int L, const VoteGrid& grid, double* scores,
+                                   int64_t scores_ld, int32_t* err_flag, cudaStream_t stream) {
+  if (B == 0) return cudaSuccess;
+  const int k = grid.ks[grid.n_k - 1];
+  const size_t smem = multilabel_warp_bytes(k < kVoteChunk ? k : kVoteChunk) * kVoteWarps;
+  const auto kernel = k > kVoteChunk ? vote_multilabel_kernel<true> : vote_multilabel_kernel<false>;
+  if (smem > 48 * 1024) {
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+    if (e != cudaSuccess) return e;
+  }
+  const int64_t blocks = (B + kVoteWarps - 1) / kVoteWarps;
+  kernel<<<unsigned(blocks), kVoteWarps * 32, smem, stream>>>(keys, label_bits, B, n_labels, label_offset, L,
+                                                               grid, scores, scores_ld, err_flag);
   return cudaGetLastError();
 }
 
