@@ -233,6 +233,38 @@ int b200knn_drop_group(const uint64_t* keys_in, int64_t B, int k_in, const int64
                        const int32_t* group_ids, int64_t N, int k_out, uint64_t* keys_out,
                        int32_t* err_flag, void* stream);
 
+/*
+ * Radius-search compaction (no counterpart in the reference): the keys of (n, m) lists, each row
+ * sorted descending, that are non-empty, have similarity >= tau and are not the row's own key,
+ * turned into CSR rows.  Row i of the lists is row b = row_ids[i] of the result (row_ids: (n,)
+ * int64, or NULL: b = i); the row's own key is the one with index self_offset + b (self_offset < 0: none).  Two
+ * passes of one warp per list row:
+ *   count (offsets NULL): counts[b] = min(kept keys, cap) (int64), and when full is not NULL,
+ *       full[i] (int32) = bit 0: the list's last slot is non-empty, bit 1: and its similarity is
+ *       >= tau;
+ *   emit  (offsets = the (rows + 1) int64 CSR offsets): indices / sims [offsets[b], offsets[b + 1])
+ *       = the first offsets[b + 1] - offsets[b] kept keys of the row, in list order (int64 index,
+ *       fp32 similarity).
+ * tau not NaN, m >= 1, cap >= 1; n == 0 launches nothing.
+ */
+int b200knn_radius_compact(const uint64_t* keys, int64_t n, int m, const int64_t* row_ids, float tau,
+                           int64_t self_offset, int64_t cap, int64_t* counts, int32_t* full,
+                           const int64_t* offsets, int64_t* indices, float* sims, void* stream);
+
+/*
+ * Connected components of a graph over n <= 2^31 - 1 nodes whose edges arrive in batches of CSR
+ * rows (no counterpart in the reference).  parent: (n,) int32, parent[x] = x before the first
+ * batch.
+ *   b200knn_union_edges: unions the edges (row_offset + r, indices[j]), j in [offsets[r],
+ *       offsets[r + 1]) for r < n_rows, offsets int64 relative to offsets[0]; edges are taken as
+ *       undirected.  An endpoint outside [0, n) is skipped and sets *err_flag = 2.
+ *   b200knn_components: labels (n,) int64, labels[x] = the smallest node of x's component, after
+ *       every batch is unioned; the same whatever order the edges were unioned in.
+ */
+int b200knn_union_edges(int32_t* parent, int64_t n, const int64_t* offsets, const int64_t* indices,
+                        int64_t n_rows, int64_t row_offset, int32_t* err_flag, void* stream);
+int b200knn_components(const int32_t* parent, int64_t n, int64_t* labels, void* stream);
+
 /* keys (B,k) -> sims (B,k) f32 and idx (B,k) int64  (Tensor.topk's two outputs).
  * Empty slots (fewer than k finite candidates) decode to sim=-inf, idx=-1. */
 int b200knn_decode_keys(const uint64_t* keys, int64_t n_keys, float* sims,
@@ -369,6 +401,20 @@ int b200knn_rescore_vote(const float* q, int64_t q_ld, const float* rows, int64_
                          uint64_t* band_keys, int32_t* band_info, int64_t* pred,
                          int32_t* uncertified, int32_t* status, void* workspace,
                          size_t workspace_bytes, void* stream);
+
+/*
+ * b200knn_radius_tau0: admission thresholds of a radius search (similarity >= tau, tau finite) for
+ * b200knn_topk_opt's tau0 option.  q (B, dim) fp32, row-major, ld = q_ld.  With E_b the bound
+ * b200knn_rescore_vote states (bank_resid NULL: b200knn_rescore's), tau0[b] = the largest fp32
+ * value strictly below the exact tau - E_b, so every bank row whose exact similarity is >= tau
+ * has an approximate one > tau0[b].  refused[b] = 1 (and tau0[b] = +inf, admitting nothing) where
+ * the bound does not cover the row: ||q_b|| or M >= max_abs (max_abs > 0), or E_b not finite.
+ * e_out: optional (B,) fp32, E_b itself (NULL: not written).
+ */
+int b200knn_radius_tau0(const float* q, int64_t q_ld, int64_t B, int dim, float tau, float err_coef,
+                        float err_abs, float max_abs, const float* bank_max_norm,
+                        const float* bank_resid, float acc_coef, float* tau0, int32_t* refused,
+                        float* e_out, void* stream);
 
 /*
  * Sharded fp32 mode (no counterpart in the reference, which is single-device): the owner of a

@@ -15,6 +15,8 @@ Public surface (mirrors the reference names for this path):
     ShardedBank                                   -> bank row-sharded over the GPUs of a node
     FeatureBank                                   -> fused normalise + bank build (knn.py:67-81)
     L2Index / l2_topk / knn_graph                 -> the notebooks' nearest-neighbour search, batched
+    knn_radius / radius_graph                     -> every neighbour above a similarity threshold (CSR rows)
+    near_duplicate_groups                         -> near-duplicate groups for knn_predict_loo(groups=)
     knn_metrics                                   -> macro accuracy / F1 / confusion matrix on the device
     knn_multilabel_metrics                        -> multi-label F1, subset accuracy, Hamming loss, AUC
 """
@@ -50,7 +52,16 @@ from .metrics import (  # noqa: F401
     metrics_from_counts,
     multilabel_metrics_from_scores,
 )
-from .retrieval import L2Index, knn_graph, l2_topk, load_embedding_table  # noqa: F401
+from .retrieval import (  # noqa: F401
+    L2Index,
+    RadiusNeighbors,
+    knn_graph,
+    knn_radius,
+    l2_topk,
+    load_embedding_table,
+    near_duplicate_groups,
+    radius_graph,
+)
 from .sharded import ShardedBank, shard_bounds  # noqa: F401
 
 __version__ = "0.1.0"

@@ -78,6 +78,14 @@ SIGNATURES = {
          ctypes.POINTER(c_double), c_int, c_void_p, c_int64, c_void_p, c_void_p],
     ),
     "b200knn_key_sim_column": (c_int, [c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p]),
+    "b200knn_radius_compact": (
+        c_int, [c_void_p, c_int64, c_int, c_void_p, ctypes.c_float, c_int64, c_int64, c_void_p, c_void_p, c_void_p,
+                c_void_p, c_void_p, c_void_p]),
+    "b200knn_radius_tau0": (
+        c_int, [c_void_p, c_int64, c_int64, c_int, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float,
+                c_void_p, c_void_p, ctypes.c_float, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "b200knn_union_edges": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p]),
+    "b200knn_components": (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
     "b200knn_normalize_rows": (c_int, [c_void_p, c_int, c_int64, c_int, c_int64, ctypes.c_float, c_void_p, c_void_p]),
     "b200knn_row_sqnorms": (c_int, [c_void_p, c_int, c_int64, c_int, c_int64, c_void_p, c_void_p]),
     "b200knn_confusion": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p]),
@@ -132,6 +140,7 @@ KERNELS_PER_CALL = {
     "b200knn_key_sim_column": 1, "b200knn_normalize_rows": 1, "b200knn_confusion": 1, "b200knn_row_sqnorms": 1, "b200knn_rescore": 2, "b200knn_rescore_vote": 3, "b200knn_route_keys": 1, "b200knn_certify": 1,
     "b200knn_row_norm_max": 1, "b200knn_row_f16_residual_max": 1, "b200knn_debug_topk_dump": 1, "b200knn_broadcast_f32": 1,
     "b200knn_route_scatter": 1, "b200knn_rescore_scatter": 2, "b200knn_compact_rows": 1, "b200knn_scatter_rows": 1,
+    "b200knn_radius_compact": 1, "b200knn_radius_tau0": 1, "b200knn_union_edges": 1, "b200knn_components": 1,
 }
 launch_counter = {"kernels": 0}
 

@@ -1222,6 +1222,82 @@ def drop_group(keys: torch.Tensor, row_ids: torch.Tensor, group_ids: torch.Tenso
     return out
 
 
+def radius_tau0(feature: torch.Tensor, feature_bank: torch.Tensor, tau: float, cfg: dict, cand_mode: str,
+                return_e: bool = False):
+    """(tau0 (B,) fp32, refused (B,) int32) of a radius search at similarity >= tau (fp32) whose
+    candidates come from `cand_mode` under the bound of level `cfg` (``b200knn_radius_tau0``); the
+    residual form of the bound where the level has it and the candidates really are fp16.
+    return_e: also the (B,) fp32 bound E of every row (tests)."""
+    B, D = feature.shape
+    pb = bank_cache.get(feature_bank, cand_mode)
+    err_coef, err_abs, acc_coef, resid = _bound_terms(cfg, pb, D, cfg.get("residual_bound", False) and
+                                                      cand_mode == "f16")
+    q = feature if feature.dtype == torch.float32 else feature.float()
+    if q.stride(1) != 1:
+        q = q.contiguous()
+    tau0 = torch.empty((B,), dtype=torch.float32, device=q.device)
+    refused = torch.empty((B,), dtype=torch.int32, device=q.device)
+    e = torch.empty((B,), dtype=torch.float32, device=q.device) if return_e else None
+    with torch.cuda.device(q.device):
+        _lib.check(_lib.load().b200knn_radius_tau0(q.data_ptr(), q.stride(0), B, D, float(tau), float(err_coef),
+                                                   float(err_abs), float(cfg.get("max_abs", 0.0)),
+                                                   pb.max_norm().data_ptr(), _ptr(resid), float(acc_coef),
+                                                   tau0.data_ptr(), refused.data_ptr(), _ptr(e), _stream()),
+                   "radius_tau0")
+    return (tau0, refused, e) if return_e else (tau0, refused)
+
+
+def radius_count(keys: torch.Tensor, rows: Optional[torch.Tensor], tau: float, self_offset: int, cap: int,
+                 counts: torch.Tensor) -> torch.Tensor:
+    """Count pass of ``b200knn_radius_compact``: counts[rows[i]] (rows None: i) = the keys of list
+    row i with sim >= tau, not the row's own, at most cap; returns the (n,) int32 `full` bits
+    (1: last slot non-empty, 2: and its sim >= tau)."""
+    n, m = keys.shape
+    full = torch.zeros((n,), dtype=torch.int32, device=keys.device)
+    if n:
+        keys = keys.contiguous()
+        with torch.cuda.device(keys.device):
+            _lib.check(_lib.load().b200knn_radius_compact(keys.data_ptr(), n, m, _ptr(rows), float(tau),
+                                                          int(self_offset), int(cap), counts.data_ptr(),
+                                                          full.data_ptr(), None, None, None, _stream()),
+                       "radius_compact")
+    return full
+
+
+def radius_emit(keys: torch.Tensor, rows: Optional[torch.Tensor], tau: float, self_offset: int,
+                offsets: torch.Tensor, indices: torch.Tensor, sims: torch.Tensor) -> None:
+    """Emit pass of ``b200knn_radius_compact`` into the CSR arrays (offsets from the count pass)."""
+    n, m = keys.shape
+    if n and indices.numel():
+        keys = keys.contiguous()
+        with torch.cuda.device(keys.device):
+            _lib.check(_lib.load().b200knn_radius_compact(keys.data_ptr(), n, m, _ptr(rows), float(tau),
+                                                          int(self_offset), 1, None, None, offsets.data_ptr(),
+                                                          indices.data_ptr(), sims.data_ptr(), _stream()),
+                       "radius_compact")
+
+
+def union_edges(parent: torch.Tensor, offsets: torch.Tensor, indices: torch.Tensor, row_offset: int,
+                flag: torch.Tensor) -> None:
+    """Union the CSR edges (row_offset + r, indices[j]) into the int32 parent array (``b200knn_union_edges``)."""
+    n_rows = offsets.numel() - 1
+    if n_rows > 0 and indices.numel():
+        with torch.cuda.device(parent.device):
+            _lib.check(_lib.load().b200knn_union_edges(parent.data_ptr(), parent.numel(), offsets.data_ptr(),
+                                                       indices.data_ptr(), n_rows,
+                                                       int(row_offset), flag.data_ptr(), _stream()), "union_edges")
+
+
+def components(parent: torch.Tensor) -> torch.Tensor:
+    """(n,) int64: the smallest node of every node's component (``b200knn_components``)."""
+    labels = torch.empty((parent.numel(),), dtype=torch.int64, device=parent.device)
+    if parent.numel():
+        with torch.cuda.device(parent.device):
+            _lib.check(_lib.load().b200knn_components(parent.data_ptr(), parent.numel(), labels.data_ptr(),
+                                                      _stream()), "components")
+    return labels
+
+
 def merge_keys(keys_in: torch.Tensor, k_out: int) -> torch.Tensor:
     """(G,B,k_in) sorted candidate lists -> (B,k_out): the shard-merge step."""
     lib = _lib.load()
@@ -1469,6 +1545,16 @@ def _certified_vote_applies(feature, feature_bank, num_classes, knn_k, knn_t, mo
             and feature_bank.shape[1] > max(int(knn_k), MAX_K))
 
 
+def _bound_terms(cfg: dict, pb: "PreparedRows", D: int, residual: bool):
+    """(err_coef, err_abs, acc_coef, bank_resid) of the bound E of a level (the arguments of
+    b200knn_rescore_vote and b200knn_radius_tau0): with residual, the measured fp16 residuals of the
+    bank pb (err_coef = the exact chain's gamma_D), else the level's worst-case model."""
+    if residual:
+        u = D * 2.0 ** -24
+        return u / (1.0 - u), 0.0, 1.01 * cfg["acc_c"] * padded_dim(D) * ACC_ULP, pb.f16_residuals()
+    return cfg["err_coef"], cfg.get("err_abs", 0.0) * math.sqrt(padded_dim(D)), 0.0, None
+
+
 def _predict_certified(feature, feature_bank, feature_labels, num_classes, knn_k, knn_t, mode, track, boost, status):
     """The certified vote of a rescored-mode call, nothing synchronises: (pred (B,C), flags (B,) int32, fix).
     status[1] counts the rows it leaves uncertified; fix(rows, n) returns their exact keys: their full
@@ -1486,15 +1572,7 @@ def _predict_certified(feature, feature_bank, feature_labels, num_classes, knn_k
     pb = bank_cache.get(feature_bank, cfg["cand"])
     rows, _ = pb.rescore_rows()
     max_norm = pb.max_norm()
-    if cfg.get("residual_bound"):
-        resid = pb.f16_residuals()
-        u = D * 2.0 ** -24
-        err_coef, err_abs = u / (1.0 - u), 0.0
-        acc_coef = 1.01 * cfg["acc_c"] * padded_dim(D) * ACC_ULP
-    else:
-        resid = None
-        err_coef, err_abs = cfg["err_coef"], cfg.get("err_abs", 0.0) * math.sqrt(padded_dim(D))
-        acc_coef = 0.0
+    err_coef, err_abs, acc_coef, resid = _bound_terms(cfg, pb, D, cfg.get("residual_bound", False))
     q = feature if feature.dtype == torch.float32 else feature.float()
     if q.stride(1) != 1:
         q = q.contiguous()

@@ -368,6 +368,35 @@ int b200knn_drop_group(const uint64_t* keys_in, int64_t B, int k_in, const int64
   return e == cudaSuccess ? B200KNN_OK : fail_cuda("drop_group", e);
 }
 
+int b200knn_radius_compact(const uint64_t* keys, int64_t n, int m, const int64_t* row_ids, float tau,
+                           int64_t self_offset, int64_t cap, int64_t* counts, int32_t* full, const int64_t* offsets,
+                           int64_t* indices, float* sims, void* stream) {
+  if (!keys || n < 0 || m < 1 || cap < 1) return fail(B200KNN_E_ARG, "radius_compact: bad argument (null keys, n < 0, m < 1 or cap < 1)");
+  if (std::isnan(tau)) return fail(B200KNN_E_ARG, "radius_compact: tau is NaN");
+  if (offsets == nullptr ? !counts : (!indices || !sims))
+    return fail(B200KNN_E_ARG, "radius_compact: the count pass needs counts, the emit pass indices and sims");
+  cudaError_t e = b200knn::launch_radius_compact(keys, n, m, row_ids, tau, self_offset, cap, counts, full, offsets,
+                                                 indices, sims, static_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? B200KNN_OK : fail_cuda("radius_compact", e);
+}
+
+int b200knn_union_edges(int32_t* parent, int64_t n, const int64_t* offsets, const int64_t* indices, int64_t n_rows,
+                        int64_t row_offset, int32_t* err_flag, void* stream) {
+  if (!parent || !offsets || !err_flag || n < 0 || n_rows < 0 || (n_rows > 0 && !indices))
+    return fail(B200KNN_E_ARG, "union_edges: bad argument (null pointer, n < 0 or n_rows < 0)");
+  if (n > INT32_MAX) return fail(B200KNN_E_ARG, "union_edges: more than 2^31 - 1 nodes");
+  cudaError_t e = b200knn::launch_union_edges(parent, n, offsets, indices, n_rows, row_offset, err_flag,
+                                              static_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? B200KNN_OK : fail_cuda("union_edges", e);
+}
+
+int b200knn_components(const int32_t* parent, int64_t n, int64_t* labels, void* stream) {
+  if (!parent || !labels || n < 0) return fail(B200KNN_E_ARG, "components: bad argument");
+  if (n > INT32_MAX) return fail(B200KNN_E_ARG, "components: more than 2^31 - 1 nodes");
+  cudaError_t e = b200knn::launch_components(parent, n, labels, static_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? B200KNN_OK : fail_cuda("components", e);
+}
+
 int b200knn_row_norm_max(const float* rows_a, const float* rows_b, int64_t n, int dim_pad,
                          float* out_dev, void* stream) {
   if (!rows_a || !out_dev || n < 0 || dim_pad <= 0) return fail(B200KNN_E_ARG, "row_norm_max: bad argument");
@@ -415,6 +444,29 @@ int b200knn_rescore(const void* q, int q_dtype, int64_t q_ld, const float* rows_
   p.n_uncertified = n_uncertified;
   cudaError_t e = b200knn::launch_rescore(p, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
   return e == cudaSuccess ? B200KNN_OK : fail_cuda("rescore", e);
+}
+
+int b200knn_radius_tau0(const float* q, int64_t q_ld, int64_t B, int dim, float tau, float err_coef, float err_abs,
+                        float max_abs, const float* bank_max_norm, const float* bank_resid, float acc_coef,
+                        float* tau0, int32_t* refused, float* e_out, void* stream) {
+  if (!q || !bank_max_norm || !tau0 || !refused) return fail(B200KNN_E_ARG, "radius_tau0: null pointer");
+  if (B < 0 || dim <= 0 || q_ld < dim) return fail(B200KNN_E_ARG, "radius_tau0: bad shape (need B >= 0, 0 < dim <= q_ld)");
+  if (!std::isfinite(tau)) return fail(B200KNN_E_ARG, "radius_tau0: tau must be finite");
+  b200knn::RescoreParams p{};
+  p.q = q;
+  p.q_dtype = B200KNN_F32;
+  p.q_ld = q_ld;
+  p.dim = dim;
+  p.dim_pad = (dim + 63) / 64 * 64;
+  p.B = B;
+  p.err_coef = err_coef;
+  p.err_abs = err_abs;
+  p.max_abs = max_abs;
+  p.bank_max_norm = bank_max_norm;
+  p.bank_resid = bank_resid;
+  p.acc_coef = acc_coef;
+  cudaError_t e = b200knn::launch_radius_tau0(p, tau, tau0, refused, e_out, static_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? B200KNN_OK : fail_cuda("radius_tau0", e);
 }
 
 int b200knn_rescore_vote(const float* q, int64_t q_ld, const float* rows, int64_t N, int dim,

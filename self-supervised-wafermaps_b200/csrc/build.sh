@@ -13,7 +13,7 @@ BUILD="${BUILD_DIR:-build}"
 mkdir -p "$here/$BUILD"
 pids=()
 TC_INST="tc_inst_bf16_pair tc_inst_bf16_single tc_inst_f16_pair tc_inst_f16_single tc_inst_f16x2_pair tc_inst_f16x2_single tc_inst_bf16x3 tc_inst_tf32x3"
-SRCS="$TC_INST api exact select vote prepare rescore tc_topk sharded_ops"
+SRCS="$TC_INST api exact select vote prepare rescore tc_topk sharded_ops graph"
 for f in $SRCS; do
   ( "$NVCC" "${FLAGS[@]}" -c "$here/$f.cu" -o "$here/$BUILD/$f.o" > "$here/$BUILD/$f.log" 2>&1 ) &
   pids+=($!)

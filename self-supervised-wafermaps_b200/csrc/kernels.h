@@ -68,6 +68,16 @@ cudaError_t launch_vote_multi(const uint64_t* keys, const int64_t* labels, int64
 cudaError_t launch_vote_multilabel(const uint64_t* keys, const uint64_t* label_bits, int64_t B, int64_t n_labels,
                                    int64_t label_offset, int L, const VoteGrid& grid, double* scores,
                                    int64_t scores_ld, int32_t* err_flag, cudaStream_t stream);
+// radius-search compaction of (n, m) sorted key lists (b200knn_radius_compact): offsets == nullptr
+// counts (counts[b], full[i]), otherwise emits (indices, sims) at offsets[b]
+cudaError_t launch_radius_compact(const uint64_t* keys, int64_t n, int m, const int64_t* row_ids, float tau,
+                                  int64_t self_offset, int64_t cap, int64_t* counts, int32_t* full,
+                                  const int64_t* offsets, int64_t* indices, float* sims, cudaStream_t stream);
+// connected components (graph.cu): union the edges of n_rows CSR rows into parent (n,), then
+// labels[x] = smallest index of x's component
+cudaError_t launch_union_edges(int32_t* parent, int64_t n, const int64_t* offsets, const int64_t* indices,
+                               int64_t n_rows, int64_t row_offset, int32_t* err_flag, cudaStream_t stream);
+cudaError_t launch_components(const int32_t* parent, int64_t n, int64_t* labels, cudaStream_t stream);
 // out[b] = similarity of keys[b, j] (-inf for an empty slot)
 cudaError_t launch_key_sim_column(const uint64_t* keys, int64_t B, int k, int j, float* out,
                                   cudaStream_t stream);
@@ -123,6 +133,10 @@ size_t rescore_workspace_bytes(int64_t B, int k_in);
 cudaError_t launch_rescore_vote(const RescoreParams& p, uint64_t* band, int32_t* info, const int64_t* labels,
                                 int64_t n_labels, int C, double t, int64_t* pred, int32_t* status,
                                 void* workspace, cudaStream_t stream);
+// radius-search admission thresholds: tau0[b] = largest fp32 < tau - cert_bound(row b); refused[b] = 1
+// (tau0 = +inf) where the bound does not cover the row (fp32 queries p.q, p.B rows); e_out (optional): E
+cudaError_t launch_radius_tau0(const RescoreParams& p, float tau, float* tau0, int32_t* refused, float* e_out,
+                               cudaStream_t stream);
 // the certificate alone: p.out = merged exact keys (read), p.cand = merged approximate candidates
 cudaError_t launch_certify(const RescoreParams& p, cudaStream_t stream);
 // split (n, k) key lists by owning shard: out (G, n, k), each shard's keys compacted to the front

@@ -624,6 +624,71 @@ int dot_stages() {
   return v;
 }
 
+// The norms cert_bound takes for one fp32 query row, computed by a whole warp: qn = ||q|| (the select
+// kernel's fp32 sum of squares, so that E is the certificate's E) and, when the bank's fp16 residuals
+// are given, qtn = ||f16(q)|| and rho = ||q - f16(q)|| (0 otherwise); each inflated for its rounding.
+__device__ __forceinline__ void query_norms(const RescoreParams& p, const float* qrow, int lane, float* qn,
+                                            float* qtn, float* rho) {
+  const bool resid = p.bank_resid != nullptr;
+  float qq = 0.0f;
+  // ||f16(q)||^2 and ||q - f16(q)||^2 in fp64: the squares are exact and cannot underflow
+  double tt = 0.0, rr = 0.0;
+  for (int d = lane; d < p.dim; d += 32) {
+    const float v = qrow[d];
+    qq = fmaf(v, v, qq);
+    if (resid) {
+      const double t = __half2float(f16_operand(v)), r = double(v) - t;  // exact below the max_abs range
+      tt = fma(t, t, tt);
+      rr = fma(r, r, rr);
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) qq += __shfl_xor_sync(kFull, qq, o);
+  *qtn = 0.0f;
+  *rho = 0.0f;
+  if (resid) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      tt += __shfl_xor_sync(kFull, tt, o);
+      rr += __shfl_xor_sync(kFull, rr, o);
+    }
+    *qtn = __double2float_ru(sqrt(tt)) * 1.001f;
+    *rho = __double2float_ru(sqrt(rr)) * 1.001f;
+  }
+  *qn = sqrtf(qq) * 1.001f;
+}
+
+// The largest fp32 value strictly below the exact real t - e (fp32 t, e >= 0): the rounded-down
+// difference when the subtraction is inexact (it is then below the exact value), else the next
+// value below the exact difference.
+__device__ __forceinline__ float below_difference(float t, float e) {
+  const float lo = __fsub_rd(t, e), hi = __fsub_ru(t, e);
+  return lo == hi ? nextafterf(lo, -INFINITY) : lo;
+}
+
+// Admission thresholds of a radius search (b200knn_radius_tau0), one warp per fp32 query row:
+// tau0[b] = the largest fp32 strictly below tau - E_b, E_b = cert_bound of the row.  Every column
+// whose exact similarity is >= tau then has an approximate one > tau0[b], since |a - s| <= E_b.
+// Rows the bound does not cover (operand range max_abs, non-finite E) get refused[b] = 1 and
+// tau0[b] = +inf, which admits no column.  e_out (optional): E_b itself.
+__global__ void __launch_bounds__(128)
+    radius_tau0_kernel(RescoreParams p, float tau, float* __restrict__ tau0, int32_t* __restrict__ refused,
+                       float* __restrict__ e_out) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int64_t b = int64_t(blockIdx.x) * 4 + warp;
+  if (b >= p.B) return;
+  float qn, qtn, rho;
+  query_norms(p, static_cast<const float*>(p.q) + b * p.q_ld, lane, &qn, &qtn, &rho);
+  const float m = *p.bank_max_norm;
+  const float e = cert_bound(p, qn, qtn, rho);
+  const bool ok = isfinite(e) && !(p.max_abs > 0.0f && !(qn < p.max_abs && m < p.max_abs));
+  if (lane == 0) {
+    tau0[b] = ok ? below_difference(tau, e) : INFINITY;
+    refused[b] = ok ? 0 : 1;
+    if (e_out != nullptr) e_out[b] = e;
+  }
+}
+
 // ------------------------------------------------------------------ certified class vote (DESIGN §4.1c)
 // knn_predict needs the class ranking, not the neighbour keys.  Per query (warp), with the
 // approximate candidates a_1 >= ... >= a_m (m = k_in) and the row's certificate bound E:
@@ -639,33 +704,9 @@ __global__ void __launch_bounds__(128)
   const int64_t b = int64_t(blockIdx.x) * 4 + warp;
   if (b >= p.B) return;
   const uint64_t* cand = p.cand + b * p.k_in;
-  const float* qrow = static_cast<const float*>(p.q) + b * p.q_ld;
-  const bool resid = p.bank_resid != nullptr;
-  float qq = 0.0f;  // the select kernel's ||q||, so that E is the certificate's E
-  // ||f16(q)||^2 and ||q - f16(q)||^2 in fp64: the squares are exact and cannot underflow
-  double tt = 0.0, rr = 0.0;
-  for (int d = lane; d < p.dim; d += 32) {
-    const float v = qrow[d];
-    qq = fmaf(v, v, qq);
-    if (resid) {
-      const double t = __half2float(f16_operand(v)), r = double(v) - t;  // exact below the max_abs range
-      tt = fma(t, t, tt);
-      rr = fma(r, r, rr);
-    }
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) qq += __shfl_xor_sync(kFull, qq, o);
-  float qtn = 0.0f, rho = 0.0f;
-  if (resid) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      tt += __shfl_xor_sync(kFull, tt, o);
-      rr += __shfl_xor_sync(kFull, rr, o);
-    }
-    qtn = __double2float_ru(sqrt(tt)) * 1.001f;
-    rho = __double2float_ru(sqrt(rr)) * 1.001f;
-  }
-  const float qn = sqrtf(qq) * 1.001f, m = *p.bank_max_norm;
+  float qn, qtn, rho;
+  query_norms(p, static_cast<const float*>(p.q) + b * p.q_ld, lane, &qn, &qtn, &rho);
+  const float m = *p.bank_max_norm;
   const float e = cert_bound(p, qn, qtn, rho);
   const bool ok = cand[p.k_in - 1] != 0ull && isfinite(e) &&
                   !(p.max_abs > 0.0f && !(qn < p.max_abs && m < p.max_abs));
@@ -908,6 +949,13 @@ cudaError_t launch_rescore_vote(const RescoreParams& p, uint64_t* band, int32_t*
   if (g32 <= 16) return launch_rescore_vote_t<16>(p, tmp, g32, inf, labels, n_labels, C, t, pred, status, stream);
   if (g32 <= 32) return launch_rescore_vote_t<32>(p, tmp, g32, inf, labels, n_labels, C, t, pred, status, stream);
   return cudaErrorInvalidValue;
+}
+
+cudaError_t launch_radius_tau0(const RescoreParams& p, float tau, float* tau0, int32_t* refused, float* e_out,
+                               cudaStream_t stream) {
+  if (p.B == 0) return cudaSuccess;
+  radius_tau0_kernel<<<unsigned((p.B + 3) / 4), 128, 0, stream>>>(p, tau, tau0, refused, e_out);
+  return cudaGetLastError();
 }
 
 cudaError_t launch_certify(const RescoreParams& p, cudaStream_t stream) {

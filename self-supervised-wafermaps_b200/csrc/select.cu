@@ -1,6 +1,6 @@
 // select.cu — candidate-list merge (the exchange step of the sharded mode and
 // of bank splits inside one GPU), the self- and group-exclusion of leave-one-out
-// lists and key decoding.
+// lists, the compaction of radius-search lists and key decoding.
 //
 // Inputs are lists of 64-bit selection keys sorted descending under the
 // canonical (sim desc, idx asc) order, so merging G lists is itself a top-k of
@@ -382,6 +382,69 @@ __global__ void __launch_bounds__(256) drop_group_kernel(const uint64_t* __restr
   if (bad) atomicExch(err_flag, 2);
 }
 
+// Radius-search compaction (b200knn_radius_compact), one warp per row of a (n, m) key list sorted
+// descending: a key is kept when it is non-empty, its similarity is >= tau and its index is not the
+// row's own (self_offset + the row's number; self_offset < 0: none).  Row i of the list is row
+// b = row_ids[i] of the result (row_ids NULL: b = i).  Every key of the list is examined: a NaN
+// similarity sorts first and is not kept, so the kept keys need not be a prefix.  A ballot plus a
+// prefix popcount gives each kept key its position, as in drop_group_kernel.
+__device__ __forceinline__ bool radius_keep(uint64_t key, float tau, int64_t self) {
+  return key != 0ull && key_sim(key) >= tau && key_idx(key) != self;
+}
+
+// counts[b] = min(kept, cap); full[i] = bit 0: the list's last slot is non-empty, bit 1: and its
+// similarity is >= tau (the row may continue past this list)
+__global__ void __launch_bounds__(256) radius_count_kernel(const uint64_t* __restrict__ keys, int64_t n, int m,
+                                                           const int64_t* __restrict__ row_ids, float tau,
+                                                           int64_t self_offset, int64_t cap,
+                                                           int64_t* __restrict__ counts, int32_t* __restrict__ full) {
+  const int lane = threadIdx.x & 31;
+  const int64_t row = int64_t(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (row >= n) return;
+  const int64_t b = row_ids != nullptr ? row_ids[row] : row;
+  const int64_t self = self_offset >= 0 ? b + self_offset : -1;
+  const uint64_t* src = keys + row * m;
+  int64_t c = 0;
+  for (int j0 = 0; j0 < m; j0 += 32) {
+    const uint64_t key = j0 + lane < m ? src[j0 + lane] : 0ull;
+    c += __popc(__ballot_sync(kFull, radius_keep(key, tau, self)));
+  }
+  if (lane == 0) {
+    counts[b] = c < cap ? c : cap;
+    if (full != nullptr) {
+      const uint64_t last = src[m - 1];
+      full[row] = last != 0ull ? (key_sim(last) >= tau ? 3 : 1) : 0;
+    }
+  }
+}
+
+// indices / sims [offsets[b], offsets[b + 1]) = the first offsets[b + 1] - offsets[b] kept keys of row b
+__global__ void __launch_bounds__(256) radius_emit_kernel(const uint64_t* __restrict__ keys, int64_t n, int m,
+                                                          const int64_t* __restrict__ row_ids, float tau,
+                                                          int64_t self_offset, const int64_t* __restrict__ offsets,
+                                                          int64_t* __restrict__ indices, float* __restrict__ sims) {
+  const int lane = threadIdx.x & 31;
+  const int64_t row = int64_t(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (row >= n) return;
+  const int64_t b = row_ids != nullptr ? row_ids[row] : row;
+  const int64_t self = self_offset >= 0 ? b + self_offset : -1;
+  const int64_t base = offsets[b], n_out = offsets[b + 1] - base;
+  const uint64_t* src = keys + row * m;
+  const unsigned lt_mask = (1u << lane) - 1u;
+  int64_t c = 0;  // kept so far (warp-uniform)
+  for (int j0 = 0; j0 < m && c < n_out; j0 += 32) {
+    const uint64_t key = j0 + lane < m ? src[j0 + lane] : 0ull;
+    const bool keep = radius_keep(key, tau, self);
+    const unsigned bm = __ballot_sync(kFull, keep);
+    const int64_t pos = c + __popc(bm & lt_mask);
+    if (keep && pos < n_out) {
+      indices[base + pos] = key_idx(key);
+      sims[base + pos] = key_sim(key);
+    }
+    c += __popc(bm);
+  }
+}
+
 __global__ void key_sim_column_kernel(const uint64_t* __restrict__ keys, int64_t B, int k, int j,
                                       float* __restrict__ out) {
   const int64_t b = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -454,6 +517,20 @@ cudaError_t launch_drop_group(const uint64_t* in, int64_t B, int k_in, const int
   constexpr int kWarps = 8;
   drop_group_kernel<<<unsigned((B + kWarps - 1) / kWarps), kWarps * 32, 0, stream>>>(
       in, B, k_in, row_ids, group_ids, N, k_out, out, err_flag);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_radius_compact(const uint64_t* keys, int64_t n, int m, const int64_t* row_ids, float tau,
+                                  int64_t self_offset, int64_t cap, int64_t* counts, int32_t* full,
+                                  const int64_t* offsets, int64_t* indices, float* sims, cudaStream_t stream) {
+  if (n == 0) return cudaSuccess;
+  constexpr int kWarps = 8;
+  const unsigned blocks = unsigned((n + kWarps - 1) / kWarps);
+  if (offsets == nullptr)
+    radius_count_kernel<<<blocks, kWarps * 32, 0, stream>>>(keys, n, m, row_ids, tau, self_offset, cap, counts, full);
+  else
+    radius_emit_kernel<<<blocks, kWarps * 32, 0, stream>>>(keys, n, m, row_ids, tau, self_offset, offsets, indices,
+                                                           sims);
   return cudaGetLastError();
 }
 
